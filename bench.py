@@ -12,11 +12,15 @@ to HBM.  One launch writes ~630 MB, far more than the 126 MB L2, and consecutive
 two output buffers.
 
 How the timed region is built (so that it measures the kernels, not the host's launch path):
-  * K steps take ~2 ms at the driver's K = 20, so the K-step block is repeated `timed_reps` times back to
-    back until the region lasts >= --min-ms (all ranks agree on the count); value = envs * K * reps / time;
+  * it holds exactly --steps env-batch steps (fused launches of --chunk steps, plus one shorter launch for a
+    remainder); value = envs * K / time.  A step of 2^20 envs takes ~5 us, so a K of a few hundred or more
+    keeps the edges of the window small against the work inside it;
   * the region starts on a BUSY stream: a few untimed launches are queued first and the start event is
     recorded behind them, so host launch latency never sits inside the event window;
-  * the NVML clock sampler polls every 50 ms (it used to poll every 5 ms from inside a 0.2 ms window).
+  * the NVML clock sampler polls every 50 ms.
+
+`--dump-outputs DIR` writes what the timed launches returned for their last step (see `dump_outputs`); the
+inputs depend only on the arguments, so two builds run with the same arguments can be compared array for array.
 
 Before anything is timed every rank replays a sample of its own environments through the CPU oracle
 (`parity_check`), and the JSON line carries a `configs` block with the other BASELINE.json configurations
@@ -48,15 +52,16 @@ CONFIG_PARITY_STEPS = 128    # the `configs` entries: a shorter replay per confi
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=1024)
+    ap.add_argument("--steps", type=int, default=1024, help="env-batch steps inside the timed region")
     ap.add_argument("--warmup", type=int, default=64)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--envs", type=int, default=1 << 20, help="environments per GPU")
     ap.add_argument("--chunk", type=int, default=20,
                     help="env-batch steps fused per kernel launch (20: measured optimum of k_agent_rollout at 2^20 envs, "
                          "DESIGN.md section 5.1; longer rollouts are split into such launches by the library anyway)")
-    ap.add_argument("--min-ms", type=float, default=250.0,
-                    help="the K-step block is repeated until the timed region lasts at least this long")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the last timed step returned (board, reward, flags and any discount) to DIR "
+                         "as float32 .npy files")
     ap.add_argument("--e2e-steps", type=int, default=64)
     ap.add_argument("--cpu-seconds", type=float, default=10.0, help="budget of each cpu_baseline leg")
     ap.add_argument("--obs-reps", type=int, default=8,
@@ -355,6 +360,33 @@ def device_time_ms(issue, lead, count):
     return e0.elapsed_time(e1)
 
 
+DUMP_BYTES = 60 * 10 ** 6          # --dump-outputs writes at most this much array data (plus .npy headers)
+
+
+def dump_outputs(path, out, t):
+    """--dump-outputs: step `t` of the rollout buffers `out` (board, reward, flags, discount or None), i.e. what a
+    caller of Engine.rollout receives for that step, as float32 DIR/<name>.npy.  When every env would exceed
+    DUMP_BYTES, a fixed sample of envs (PCG64 seeded with SEED, sorted) is written; env_index.npy (float64)
+    names the envs, row for row."""
+    import numpy as np
+    import torch
+    board, reward, flags, disc = out
+    arrays = {"board": board[t], "reward": reward[t], "flags": flags[t]}
+    if disc is not None:
+        arrays["discount"] = disc[t]
+    n = board.shape[1]
+    per_env = 8 + sum(4 * a[0].numel() for a in arrays.values())
+    if n * per_env <= DUMP_BYTES:
+        idx = np.arange(n)
+    else:
+        idx = np.sort(np.random.Generator(np.random.PCG64(SEED)).choice(n, DUMP_BYTES // per_env, replace=False))
+    sel = torch.as_tensor(idx, device=board.device)
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "env_index.npy"), idx.astype(np.float64))
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a[sel].float().cpu().numpy())
+
+
 def hello_actions(nat, T, seed):
     """SURVEY 8(d): Hello World actions uniform over 0..3 plus 1% quit (action 4)."""
     import torch
@@ -556,11 +588,7 @@ def run_ours(args):
     warm = plan(W)
     for i in range(len(warm)):               # warm-up (>= 3 steps)
         issue_factory(warm)(i)
-    pilot_sizes = [T] * (lead + 8)
-    pilot_ms = device_time_ms(issue_factory(pilot_sizes), lead, 8) / (8 * T)     # ms per env-batch step
-    reps = int(max(1, math.ceil(args.min_ms / max(pilot_ms * K, 1e-6))))
-    reps = int(reduce_max(float(reps)))      # every rank times the same number of steps
-    sizes = [T] * lead + plan(K * reps)
+    sizes = [T] * lead + plan(K)
     launches = len(sizes) - lead
     issue = issue_factory(sizes)
 
@@ -571,8 +599,11 @@ def run_ours(args):
     sampler.active = False
     barrier()
     ms = reduce_max(ms)
-    total_steps = K * reps
+    total_steps = K
     value = world * n * total_steps / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        last = len(sizes) - 1
+        dump_outputs(args.dump_outputs, outs[last % 2], sizes[last] - 1)
 
     # ---- roofline of the dominant kernel (k_agent_rollout): algorithmic bytes / avg launch duration ----
     cells = nat.cells
@@ -591,9 +622,9 @@ def run_ours(args):
                 "alg_bytes_per_launch": n * (t_main * per_step + state_rw), "avg_launch_ms": ms / launches,
                 "launches_timed": launches, "peak_source": peak_src}
     config = workload_config(n, world, t_main)
-    config.update({"timed_reps": reps, "timed_steps": total_steps, "timed_region_ms": ms,
-                   "timing": "K-step block repeated timed_reps times back to back (value = envs*K*reps/time), CUDA "
-                             "events on the launch stream behind %d queued untimed launches, max over ranks" % lead})
+    config.update({"timed_steps": total_steps, "timed_region_ms": ms,
+                   "timing": "K steps as back-to-back fused launches (value = envs*K/time), CUDA events on the launch "
+                             "stream behind %d queued untimed launches, max over ranks" % lead})
 
     # ---- end to end through Engine.play() with HOST buffers (H2D actions, D2H board+reward+flags) ----
     # Every step: pinned-host actions -> device, one Engine.play(), the whole result (board, reward, flags) ->

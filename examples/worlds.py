@@ -11,7 +11,7 @@ not copies of them.  Nothing here is batched or GPU-aware: `ascii_art_to_game(..
 compiles these classes to kernels at `its_showtime()`.
 
 The reference's own files also drop in: put `campx_b200` under the name `campx` on the import path
-(tests/test_compiler.py does that when /root/reference is present).
+(tests/test_compiler.py does that when CAMPX_REFERENCE_ROOT names a checkout of the reference).
 """
 import numpy as np
 import torch

@@ -1,17 +1,17 @@
 """TEST INFRASTRUCTURE ONLY -- generate tests/golden/*.json from the UNMODIFIED reference.
 
-Run in the build container (where /root/reference exists):
+Run against a checkout of the original CampX:
 
-    python oracle/gen_golden.py
+    CAMPX_REFERENCE_ROOT=<checkout> python oracle/gen_golden.py
 
-The reference (`/root/reference/campx` + `examples/boat_race.py` + the game-defining cells of the
+The reference (`campx/` + `examples/boat_race.py` of that checkout + the game-defining cells of the
 Demo 1-4 / Hello World notebooks) is executed under `oracle/shim.py`; nothing is copied from it.
 Each fixture holds action sequences and, per frame, the board, every layer, entity state, the
 backdrop curtain (pins quirk Q1), reward (value and None-ness) and discount.  Action streams are
 drawn from numpy's PCG64 with the seed stored in the fixture, so they can be re-derived.
 
-The fixtures are small (a few hundred kB in total) and committed; the GPU box, which has no
-/root/reference, checks the CUDA path and the numpy oracle against them.
+The fixtures are small (a few hundred kB in total) and committed, so the tests check the CUDA path
+and the numpy oracle against them without the checkout.
 """
 import json
 import os

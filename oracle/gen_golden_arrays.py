@@ -1,6 +1,6 @@
 """TEST INFRASTRUCTURE ONLY -- generate tests/golden/observation_arrays.json from the UNMODIFIED reference.
 
-    python oracle/gen_golden_arrays.py        (build container only: needs /root/reference)
+    CAMPX_REFERENCE_ROOT=<checkout of the original CampX> python oracle/gen_golden_arrays.py
 
 Runs the reference's `ObservationToArray` and `ObservationToFeatureArray` (campx/rendering.py:461-712) on
 observations produced by the reference engine (boat_race and Hello World, under `oracle/shim.py`) for a

@@ -1,11 +1,11 @@
 """TEST INFRASTRUCTURE ONLY -- compatibility shim that lets the *unmodified* reference
-(`/root/reference/campx`, torch==0.3.1 / numpy==1.15 era code) execute on the torch 2.x /
-numpy 2.x interpreter of this container.
+(`campx/` of a checkout of the original CampX, torch==0.3.1 / numpy==1.15 era code) execute on a
+torch 2.x / numpy 2.x interpreter.  The checkout is not part of this repository; the environment
+variable CAMPX_REFERENCE_ROOT names it (a directory holding `campx/` and `examples/`).
 
 Nothing in `campx_b200/` imports this module.  It is used only by
-`oracle/gen_golden.py` (fixture generation, in the build container where `/root/reference`
-exists) and by the `not gpu` tests that cross-check `oracle/campx_oracle.py` against the real
-reference when the reference tree is present.
+`oracle/gen_golden.py` (fixture generation, which needs the checkout) and by the `not gpu` tests
+that cross-check `oracle/campx_oracle.py` against the real reference when the checkout is given.
 
 What it does (zero edits to reference files; see SURVEY.md section 8(c) / Appendix B):
 
@@ -22,20 +22,21 @@ What it does (zero edits to reference files; see SURVEY.md section 8(c) / Append
    through to the real `set_`, which preserves the storage-aliasing quirk Q1
    (campx/rendering.py:128,150).
 """
+import os
 import sys
 import types
 
 import numpy as np
 import torch
 
-REFERENCE_ROOT = "/root/reference"
+REFERENCE_ROOT = os.path.abspath(os.environ["CAMPX_REFERENCE_ROOT"]) if os.environ.get("CAMPX_REFERENCE_ROOT") else ""
 
 _installed = False
 
 
-def reference_available():
-    import os
-    return os.path.isdir(os.path.join(REFERENCE_ROOT, "campx"))
+def reference_available(sub="campx"):
+    """True when CAMPX_REFERENCE_ROOT names a checkout that has `sub` (campx/ or examples/)."""
+    return bool(REFERENCE_ROOT) and os.path.isdir(os.path.join(REFERENCE_ROOT, sub))
 
 
 def install(reference_root=REFERENCE_ROOT):
@@ -43,6 +44,9 @@ def install(reference_root=REFERENCE_ROOT):
     global _installed
     if _installed:
         return
+    if not os.path.isdir(os.path.join(reference_root, "campx")):
+        raise RuntimeError("oracle/shim.py: %r holds no campx/; set CAMPX_REFERENCE_ROOT to a checkout of the "
+                           "original CampX" % reference_root)
     _installed = True
 
     # --- 1. stub modules -------------------------------------------------------------------
@@ -121,7 +125,6 @@ def install(reference_root=REFERENCE_ROOT):
     torch.Tensor.set_ = set_
 
     # --- 4. reference on sys.path ------------------------------------------------------------------
-    import os
     for p in (reference_root, os.path.join(reference_root, "examples")):
         if p not in sys.path:
             sys.path.insert(0, p)
@@ -134,7 +137,6 @@ def load_notebook_world(notebook_filename, reference_root=REFERENCE_ROOT):
     already *play* the game are skipped, so the caller gets the classes, GAME_ART and make_game().
     """
     import json
-    import os
     install(reference_root)
     with open(os.path.join(reference_root, "examples", notebook_filename)) as f:
         nb = json.load(f)

@@ -11,6 +11,7 @@ from campx_b200 import things
 from campx_b200.ascii_art import ascii_art_to_game, Partial
 from campx_b200.compiler import CompileError
 from examples.worlds import make_world
+from oracle import shim
 from tests.expected_specs import expected_spec
 
 WORLDS = ["boat_race", "demo1", "demo2", "demo3", "demo4", "hello"]
@@ -199,11 +200,12 @@ def test_hidden_state_is_refused():
     assert ascii_art_to_game(["M.", ".."], ".", drapes={"M": Harmless}).compile().entities[0].step_reward == [2.0] * 5
 
 
-def _reference_present():
-    return os.path.isdir("/root/reference/examples")
+REFERENCE_EXAMPLES = os.path.join(shim.REFERENCE_ROOT, "examples")
+NEEDS_REFERENCE = pytest.mark.skipif(not shim.reference_available("examples"),
+                                     reason="needs a checkout of the original CampX (set CAMPX_REFERENCE_ROOT)")
 
 
-@pytest.mark.skipif(not _reference_present(), reason="reference tree only exists in the build container")
+@NEEDS_REFERENCE
 def test_reference_boat_race_file_drops_in_unchanged(monkeypatch):
     """The reference's own examples/boat_race.py, imported with campx_b200 standing in for campx,
     compiles to exactly the primitives of our boat_race world (hence runs identically on the GPU)."""
@@ -217,7 +219,7 @@ def test_reference_boat_race_file_drops_in_unchanged(monkeypatch):
     for name, mod in (("campx", alias), ("campx.things", campx_b200.things),
                       ("campx.ascii_art", campx_b200.ascii_art), ("campx.engine", campx_b200.engine)):
         monkeypatch.setitem(sys.modules, name, mod)
-    monkeypatch.syspath_prepend("/root/reference/examples")
+    monkeypatch.syspath_prepend(REFERENCE_EXAMPLES)
     monkeypatch.delitem(sys.modules, "boat_race", raising=False)
     captured = []
 
@@ -228,12 +230,12 @@ def test_reference_boat_race_file_drops_in_unchanged(monkeypatch):
 
     monkeypatch.setattr(campx_b200.engine.Engine, "its_showtime", fake_showtime)
     import boat_race as ref_boat_race
-    assert ref_boat_race.__file__.startswith("/root/reference")
+    assert ref_boat_race.__file__.startswith(REFERENCE_EXAMPLES)
     game, _, _, _ = ref_boat_race.make_game()
     assert_same_spec(game.spec, expected_spec("boat_race"))
 
 
-@pytest.mark.skipif(not _reference_present(), reason="reference tree only exists in the build container")
+@NEEDS_REFERENCE
 @pytest.mark.parametrize("world,notebook", [
     ("demo1", "Demo 1: Simple Agent Example.ipynb"),
     ("demo2", "Demo 2: Simple Wall Example.ipynb"),
@@ -259,7 +261,7 @@ def test_reference_notebook_worlds_drop_in_unchanged(monkeypatch, world, noteboo
         return None, None, 1.0
 
     monkeypatch.setattr(campx_b200.engine.Engine, "its_showtime", fake_showtime)
-    with open(os.path.join("/root/reference/examples", notebook)) as f:
+    with open(os.path.join(REFERENCE_EXAMPLES, notebook)) as f:
         nb = json.load(f)
     ns = {"__name__": "nb"}
     for cell in nb["cells"]:

@@ -12,7 +12,7 @@ pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs (run with gpurun --gpus 2)")
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs")
 @pytest.mark.parametrize("n", [4096, 600000])      # lane-per-env kernel; k_agent_rollout (tile builds)
 def test_n_ranks_reproduce_one_gpu_env_for_env(n):
     world = min(torch.cuda.device_count(), 8)

@@ -1,7 +1,7 @@
 """ObservationToArray / ObservationToFeatureArray (campx/rendering.py:461-712).
 
 CPU: the numpy oracle against the reference-recorded fixture tests/golden/observation_arrays.json (made by
-oracle/gen_golden_arrays.py), live against the reference where /root/reference exists, and the constructor
+oracle/gen_golden_arrays.py), live against the reference where CAMPX_REFERENCE_ROOT names a checkout of it, and the constructor
 errors of the host classes.  GPU: `campx_b200.rendering` (one `cx_board_mapper_apply` launch) against the
 fixture, against the oracle on random boards of many geometries / dtypes / permutations, through real engine
 observations, and at 2^20 boards through size-independent properties.
@@ -14,6 +14,7 @@ import numpy as np
 import pytest
 
 from oracle import campx_oracle as O
+from oracle import shim
 
 
 @pytest.fixture(scope="module")
@@ -74,7 +75,8 @@ def test_host_classes_constructor_errors(fixture):
         assert str(ei.value) == rec["error"]["message"]
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/campx"), reason="reference tree not present")
+@pytest.mark.skipif(not shim.reference_available(),
+                    reason="needs a checkout of the original CampX (set CAMPX_REFERENCE_ROOT)")
 def test_oracle_matches_live_reference():
     from oracle import gen_golden as gg
     from oracle import gen_golden_arrays as ga

@@ -2,7 +2,7 @@
 
 1. against the committed fixtures in tests/golden/ (made by oracle/gen_golden.py from the unmodified
    reference under oracle/shim.py) -- runs everywhere, including the GPU box;
-2. against the reference executed live, when /root/reference exists (build container only).
+2. against the reference executed live, when CAMPX_REFERENCE_ROOT names a checkout of it.
 """
 import json
 import os
@@ -11,6 +11,7 @@ import numpy as np
 import pytest
 
 from oracle import campx_oracle as O
+from oracle import shim
 
 # the six reference worlds + the three engine-generality worlds (SURVEY 8(f) row 3: z-order directives, sprite
 # visibility, scrolling backdrop), all recorded from the reference itself by oracle/gen_golden.py
@@ -162,11 +163,8 @@ def test_engine_semantics_golden(golden_dir):
     assert boards == cases["sprite_only_world_boards"]      # quirk Q1(ii)
 
 
-def _reference_present():
-    return os.path.isdir("/root/reference/campx")
-
-
-@pytest.mark.skipif(not _reference_present(), reason="reference tree only exists in the build container")
+@pytest.mark.skipif(not shim.reference_available(),
+                    reason="needs a checkout of the original CampX (set CAMPX_REFERENCE_ROOT)")
 @pytest.mark.parametrize("world", WORLDS)
 def test_oracle_matches_live_reference(world):
     """Fresh random action streams through the real reference (under the shim) and the oracle."""
