@@ -90,19 +90,10 @@ __device__ __forceinline__ uint64_t l2_evict_first_policy() {
   asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
   return pol;
 }
-#ifndef CX_OPT_L2HINT
-#define CX_OPT_L2HINT 1   // bulk stores carry the L2 evict-first policy (0: default policy; development knob)
-#endif
 __device__ __forceinline__ void bulk_store_s2g(void* gdst, const void* ssrc, uint32_t bytes, uint64_t pol) {
-#if CX_OPT_L2HINT
   asm volatile("cp.async.bulk.global.shared::cta.bulk_group.L2::cache_hint [%0], [%1], %2, %3;" ::"l"(gdst),
                "r"((uint32_t)__cvta_generic_to_shared(ssrc)), "r"(bytes), "l"(pol)
                : "memory");
-#else
-  asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gdst),
-               "r"((uint32_t)__cvta_generic_to_shared(ssrc)), "r"(bytes)
-               : "memory");
-#endif
 }
 __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 // the source bytes of every committed bulk store have been read: the tile may be modified again

@@ -16,35 +16,14 @@
 //     statistics are striped, the figures below are for 256) for all T steps; its env state lives in registers;
 //   * the static scene (backdrop + fixed drapes composed in z-order) is staged once in shared memory as
 //     a pre-tiled byte image of the warp's 256 boards (256*cells bytes);  a step only un-pokes the
-//     agent's old cell and pokes its new one (2 byte stores per env), then the warp streams the tile to
-//     HBM with LDS.128 -> STG.128 (st.global.cs), 512 contiguous bytes per instruction;
+//     agent's old cell and pokes its new one (2 byte stores per env), then the warp sends the tile to
+//     HBM as one bulk copy (cp.async.bulk);
 //   * rewards / flags / actions are float4 / uchar4 per lane, laid out so that each instruction covers a
 //     contiguous 512 B / 128 B span;
 //   * warps only __syncwarp(); CTAs of 4 warps exist just to share the staged tables, so 1024 CTAs cover
 //     2^20 envs in one resident wave on 148 SMs (7 CTAs/SM, 25.6 KB of tile per CTA).
-#include <stdlib.h>
-
 #include "cx_agent_common.cuh"
 #include "cx_philox.cuh"
-
-#ifndef CX_OPT_MINBLOCKS
-#define CX_OPT_MINBLOCKS 7
-#endif
-#ifndef CX_OPT_PDL
-#define CX_OPT_PDL 1   // programmatic dependent launch: the next launch's prologue overlaps this launch's tail
-#endif
-#ifndef CX_OPT_PF
-#define CX_OPT_PF 2    // L2 prefetch of action rows: 0 none, 1 plain, 2 evict_last
-#endif
-#ifndef CX_OPT_ACT2
-#define CX_OPT_ACT2 1  // action loads run two steps ahead of their use
-#endif
-#ifndef CX_OPT_CTASYNC
-#define CX_OPT_CTASYNC 2   // the CTA's warps meet at a named barrier before every step (2^20 envs, 64-env build: 95.8 % against 94.7 %)
-#endif
-#ifndef CX_OPT_TMA
-#define CX_OPT_TMA 1   // board tiles leave shared memory as one cp.async.bulk (UBLKCP) per warp and step
-#endif
 
 namespace {
 
@@ -76,7 +55,7 @@ struct AgentParams {
 //   NG 1, GW 2    64 envs per warp: four times the warps for small ones (BASELINE config 1: 65,536 envs)
 // CTAs are 1..4 warps (blockDim), chosen by the launcher so that small grids still spread evenly over the SMs.
 template <bool TRACK, bool VEC, bool SYNTH, int NG, int GW>
-__global__ void __launch_bounds__(CX_AGENT_CTA_THREADS, CX_OPT_MINBLOCKS)  // 7 CTAs/SM: 1024 CTAs (2^20 envs) in one wave
+__global__ void __launch_bounds__(CX_AGENT_CTA_THREADS, 7)  // 7 CTAs/SM: 1024 CTAs (2^20 envs) in one wave
 k_agent_rollout(const __grid_constant__ AgentParams P) {
   constexpr int WT = NG * 32 * GW;                 // envs per warp
   constexpr int LPR = WT >= 128 ? WT / 128 : 1;    // 128-byte lines per row of this warp's actions
@@ -87,11 +66,9 @@ k_agent_rollout(const __grid_constant__ AgentParams P) {
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int cells = H.cells;
 
-#if CX_OPT_PDL
   // Let the next launch in the stream become resident as our CTAs retire and run its prologue (tables and
   // tile staging touch only immutable data); it blocks at griddepcontrol.wait until this grid has completed.
   asm volatile("griddepcontrol.launch_dependents;");
-#endif
   // ---- stage the static tables (transition table, rewards, base board, tile pattern) ----
   {
     const uint4* src = reinterpret_cast<const uint4*>(P.blob);
@@ -126,9 +103,7 @@ k_agent_rollout(const __grid_constant__ AgentParams P) {
   }
   __syncwarp();
 
-#if CX_OPT_PDL
   asm volatile("griddepcontrol.wait;" ::: "memory");  // everything earlier in the stream is complete and visible
-#endif
   // ---- load env state into registers; paint the agents into the tile ----
   uint32_t cellv[NG][GW];   // agent cell
   uint32_t drawnq[NG];      // per env one byte: cell where the agent is currently drawn in the tile (none: nowhere)
@@ -182,20 +157,12 @@ k_agent_rollout(const __grid_constant__ AgentParams P) {
       const int tr = t0 + lane / LPR;   // a row of this warp's actions is LPR 128-byte lines (or part of one)
       if (tr < P.T) {
         const uint8_t* a = P.actions + (int64_t)tr * n + env0 + (lane % LPR) * 128;
-#if CX_OPT_PF >= 2
         asm volatile("prefetch.global.L2::evict_last [%0];" ::"l"(a));
-#elif CX_OPT_PF == 1
-        asm volatile("prefetch.global.L2 [%0];" ::"l"(a));
-#endif
       }
     }
   };
-#if CX_OPT_PF == 3
-  for (int t0 = 0; t0 < P.T; t0 += 16) prefetch_actions(t0);
-#else
   prefetch_actions(0);
   prefetch_actions(16);
-#endif
 
   // the quad of envs a lane owns: actions are read from HBM, or generated (same Philox stream as
   // cx_fill_actions: counter = (global env >> 2, step))
@@ -217,26 +184,24 @@ k_agent_rollout(const __grid_constant__ AgentParams P) {
 #pragma unroll
   for (int j = 0; j < NG; ++j) {
     actq[j] = quad_actions(j, 0);
-    actn[j] = (CX_OPT_ACT2 && P.T > 1) ? quad_actions(j, 1) : 0u;
+    actn[j] = P.T > 1 ? quad_actions(j, 1) : 0u;
   }
 
-  constexpr bool TMA = VEC && (CX_OPT_TMA != 0);
+  // Vector warps send their board tiles out of shared memory as one cp.async.bulk (UBLKCP) per warp and step, with the
+  // L2 evict-first policy; the scalar path copies them byte by byte.
   const uint64_t l2pol = l2_evict_first_policy();
 
-  // The warps of a CTA meet at a named barrier before every step.  Nothing they compute depends on it; it keeps their
-  // tiles (contiguous in HBM) leaving at the same time, and with them the DRAM rows they share: 256-env build +1.3 % at
-  // 2^20 envs (91.9 % against 90.6 % of the copy peak at 20 steps per launch; a barrier every fourth step: +0.5 %),
-  // 64-env build +1 % (95.8 % against 94.7 %).
-  constexpr bool CTASYNC = CX_OPT_CTASYNC != 0 && (NG == 2 || CX_OPT_CTASYNC == 2) && VEC;   // 1: the 256-env build only
+  // The vector warps of a CTA meet at a named barrier before every step.  Nothing they compute depends on it; it keeps
+  // their tiles (contiguous in HBM) leaving at the same time, and with them the DRAM rows they share: 256-env build
+  // +1.3 % at 2^20 envs (91.9 % against 90.6 % of the copy peak at 20 steps per launch; a barrier every fourth step:
+  // +0.5 %), 64-env build +1 % (95.8 % against 94.7 %).
   const int64_t warps_total = (P.n_end - P.env_base + WT - 1) / WT;
   const int active_threads = 32 * (int)min((int64_t)WARPS, warps_total - (int64_t)blockIdx.x * WARPS);
   for (int t = 0; t < P.T; ++t) {
-    if (CTASYNC && active_threads > 32) asm volatile("bar.sync 1, %0;" ::"r"(active_threads) : "memory");
+    if (VEC && active_threads > 32) asm volatile("bar.sync 1, %0;" ::"r"(active_threads) : "memory");
     const int64_t row = (int64_t)t * n + env0;  // index of this warp's first env in [T, n] arrays
     const int64_t row_end = (int64_t)(t + 1) * n;
-#if CX_OPT_PF != 3
     if ((t & 15) == 0) prefetch_actions(t + 32);
-#endif
     // ---- phase A (registers and tables only): the step of every env this lane owns ----
     uint32_t shwq[NG];  // per env one byte: where the agent is drawn after this step
 #pragma unroll
@@ -299,14 +264,10 @@ k_agent_rollout(const __grid_constant__ AgentParams P) {
     }
 #pragma unroll
     for (int j = 0; j < NG; ++j) {
-#if CX_OPT_ACT2
       actq[j] = actn[j];
       if (t + 2 < P.T) actn[j] = quad_actions(j, t + 2);
-#else
-      if (t + 1 < P.T) actq[j] = quad_actions(j, t + 1);
-#endif
     }
-    if (TMA) {  // the previous step's bulk store must have read the tile before it is modified
+    if (VEC) {  // the previous step's bulk store must have read the tile before it is modified
       if (lane == 0) bulk_wait_read();
       __syncwarp();
     }
@@ -331,7 +292,7 @@ k_agent_rollout(const __grid_constant__ AgentParams P) {
     }
     // ---- stream the finished boards of this warp's envs to HBM ----
     uint8_t* dst = P.board + row * cells;
-    if (TMA) {
+    if (VEC) {
       fence_async_smem();
       __syncwarp();
       if (lane == 0) {
@@ -340,20 +301,12 @@ k_agent_rollout(const __grid_constant__ AgentParams P) {
       }
     } else {
       __syncwarp();
-      if (VEC) {
-        const uint4* t16 = reinterpret_cast<const uint4*>(tile);
-        uint4* d16 = reinterpret_cast<uint4*>(dst);
-        const int nchunks = WT * cells / 16;
-#pragma unroll 4
-        for (int k = lane; k < nchunks; k += 32) __stcs(d16 + k, t16[k]);
-      } else {
-        const int nbytes = nenv * cells;
-        for (int k = lane; k < nbytes; k += 32) dst[k] = tile[k];
-      }
+      const int nbytes = nenv * cells;
+      for (int k = lane; k < nbytes; k += 32) dst[k] = tile[k];
       __syncwarp();
     }
   }
-  if (TMA) {  // shared memory must outlive the last bulk read
+  if (VEC) {  // shared memory must outlive the last bulk read
     if (lane == 0) bulk_wait_read();
     __syncwarp();
   }
@@ -422,7 +375,7 @@ int launch(const AgentParams& P, unsigned grid, unsigned block, size_t smem, cud
                                     227 * 1024));
     configured.mark();
   }
-#if CX_OPT_PDL
+  // programmatic dependent launch: the next launch's prologue overlaps this launch's tail
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(grid);
   cfg.blockDim = dim3(block);
@@ -430,16 +383,10 @@ int launch(const AgentParams& P, unsigned grid, unsigned block, size_t smem, cud
   cfg.stream = s;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  const char* pdl_env = getenv("CX_AGENT_PDL");   // development knob, read per launch
-  const bool pdl = pdl_env == nullptr || atoi(pdl_env) != 0;
-  attr[0].val.programmaticStreamSerializationAllowed = pdl ? 1 : 0;
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
   CX_CUDA_OK(cudaLaunchKernelEx(&cfg, k_agent_rollout<TRACK, VEC, SYNTH, NG, GW>, P));
-#else
-  k_agent_rollout<TRACK, VEC, SYNTH, NG, GW><<<grid, block, smem, s>>>(P);
-  CX_CUDA_OK(cudaGetLastError());
-#endif
   return CX_OK;
 }
 
@@ -463,7 +410,7 @@ int launch_s(bool synth, bool track, bool vec, const AgentParams& P, unsigned gr
 
 int cx_launch_agent_rollout(const cx_game* g, void* d_state, int64_t n, int32_t T, const uint8_t* d_actions,
                             const CxSynth& synth, float* d_reward, float* d_discount, uint8_t* d_flags,
-                            uint8_t* d_board, cudaStream_t s) {
+                            uint8_t* d_board, CxRoute route, cudaStream_t s) {
   const CxStateLayout L = cx_layout(g, n);
   uint8_t* base = static_cast<uint8_t*>(d_state);
   AgentParams P;
@@ -489,7 +436,7 @@ int cx_launch_agent_rollout(const cx_game* g, void* d_state, int64_t n, int32_t 
   auto al16 = [](const void* p) { return p == nullptr || (reinterpret_cast<uintptr_t>(p) & 15) == 0; };
   // envs per warp, by envs per SM (measured on 148 SMs, Demo 1, 32-step launches, % of the HBM copy peak for
   // 64 / 128 / 256 envs per warp: 65,536 envs 45 / 36 / 19, 2^17 65 / 62 / 37, 2^18 79 / 87 / 63, 2^19 83 / 82 / 79,
-  // 2^20 77 / 84 / 86; scripts/r02_probe.py).  CX_AGENT_WT = 64 | 128 | 256 forces a build.
+  // 2^20 77 / 84 / 86; scripts/r02_probe.py).  The routes tile64 / tile128 / tile256 force a build.
   // Since the episode statistics are striped (cx_internal.cuh: CX_STAT_STRIPES; the end-of-launch atomics of 4,096 warps
   // on one line used to cost the 256-env build least) the 64-env build wins at every size that reaches this kernel:
   // boat_race, % of the copy peak for 64 / 128 / 256 envs per warp: 2^19 envs 91.5 / 84.6 / 73, 2^20 95 / 89-92 / 88-93.
@@ -500,10 +447,9 @@ int cx_launch_agent_rollout(const cx_game* g, void* d_state, int64_t n, int32_t 
   // 15.3 / 13.8 / 18.3 (scripts/r02_probe.py tsmall).
   const int64_t per_sm = (n + g->sm_count - 1) / g->sm_count;
   if (T <= 4 && per_sm >= 1800) WT = (T == 1 && per_sm >= 6000) ? 256 : 128;
-  if (const char* dbg = getenv("CX_AGENT_WT")) {
-    const int w = atoi(dbg);
-    if (w == 64 || w == 128 || w == 256) WT = w;
-  }
+  if (route == CX_ROUTE_TILE64) WT = 64;
+  if (route == CX_ROUTE_TILE128) WT = 128;
+  if (route == CX_ROUTE_TILE256) WT = 256;
   // Vector path: every warp owns a full tile of WT envs and every [T, n] row starts 16-byte aligned.  A batch of a
   // multiple of 16 envs that is not a whole number of tiles runs its whole tiles here and the rest (16..WT-16 envs) as
   // one or two warps of k_agent_rollout_lane, not on the scalar path: boat_race, 20 steps, 500,000 envs ran entirely
@@ -548,10 +494,9 @@ int cx_launch_agent_rollout(const cx_game* g, void* d_state, int64_t n, int32_t 
   // of a launch synchronise only inside their CTA, so over a long launch the CTAs drift apart and the write stream
   // loses its DRAM row locality: measured at 2^20 envs with the 64-env build, % of the copy peak by steps per launch
   // -- 12: 95.2, 16: 96.1, 24: 96.0, 32: 96.1, 48: 95.5, 100: 92.3 (256-env build before the statistics were striped:
-  // 20: 91.0, 32: 87.4, 100: 79.8).  CX_AGENT_SUBT overrides the piece length (0: never split).
-  int sub = 32;
-  if (const char* dbg = getenv("CX_AGENT_SUBT")) sub = atoi(dbg);
-  if (sub <= 0 || T <= sub + sub / 2 || n < (int64_t)g->sm_count * 3000) return launch_wt(P);   // small batches: one launch
+  // 20: 91.0, 32: 87.4, 100: 79.8).
+  constexpr int sub = 32;
+  if (T <= sub + sub / 2 || n < (int64_t)g->sm_count * 3000) return launch_wt(P);   // small batches: one launch
   const int pieces = (T + sub - 1) / sub;
   for (int i = 0, t = 0; i < pieces; ++i) {
     const int steps = (T - t + (pieces - i) - 1) / (pieces - i);   // balanced: 100 -> 4 x 25

@@ -19,8 +19,6 @@
 //     straight from the generic proxy: no proxy fence, no TMA issue latency, no read-wait; two tiles alternate so that
 //     one __syncwarp per step orders the pokes of step t+2 behind the reads of step t.
 // Large batches stay on k_agent_rollout (TMA bulk stores: fewer LSU instructions once the SM is full of warps).
-#include <stdlib.h>
-
 #include "cx_agent_common.cuh"
 #include "cx_philox.cuh"
 
@@ -340,10 +338,6 @@ int cx_launch_agent_rollout_lane(const cx_game* g, void* d_state, int64_t n, int
   // warps per CTA: 4, fewer while that leaves the grid under ~8 CTAs per SM (small grids spread more evenly)
   int wpc = LANE_MAX_WARPS;
   while (wpc > 1 && (warps + wpc - 1) / wpc < (int64_t)g->sm_count * 8) wpc >>= 1;
-  if (const char* dbg = getenv("CX_LANE_WPC")) {
-    const int w = atoi(dbg);
-    if (w == 1 || w == 2 || w == 4) wpc = w;
-  }
   const int64_t grid = (warps + wpc - 1) / wpc;
   if (grid > 0x7fffffff) {
     cx_set_error("cx_rollout: too many environments for one launch");
@@ -355,10 +349,9 @@ int cx_launch_agent_rollout_lane(const cx_game* g, void* d_state, int64_t n, int
   // runs.  For grids of 12-30 one-warp CTAs per SM that costs more than it hides -- the early CTAs take their slots
   // wherever room is, and the launch then runs unevenly spread over the SMs: Demo 1, 32 / 100 steps per launch, us per
   // launch with / without: 8,192 envs 9.1 / 10.8, 32,768 12.3 / 12.2, 65,536 18.9 / 16.1 (100 steps: 51.8 / 40.7),
-  // 98,304 23.6 / 21.8, 2^17 29.3 / 28.5, 2^18 50.0 / 50.4.  CX_AGENT_PDL = 0 | 1 forces it.
+  // 98,304 23.6 / 21.8, 2^17 29.3 / 28.5, 2^18 50.0 / 50.4.
   const int64_t warps_per_sm = warps / g->sm_count;
-  bool pdl = !(warps_per_sm >= 12 && warps_per_sm <= 30);
-  if (const char* dbg = getenv("CX_AGENT_PDL")) pdl = atoi(dbg) != 0;
+  const bool pdl = !(warps_per_sm >= 12 && warps_per_sm <= 30);
   const unsigned blk = 32u * wpc;
   // SMALL needs a first chunk for every lane: 32 <= chunks per tile <= 64, i.e. boards of 16..32 cells
   const int sel = (track ? 8 : 0) | (synth.on ? 4 : 0) | (d_discount ? 2 : 0) | ((g->ah.cells >= 16 && g->ah.cells <= 32) ? 1 : 0);

@@ -21,8 +21,6 @@
 // are too large for k_agent_rollout's 256-env warp tiles (97..254 cells): at >= 100 bytes per env-step a
 // lane-per-env warp saturates HBM as well.  It also takes ragged batches (N not a multiple of 32) and
 // unaligned buffers (coalesced byte stores instead of the bulk stores) and in-kernel Philox actions.
-#include <stdlib.h>
-
 #include "cx_agent_common.cuh"
 #include "cx_philox.cuh"
 
@@ -379,8 +377,6 @@ int cx_launch_agent_rollout_obs(const cx_game* g, void* d_state, int64_t n, int3
   const bool lay = d_layered != nullptr;
   int ring = 1;
   if (P.bulk && T > 1 && n < 65536 && obs_smem_bytes(g, lay, 2) <= (size_t)(lay ? 56 : 32) * 1024) ring = 2;
-  if (const char* dbg = getenv("CX_OBS_RING")) ring = atoi(dbg);   // development knob: 1, 2 or 4
-  ring = ring >= 4 ? 4 : (ring >= 2 ? 2 : 1);
   const size_t smem = obs_smem_bytes(g, lay, ring);
   if (smem > 227 * 1024) {
     cx_set_error("cx_rollout: board too large for the lane-per-env kernel with %d tiles per warp", ring);

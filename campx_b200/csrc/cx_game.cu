@@ -672,9 +672,6 @@ static int build_generic_tables(const cx_game_desc* d, const int* order, CxGenHe
   // direct composer eligibility (see CxGenHeader::direct)
   bool direct_ok = cells >= 16 && E > 0 && !H->dyn_render;
   {
-    bool ok = direct_ok;
-    if (const char* dbg = getenv("CX_GEN_DIRECT")) ok = ok && atoi(dbg) != 0;  // development knob
-    if (getenv("CX_GEN_SLOW") && atoi(getenv("CX_GEN_SLOW"))) ok = false;
     size_t tab_bytes = 0;
     const int xw = (cells + 16 + 31) / 32 + 1;
     for (int z = 0; z < E; ++z) {
@@ -682,17 +679,16 @@ static int build_generic_tables(const cx_game_desc* d, const int* order, CxGenHe
       if (g.kind == CX_KIND_STATIC) tab_bytes += (size_t)xw * 4;
       if (g.kind == CX_KIND_ROLL) tab_bytes += (size_t)C * xw * 4;
     }
-    if (tab_bytes > 48 * 1024) ok = false;
+    if (tab_bytes > 48 * 1024) direct_ok = false;
     // every visible one-cell entity must be below all masks or above all masks
-    for (int z = 0; z < E && ok; ++z) {
+    for (int z = 0; z < E && direct_ok; ++z) {
       const CxGenEntity& g = H->ent[z];
       if (g.kind == CX_KIND_STATIC || g.kind == CX_KIND_ROLL || !g.visible) continue;
       int below = 0, above = 0;
       for (int y = 0; y < E; ++y)
         if (H->ent[y].kind == CX_KIND_STATIC || H->ent[y].kind == CX_KIND_ROLL) (y < z ? below : above)++;
-      if (below && above) ok = false;
+      if (below && above) direct_ok = false;
     }
-    direct_ok = ok;
   }
   // Mask entities (static / rolling drapes) are composed from linear bitsets.  A rolling mask, and a static
   // mask with a visible one-cell entity above it in z-order (whose cell is punched out of the mask), need a
@@ -711,9 +707,6 @@ static int build_generic_tables(const cx_game_desc* d, const int* order, CxGenHe
   }
   H->n_lin = n_lin;
   H->fast_compose = (n_lin <= CX_MAX_LIN && !wide_roll && cells >= 16 && !H->dyn_render) ? 1 : 0;
-  if (const char* dbg = getenv("CX_GEN_SLOW")) {  // development knob: force the per-cell composer
-    if (atoi(dbg)) H->fast_compose = 0;
-  }
   for (int i = 0; i < CX_MAX_LIN; ++i) H->off_colroll[i] = -1;
   if (H->fast_compose && !direct_ok) {
     // A roll by (dr, dc) is a column roll inside every board row followed by a rotation of the linear
@@ -797,8 +790,7 @@ static int build_generic_tables(const cx_game_desc* d, const int* order, CxGenHe
   for (int z = 0; z < E; ++z)
     if (H->ent[z].stamps) H->stamper[H->n_stampers++] = (uint16_t)((H->ent[z].ch << 8) | H->ent[z].dyn_slot);
   {
-    bool simple = !needs_prev && H->n_groups == 1 && !H->dyn_render;
-    if (const char* dbg = getenv("CX_GEN_SIMPLE")) simple = simple && atoi(dbg) != 0;  // development knob
+    const bool simple = !needs_prev && H->n_groups == 1 && !H->dyn_render;
     for (int z = 0; z < E; ++z) {
       const CxGenEntity& g = H->ent[z];
       if (g.dyn_slot == 0xFF) continue;
@@ -833,16 +825,10 @@ static int build_generic_tables(const cx_game_desc* d, const int* order, CxGenHe
             ((uint32_t)((H->slot_dr[dslot][a] + R) % R) << 16) | (uint32_t)((H->slot_dc[dslot][a] + C) % C);
     }
     H->fast_loop = (simple && H->direct && cells <= 496 && H->n_masks <= 2) ? 1 : 0;
-    if (const char* dbg = getenv("CX_GEN_FASTLOOP")) H->fast_loop = H->fast_loop && atoi(dbg) != 0;  // development knob
   }
   // envs per warp: one plane tile of at most 8 KB per warp keeps >= 20 warps per SM resident
   int tile = 32;
   while (tile > 1 && (size_t)tile * cells > 8 * 1024) tile >>= 1;
-  if (const char* dbg = getenv("CX_GEN_TILE")) {  // development knob
-    const int v = atoi(dbg);
-    if (v == 1 || v == 2 || v == 4 || v == 8 || v == 16 || v == 32) tile = v;
-  }
-  while (tile > 1 && (size_t)tile * cells > 96 * 1024) tile >>= 1;
   H->tile_envs = tile;
   B->pad();
   H->blob_bytes = (int32_t)B->bytes.size();
@@ -977,12 +963,34 @@ extern "C" int cx_render(const cx_game* g, const void* d_state, int64_t n, uint8
   return cx_launch_render(g, d_state, n, d_board, (cudaStream_t)stream);
 }
 
-// CX_AGENT_STEP_FLAT=0 (development knob) sends single steps through the tile kernels again
-static int step_composer_mode() {   // 0: never, 1: where it is faster (default), 2: at any batch size
-  const char* e = getenv("CX_AGENT_STEP_FLAT");   // read per call: tests flip it to compare the two routes
-  return e ? atoi(e) : 1;
+// The kernel route the environment variable CX_ROUTE forces (see CxRoute); unset or empty: automatic selection.  Read
+// per call, so that one process (a test) can run the same inputs through every kernel.  An unknown name fails the call.
+static int parse_route(CxRoute* route, const char* who) {
+  static const struct {
+    const char* name;
+    CxRoute route;
+  } kRoutes[] = {{"tile64", CX_ROUTE_TILE64},
+                 {"tile128", CX_ROUTE_TILE128},
+                 {"tile256", CX_ROUTE_TILE256},
+                 {"lane", CX_ROUTE_LANE},
+                 {"obs", CX_ROUTE_OBS},
+                 {"no_step_composer", CX_ROUTE_NO_STEP_COMPOSER},
+                 {"step_composer", CX_ROUTE_STEP_COMPOSER},
+                 {"gen96", CX_ROUTE_GEN96},
+                 {"gen80", CX_ROUTE_GEN80},
+                 {"gen_wave", CX_ROUTE_GEN_WAVE}};
+  *route = CX_ROUTE_AUTO;
+  const char* e = getenv("CX_ROUTE");
+  if (!e || !*e) return CX_OK;
+  for (const auto& r : kRoutes)
+    if (strcmp(e, r.name) == 0) {
+      *route = r.route;
+      return CX_OK;
+    }
+  cx_set_error("%s: unknown CX_ROUTE '%s' (tile64, tile128, tile256, lane, obs, no_step_composer, step_composer, "
+               "gen96, gen80, gen_wave)", who, e);
+  return CX_ERR_INVALID_ARG;
 }
-static bool step_composer_enabled() { return step_composer_mode() != 0; }
 
 static int rollout_common(const cx_game* g, void* d_state, int64_t n, int32_t T, const uint8_t* d_actions,
                           const CxSynth& synth, float* d_reward, float* d_discount, uint8_t* d_flags,
@@ -1001,28 +1009,33 @@ static int rollout_common(const cx_game* g, void* d_state, int64_t n, int32_t T,
     cx_set_error("%s: env_offset must be a multiple of 4", who);
     return CX_ERR_INVALID_ARG;
   }
+  CxRoute route;
+  rc = parse_route(&route, who);
+  if (rc) return rc;
   // one step of a small batch: the stateless composer (cx_agent_step_kernels.cu) -- 2.5 against 3.1 us at 4,096 envs,
   // equal at 65,536; large batches amortise the tile staging over enough envs (2^20: 11 us against 28 us)
-  if (g->path == CX_PATH_AGENT && T == 1 && !synth.on && (n < 65536 || step_composer_mode() == 2) &&
-      step_composer_enabled() &&
-      cx_agent_step_applies(g, d_board, nullptr))
+  if (g->path == CX_PATH_AGENT && T == 1 && !synth.on && (n < 65536 || route == CX_ROUTE_STEP_COMPOSER) &&
+      route != CX_ROUTE_NO_STEP_COMPOSER && cx_agent_step_applies(g, d_board, nullptr))
     return cx_launch_agent_step(g, d_state, n, d_actions, d_reward, d_discount, d_flags, d_board, nullptr, CX_DTYPE_U8,
                                 (cudaStream_t)stream);
   if (g->path == CX_PATH_AGENT) {
+    const bool tile = route == CX_ROUTE_TILE64 || route == CX_ROUTE_TILE128 || route == CX_ROUTE_TILE256;
     // Batches below 32,768 envs that k_agent_rollout_lane (next) does not take -- rows that are not 16-byte aligned, i.e.
     // n not a multiple of 16 -- run on the lane-per-env TMA kernel, which handles ragged warps and unaligned buffers and
     // is a little faster there than the scalar path of k_agent_rollout (Demo 1, 32 steps: 4,096 envs 16.6 against 17.9 us).
-    // CX_AGENT_SMALL_N overrides the threshold (0: always k_agent_rollout).
+    // The tile routes send them to k_agent_rollout as well, the obs route sends every batch here.
     int64_t small_n = 32768;
-    if (const char* dbg = getenv("CX_AGENT_SMALL_N")) small_n = atoll(dbg);
+    if (tile) small_n = 0;
+    if (route == CX_ROUTE_OBS) small_n = INT64_MAX;
     // Batches of a multiple of 16 envs up to ~1,800 envs per SM (2^18 on 148 SMs): k_agent_rollout_lane (lane = env, STG.128 tile
     // copies; cx_agent_lane_kernels.cu).  Demo 1, 32-step launches, % of the copy peak against the best tile build:
     // 4,096 envs 7.1 / 3.5, 65,536 56.5 / 49.7, 2^17 80.0 / 77.5, 2^18 90.3 / 90.6, 2^19 89.6 / 91.5, 2^20 86 / 95.
-    // CX_AGENT_LANE_N overrides the threshold (0: never).
+    // The lane route sends every batch it takes here, the tile and obs routes none.
     // Boards above 96 cells: only tiny batches (its tile copy is 2 * cells / 32 LDS.128 + STG.128 pairs per lane and
     // step, one bulk store in the TMA kernels: random 15x16 maze, 65,536 envs 64 against 88 %, 16,384 envs 18 against 36 us).
     int64_t lane_n = (int64_t)g->sm_count * (g->ah.cells <= CX_AGENT_TILE_MAX_CELLS ? 1800 : 200);
-    if (const char* dbg = getenv("CX_AGENT_LANE_N")) lane_n = atoll(dbg);
+    if (tile || route == CX_ROUTE_OBS) lane_n = 0;
+    if (route == CX_ROUTE_LANE) lane_n = INT64_MAX;
     if (n <= lane_n && T > 1 &&
         cx_agent_lane_applies(g, n, d_actions, synth.actions_out, d_reward, d_discount, d_flags, d_board))
       return cx_launch_agent_rollout_lane(g, d_state, n, T, d_actions, synth, d_reward, d_discount, d_flags, d_board,
@@ -1030,10 +1043,10 @@ static int rollout_common(const cx_game* g, void* d_state, int64_t n, int32_t T,
     if (g->ah.cells > CX_AGENT_TILE_MAX_CELLS || n < small_n)  // large boards, small batches: lane-per-env kernel, board only
       return cx_launch_agent_rollout_obs(g, d_state, n, T, d_actions, synth, d_reward, d_discount, d_flags, d_board,
                                          nullptr, (cudaStream_t)stream);
-    return cx_launch_agent_rollout(g, d_state, n, T, d_actions, synth, d_reward, d_discount, d_flags, d_board,
+    return cx_launch_agent_rollout(g, d_state, n, T, d_actions, synth, d_reward, d_discount, d_flags, d_board, route,
                                    (cudaStream_t)stream);
   }
-  return cx_launch_generic_rollout(g, d_state, n, T, d_actions, synth, d_reward, d_discount, d_flags, d_board,
+  return cx_launch_generic_rollout(g, d_state, n, T, d_actions, synth, d_reward, d_discount, d_flags, d_board, route,
                                    (cudaStream_t)stream);
 }
 
@@ -1065,15 +1078,18 @@ extern "C" int cx_rollout_observations(const cx_game* g, void* d_state, int64_t 
     cx_set_error("cx_rollout_observations: layered must not be NULL");
     return CX_ERR_INVALID_ARG;
   }
-  if (g && d_actions && d_reward && d_flags && d_board && T == 1 && step_composer_enabled() &&
+  CxRoute route;
+  int rc = parse_route(&route, "cx_rollout_observations");
+  if (rc) return rc;
+  if (g && d_actions && d_reward && d_flags && d_board && T == 1 && route != CX_ROUTE_NO_STEP_COMPOSER &&
       cx_agent_step_applies(g, d_board, d_layered)) {
-    int rc = check_common(g, d_state, n, "cx_rollout_observations");
+    rc = check_common(g, d_state, n, "cx_rollout_observations");
     if (rc) return rc;
     return cx_launch_agent_step(g, d_state, n, d_actions, d_reward, d_discount, d_flags, d_board, d_layered,
                                 CX_DTYPE_U8, (cudaStream_t)stream);
   }
   if (g && d_actions && d_reward && d_flags && d_board && T >= 1 && cx_agent_obs_applies(g, true)) {
-    int rc = check_common(g, d_state, n, "cx_rollout_observations");
+    rc = check_common(g, d_state, n, "cx_rollout_observations");
     if (rc) return rc;
     CxSynth none;
     memset(&none, 0, sizeof(none));
@@ -1083,19 +1099,19 @@ extern "C" int cx_rollout_observations(const cx_game* g, void* d_state, int64_t 
   if (g && g->desc.unoccluded_layers) {
     if (g->path == CX_PATH_GENERIC && d_actions && d_reward && d_flags && d_board && T >= 1) {
       // generic games: the kernel reads the unoccluded layers off its entity state at every step
-      int rc = check_common(g, d_state, n, "cx_rollout_observations");
+      rc = check_common(g, d_state, n, "cx_rollout_observations");
       if (rc) return rc;
       CxSynth none;
       memset(&none, 0, sizeof(none));
       return cx_launch_generic_rollout(g, d_state, n, T, d_actions, none, d_reward, d_discount, d_flags, d_board,
-                                       (cudaStream_t)stream, d_layered);
+                                       route, (cudaStream_t)stream, d_layered);
     }
     cx_set_error("cx_rollout_observations: unoccluded layers need the fused kernels (16-byte aligned buffers, "
                  "boards that fit the lane-per-env kernel)");
     return CX_ERR_UNSUPPORTED;
   }
   // any other game or geometry: the step kernel, then the layers from the finished boards
-  int rc = cx_rollout(g, d_state, n, T, d_actions, d_reward, d_discount, d_flags, d_board, stream);
+  rc = cx_rollout(g, d_state, n, T, d_actions, d_reward, d_discount, d_flags, d_board, stream);
   if (rc) return rc;
   return cx_layers_from_board(g, d_board, (int64_t)T * n, d_layered, stream);
 }
@@ -1133,7 +1149,10 @@ extern "C" int cx_step_observations(const cx_game* g, void* d_state, int64_t n, 
     cx_set_error("cx_step_observations: unknown layered_dtype %d", dtype);
     return CX_ERR_INVALID_ARG;
   }
-  if (step_composer_enabled() && cx_agent_step_applies(g, d_board, d_layered))
+  CxRoute route;
+  rc = parse_route(&route, "cx_step_observations");
+  if (rc) return rc;
+  if (route != CX_ROUTE_NO_STEP_COMPOSER && cx_agent_step_applies(g, d_board, d_layered))
     return cx_launch_agent_step(g, d_state, n, d_actions, d_reward, d_discount, d_flags, d_board, d_layered, dtype,
                                 (cudaStream_t)stream);
   if (dtype == CX_DTYPE_U8)

@@ -43,27 +43,10 @@
 
 namespace {
 
-#ifndef CX_GEN_UNROLL
-#define CX_GEN_UNROLL 2   // chunks of the composer loop in flight per lane (ILP)
-#endif
-#ifndef CX_GEN_MIN_CTAS
-#define CX_GEN_MIN_CTAS 5  // resident CTAs per SM the register allocation aims for (5 x 128 threads x 96 registers); the
-                           // register-state kernel is also built for one CTA more, see cx_launch_generic_rollout
-#endif
-#ifndef CX_GEN_STHINT
-#define CX_GEN_STHINT 0    // board chunk stores of the flat composer: 0 default policy, 1 L2 evict-first hint, 2 evict-last... (probe)
-#endif
-#ifndef CX_GEN_CTASYNC
-#define CX_GEN_CTASYNC 0   // register-state kernel: the CTA's warps meet at a named barrier before every step (probe)
-#endif
-#ifndef CX_GEN_PROBE
-#define CX_GEN_PROBE 0
-#endif
-constexpr int kChunkUnroll = CX_GEN_UNROLL;
-#ifndef CX_GEN_FLAT_UNROLL
-#define CX_GEN_FLAT_UNROLL 5   // 512-byte groups of the flat composer in flight per warp
-#endif
-constexpr int kFlatUnroll = CX_GEN_FLAT_UNROLL;
+constexpr int kChunkUnroll = 2;  // chunks of the composer loop in flight per lane (ILP)
+constexpr int kMinCtas = 5;      // resident CTAs per SM the register allocation aims for (5 x 128 threads x 96 registers);
+                                 // the register-state kernel is also built for one CTA more, see cx_launch_generic_rollout
+constexpr int kFlatUnroll = 5;   // 512-byte groups of the flat composer in flight per warp
 constexpr int NT = CX_GEN_CTA_THREADS;
 constexpr int kWaveThreads = 448;  // fat CTAs of the one-wave build: 2 x 448 threads x 72 registers per SM
 
@@ -708,16 +691,6 @@ __device__ __forceinline__ void compose_direct_flat(const Ctx& X, const WarpMem&
   }
   const uint32_t nchunks = (uint32_t)nenv * cells >> 4;     // the tile holds whole chunks (gen_vec_ok)
   const uint32_t inv_cells = div_inverse(cells);
-#if CX_GEN_STHINT
-  uint64_t l2pol;
-#if CX_GEN_STHINT == 1
-  asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(l2pol));
-#elif CX_GEN_STHINT == 2
-  asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(l2pol));
-#else
-  asm volatile("createpolicy.fractional.L2::evict_unchanged.b64 %0, 1.0;" : "=l"(l2pol));
-#endif
-#endif
 #pragma unroll U
   for (uint32_t c0 = 0; c0 < nchunks; c0 += 32) {
     const uint32_t c = c0 + lane;
@@ -733,14 +706,7 @@ __device__ __forceinline__ void compose_direct_flat(const Ctx& X, const WarpMem&
       m.rot = q & 0xFFFu;
       overlay16(v, direct_slice(m, o, cells), ch4[i]);
     }
-#if CX_GEN_STHINT
-    if (valid && o + 16u <= cells)
-      asm volatile("st.global.L2::cache_hint.v4.b32 [%0], {%1, %2, %3, %4}, %5;" ::"l"(d16 + c), "r"(v.x), "r"(v.y),
-                   "r"(v.z), "r"(v.w), "l"(l2pol)
-                   : "memory");
-#else
     if (valid && o + 16u <= cells) d16[c] = v;  // default policy: measured 3 % faster than st.global.cs here
-#endif
   }
   // the chunk across the boundary between env i-1 and env i (lane i), if there is one
   if ((cells & 15u) != 0) {
@@ -902,7 +868,7 @@ __device__ __forceinline__ void compose_warp(const Ctx& X, const WarpMem& W, int
       __syncwarp();
     }
     compose_direct<U>(X, W, nenv, dst, lane);
-    if (H.n_above > 0 && CX_GEN_PROBE != 4) {   // development probe (4: no stores over the finished board)
+    if (H.n_above > 0) {
       __syncwarp();  // orders the chunk stores before the byte stores of other lanes to the same addresses
       if (lane < nenv) store_above(X, W, lane, dst);
     }
@@ -1007,17 +973,10 @@ __global__ void __launch_bounds__(BLK, OCC) k_generic_rollout(const __grid_const
 
   uint32_t a_next = 0;  // this lane's action for the coming step, loaded one step ahead of its use
   if (mine && !P.synth) a_next = P.actions[env0 + lane];
-#if CX_GEN_CTASYNC
-  const int64_t warps_total = (P.n + G - 1) / G;
-  const int active_threads = 32 * (int)min((int64_t)wpc, warps_total - (int64_t)blockIdx.x * wpc);
-#endif
   for (int t = 0; t < P.T; ++t) {
-#if CX_GEN_CTASYNC
-    if (FAST && active_threads > 32) asm volatile("bar.sync 1, %0;" ::"r"(active_threads) : "memory");
-#endif
     const int64_t row = (int64_t)t * P.n + env0;
     bool reset_me = false;
-    if (mine && CX_GEN_PROBE != 3) {  // development probe (3: composition only)
+    if (mine) {
       uint32_t a;
       if (P.synth) {
         a = cx_synth_action(P.seed, P.env_offset + (uint64_t)env, P.t0 + (uint64_t)t, (uint32_t)H.n_actions);
@@ -1034,11 +993,7 @@ __global__ void __launch_bounds__(BLK, OCC) k_generic_rollout(const __grid_const
         f = CX_FLAG_ALREADY_OVER | CX_FLAG_REWARD_NONE;
       } else {
         if (FAST)
-#if CX_GEN_PROBE == 2  // development probe (2: no entity updates)
-          rw = 0.0f, f = 0u, dc = 1.0f;
-#else
           fast_env_step(X, a, sreg, dyn[lane], plane + lane * cells, rw, f, dc);
-#endif
         else if (H.simple_step)
           simple_env_step(X, a, dyn[lane], plane + lane * cells, rw, f, dc);
         else
@@ -1072,9 +1027,7 @@ __global__ void __launch_bounds__(BLK, OCC) k_generic_rollout(const __grid_const
     __syncwarp();  // entity state and backdrop stamps of the warp's envs are visible
 
     // ---- phases 1b, 1c, 2: compose the boards and stream them out ----
-#if CX_GEN_PROBE != 1  // development probe (1: no composition)
     compose_warp<OCC >= 6 ? 3 : kFlatUnroll>(X, W, nenv, P.board + row * cells, fast, lane);
-#endif
     if (P.layered) {  // unoccluded layers of this frame, before any auto reset touches the state
       emit_unoccluded_layers(X, W, nenv, P.layered + row * (int64_t)H.n_chars * cells, lane);
       __syncwarp();
@@ -1204,9 +1157,9 @@ bool gen_vec_ok(const cx_game* g, int64_t n, const void* d_board) {
 int configure_once() {
   static CxPerDevice configured;
   if (configured.need()) {
-    CX_CUDA_OK(cudaFuncSetAttribute(k_generic_rollout<false, NT, CX_GEN_MIN_CTAS>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
-    CX_CUDA_OK(cudaFuncSetAttribute(k_generic_rollout<true, NT, CX_GEN_MIN_CTAS>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
-    CX_CUDA_OK(cudaFuncSetAttribute(k_generic_rollout<true, NT, CX_GEN_MIN_CTAS + 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
+    CX_CUDA_OK(cudaFuncSetAttribute(k_generic_rollout<false, NT, kMinCtas>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
+    CX_CUDA_OK(cudaFuncSetAttribute(k_generic_rollout<true, NT, kMinCtas>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
+    CX_CUDA_OK(cudaFuncSetAttribute(k_generic_rollout<true, NT, kMinCtas + 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
     CX_CUDA_OK(cudaFuncSetAttribute(k_generic_rollout<true, kWaveThreads, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
     // two 112 KB CTAs per SM need the largest shared-memory carveout (a hint the driver would otherwise derive per launch)
     CX_CUDA_OK(cudaFuncSetAttribute(k_generic_rollout<true, kWaveThreads, 2>, cudaFuncAttributePreferredSharedMemoryCarveout,
@@ -1221,7 +1174,7 @@ int configure_once() {
 
 int cx_launch_generic_rollout(const cx_game* g, void* d_state, int64_t n, int32_t T, const uint8_t* d_actions,
                               const CxSynth& synth, float* d_reward, float* d_discount, uint8_t* d_flags,
-                              uint8_t* d_board, cudaStream_t s, uint8_t* d_layered) {
+                              uint8_t* d_board, CxRoute route, cudaStream_t s, uint8_t* d_layered) {
   GenParams P = make_params(g, d_state, n);
   P.actions = d_actions;
   P.synth = synth.on;
@@ -1251,25 +1204,27 @@ int cx_launch_generic_rollout(const cx_game* g, void* d_state, int64_t n, int32_
     //  * a batch that needs slightly more warps per SM than 4-warp CTAs keep resident (Hello World, 65,536 envs: 27.7
     //    against 20-24) would run 1.2-1.4 waves; two fat CTAs per SM (up to 14 warps each, 72 registers) hold it in
     //    ONE wave instead;
-    //  * CX_GEN_MIN_CTAS + 1 resident CTAs per SM (80 registers) once the grid is at least two waves deep;
-    //  * CX_GEN_MIN_CTAS CTAs (96 registers) otherwise.
+    //  * kMinCtas + 1 resident CTAs per SM (80 registers) once the grid is at least two waves deep;
+    //  * kMinCtas CTAs (96 registers) otherwise.
+    // The routes gen96 / gen80 / gen_wave force the 96-register, the 80-register and the one-wave build (the latter with
+    // 14-warp CTAs, as far as they fit shared memory).
     const int64_t per_sm = (warps + g->sm_count - 1) / g->sm_count;
     int fat = (int)((per_sm + 1) / 2);  // warps per CTA with two CTAs per SM
-    int force = 0;                       // development knob: 1 = 5 CTAs x 96 regs, 2 = 6 x 80, 3 = fat CTAs
-    if (const char* dbg = getenv("CX_GEN_BUILD")) force = atoi(dbg);
-    if (force == 3) fat = kWaveThreads / 32;
-    if (force != 1 && force != 2 && (force == 3 || per_sm > (int64_t)wpc * CX_GEN_MIN_CTAS) && fat * 32 <= kWaveThreads &&
+    if (route == CX_ROUTE_GEN_WAVE) fat = kWaveThreads / 32;
+    const bool auto_build = route != CX_ROUTE_GEN96 && route != CX_ROUTE_GEN80 && route != CX_ROUTE_GEN_WAVE;
+    if ((route == CX_ROUTE_GEN_WAVE || (auto_build && per_sm > (int64_t)wpc * kMinCtas)) && fat * 32 <= kWaveThreads &&
         2 * (gen_smem_bytes(g, fat) + 1024 + 512) <= (size_t)g->smem_per_sm) {
       const int64_t fgrid = (warps + fat - 1) / fat;
       k_generic_rollout<true, kWaveThreads, 2><<<(unsigned)fgrid, fat * 32, gen_smem_bytes(g, fat), s>>>(P);
-    } else if (force == 2 || (force != 1 && grid >= 2 * (int64_t)g->sm_count * (CX_GEN_MIN_CTAS + 1))) {
-      k_generic_rollout<true, NT, CX_GEN_MIN_CTAS + 1><<<(unsigned)grid, wpc * 32, gen_smem_bytes(g, wpc), s>>>(P);
+    } else if (route == CX_ROUTE_GEN80 ||
+               (route != CX_ROUTE_GEN96 && grid >= 2 * (int64_t)g->sm_count * (kMinCtas + 1))) {
+      k_generic_rollout<true, NT, kMinCtas + 1><<<(unsigned)grid, wpc * 32, gen_smem_bytes(g, wpc), s>>>(P);
     } else {
-      k_generic_rollout<true, NT, CX_GEN_MIN_CTAS><<<(unsigned)grid, wpc * 32, gen_smem_bytes(g, wpc), s>>>(P);
+      k_generic_rollout<true, NT, kMinCtas><<<(unsigned)grid, wpc * 32, gen_smem_bytes(g, wpc), s>>>(P);
     }
   }
   else
-    k_generic_rollout<false, NT, CX_GEN_MIN_CTAS><<<(unsigned)grid, wpc * 32, gen_smem_bytes(g, wpc), s>>>(P);
+    k_generic_rollout<false, NT, kMinCtas><<<(unsigned)grid, wpc * 32, gen_smem_bytes(g, wpc), s>>>(P);
   CX_CUDA_OK(cudaGetLastError());
   return CX_OK;
 }

@@ -24,9 +24,7 @@
 #define CX_AGENT_CTA_THREADS 128
 
 #define CX_GEN_TILE_ENVS 32      // max envs per CTA in the generic kernels
-#ifndef CX_GEN_CTA_THREADS
 #define CX_GEN_CTA_THREADS 128
-#endif
 #define CX_MAX_DYN 8             // moving entities in the generic path
 #define CX_MAX_LIN 4             // per-env mask bitsets the fast composer keeps in shared memory
 #define CX_MAX_ZDIR_GAME 8       // change_z_order directives of a whole game in one step
@@ -234,10 +232,26 @@ struct CxSynth {
   uint8_t* actions_out;  // [T, n] or null
 };
 
+// A kernel route forced through the environment variable CX_ROUTE (cx_game.cu: parse_route), so that tests can run
+// every kernel on the same inputs.  Anything the forced route does not cover keeps its automatic choice.
+enum CxRoute {
+  CX_ROUTE_AUTO,              // CX_ROUTE unset: automatic selection
+  CX_ROUTE_TILE64,            // tile64 / tile128 / tile256: k_agent_rollout with 64 / 128 / 256 envs per warp at every
+  CX_ROUTE_TILE128,           //   batch size (its ragged rest still runs on k_agent_rollout_lane)
+  CX_ROUTE_TILE256,
+  CX_ROUTE_LANE,              // lane: k_agent_rollout_lane for every rollout it takes, whatever the batch size
+  CX_ROUTE_OBS,               // obs: k_agent_rollout_obs in place of k_agent_rollout_lane and k_agent_rollout
+  CX_ROUTE_NO_STEP_COMPOSER,  // no_step_composer: single steps never take the stateless composer (k_agent_step_flat)
+  CX_ROUTE_STEP_COMPOSER,     // step_composer: single steps take it at any batch size
+  CX_ROUTE_GEN96,             // gen96 / gen80 / gen_wave: the 96-register, 80-register or one-wave build of the
+  CX_ROUTE_GEN80,             //   register-state generic kernel
+  CX_ROUTE_GEN_WAVE,
+};
+
 // kernel launchers (defined in the kernel translation units)
 int cx_launch_agent_rollout(const cx_game* g, void* d_state, int64_t n, int32_t T, const uint8_t* d_actions,
                             const CxSynth& synth, float* d_reward, float* d_discount, uint8_t* d_flags,
-                            uint8_t* d_board, cudaStream_t s);
+                            uint8_t* d_board, CxRoute route, cudaStream_t s);
 int cx_launch_agent_rollout_obs(const cx_game* g, void* d_state, int64_t n, int32_t T, const uint8_t* d_actions,
                                 const CxSynth& synth, float* d_reward, float* d_discount, uint8_t* d_flags,
                                 uint8_t* d_board, uint8_t* d_layered /* or null */, cudaStream_t s);
@@ -264,7 +278,7 @@ int cx_launch_agent_step(const cx_game* g, void* d_state, int64_t n, const uint8
 // unoccluded layers of every frame, read off the entity state inside the kernel
 int cx_launch_generic_rollout(const cx_game* g, void* d_state, int64_t n, int32_t T, const uint8_t* d_actions,
                               const CxSynth& synth, float* d_reward, float* d_discount, uint8_t* d_flags,
-                              uint8_t* d_board, cudaStream_t s, uint8_t* d_layered = nullptr);
+                              uint8_t* d_board, CxRoute route, cudaStream_t s, uint8_t* d_layered = nullptr);
 int cx_launch_reset(const cx_game* g, void* d_state, int64_t n, const uint8_t* d_mask, cudaStream_t s);
 int cx_launch_stats_fold(void* d_state, cudaStream_t s);
 int cx_launch_render(const cx_game* g, const void* d_state, int64_t n, uint8_t* d_board, cudaStream_t s);

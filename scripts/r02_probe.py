@@ -1,5 +1,5 @@
 """Development aid (round 2): single-step latency and small/mid-batch throughput of the single-agent kernels.
-Usage: python scripts/r02_probe.py [step|ring|obs]..."""
+Usage: python scripts/r02_probe.py [step|obs]..."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -30,16 +30,16 @@ def graph_of(fn, k):
 
 def step_probe():
     for n in (4096, 65536, 1 << 20):
-        for flat in ("2", "0"):
-            os.environ["CX_AGENT_STEP_FLAT"] = flat
+        for flat in ("step_composer", "no_step_composer"):
+            os.environ["CX_ROUTE"] = flat
             g = NativeGame(expected_spec("boat_race", max_episode_steps=100, track_returns=True), n)
             nb = max(2, int(300e6 // (n * 31)) + 1)
             bufs = [g.alloc_outputs() for _ in range(nb)]
             acts = g.fill_actions(nb, seed=1)
             gr = graph_of(lambda i: g.step(acts[i % nb], *bufs[i % nb]), nb)
             ms = timed(lambda i: gr.replay(), 1, max(3, int(20 / (nb * 0.01)))) / nb
-            print("cx_step n=%d flat=%s: %.2f us/step  %.1f GB/s" % (n, flat, ms * 1e3, n * 31 / ms / 1e6), flush=True)
-        os.environ["CX_AGENT_STEP_FLAT"] = "1"
+            print("cx_step n=%d %s: %.2f us/step  %.1f GB/s" % (n, flat, ms * 1e3, n * 31 / ms / 1e6), flush=True)
+        os.environ.pop("CX_ROUTE", None)
         for dt in (torch.uint8, torch.float32, torch.bfloat16):
             g = NativeGame(expected_spec("boat_race", max_episode_steps=100, track_returns=True), n)
             es = torch.empty((), dtype=dt).element_size()
@@ -53,55 +53,23 @@ def step_probe():
             print("cx_step_observations n=%d %s: %.2f us/step  %.1f GB/s" % (n, dt, ms * 1e3, n * per / ms / 1e6), flush=True)
 
 
-def ring_probe():
-    T = 32
-    modes = {"tile256": dict(CX_AGENT_LANE_N="0", CX_AGENT_SMALL_N="0", CX_AGENT_WT="256"), "tile128": dict(CX_AGENT_LANE_N="0", CX_AGENT_SMALL_N="0", CX_AGENT_WT="128"),
-             "tile64": dict(CX_AGENT_LANE_N="0", CX_AGENT_SMALL_N="0", CX_AGENT_WT="64"),
-             "lane_ring2": dict(CX_AGENT_LANE_N="0", CX_AGENT_SMALL_N=str(1 << 40), CX_OBS_RING="2"), "stg": dict(CX_AGENT_LANE_N=str(1 << 40)),
-             "auto": dict()}
-    if os.environ.get("PROBE_MODES"):
-        modes = {k: v for k, v in modes.items() if k in os.environ["PROBE_MODES"].split(",")}
-    sizes = [int(x) for x in os.environ.get("PROBE_SIZES", "4096,16384,32768,65536,131072,262144,524288,1048576").split(",")]
-    for world in ("demo1",):
-        for n in sizes:
-            for mode, env in modes.items():
-                for k in ("CX_AGENT_SMALL_N", "CX_AGENT_WT", "CX_OBS_RING", "CX_AGENT_LANE_N"):
-                    os.environ.pop(k, None)
-                os.environ.update(env)
-                g = NativeGame(expected_spec(world, max_episode_steps=100, track_returns=True), n)
-                nb = max(2, int(400e6 // (n * T * 31)) + 1)
-                bufs = [g.alloc_outputs(T) for _ in range(nb)]
-                acts = [g.fill_actions(T, seed=1, t0=i * T) for i in range(nb)]
-                gr = graph_of(lambda i: g.rollout(acts[i % nb], *bufs[i % nb]), nb)
-                ms = timed(lambda i: gr.replay(), 1, max(3, int(30 / (nb * 0.03)))) / nb
-                print("%s n=%d T=%d %s: %.4f ms/launch  %.3e env-steps/s  %.0f GB/s (%.1f%%)" % (
-                    world, n, T, mode, ms, n * T / ms * 1e3, n * T * 31.44 / ms / 1e6, n * T * 31.44 / ms / 1e6 / 65.341), flush=True)
-                del g, bufs, acts, gr
-    for k in ("CX_AGENT_SMALL_N", "CX_AGENT_WT", "CX_OBS_RING", "CX_AGENT_LANE_N"):
-        os.environ.pop(k, None)
-
-
 def obs_probe():
     T = 16
     for n in (4096, 65536, 1 << 18, 1 << 20):
-        for ring in ("1", "2"):
-            os.environ["CX_OBS_RING"] = ring
-            g = NativeGame(expected_spec("boat_race", max_episode_steps=100, track_returns=True), n)
-            nb = max(2, int(400e6 // (n * T * 206)) + 1)
-            bufs = [g.alloc_outputs(T) for _ in range(nb)]
-            lay = [torch.empty((T, n, 7, 5, 5), dtype=torch.uint8, device="cuda") for _ in range(nb)]
-            acts = [g.fill_actions(T, seed=1, t0=i * T) for i in range(nb)]
-            gr = graph_of(lambda i: g.rollout_observations(acts[i % nb], bufs[i % nb][0], lay[i % nb], bufs[i % nb][1], bufs[i % nb][2]), nb)
-            ms = timed(lambda i: gr.replay(), 1, max(3, int(30 / (nb * 0.05)))) / nb
-            print("obs n=%d T=%d ring=%s: %.4f ms/launch  %.0f GB/s (%.1f%%)" % (n, T, ring, ms, n * T * 206 / ms / 1e6, n * T * 206 / ms / 1e6 / 65.341), flush=True)
-            del g, bufs, lay, acts, gr
-    os.environ.pop("CX_OBS_RING", None)
+        g = NativeGame(expected_spec("boat_race", max_episode_steps=100, track_returns=True), n)
+        nb = max(2, int(400e6 // (n * T * 206)) + 1)
+        bufs = [g.alloc_outputs(T) for _ in range(nb)]
+        lay = [torch.empty((T, n, 7, 5, 5), dtype=torch.uint8, device="cuda") for _ in range(nb)]
+        acts = [g.fill_actions(T, seed=1, t0=i * T) for i in range(nb)]
+        gr = graph_of(lambda i: g.rollout_observations(acts[i % nb], bufs[i % nb][0], lay[i % nb], bufs[i % nb][1], bufs[i % nb][2]), nb)
+        ms = timed(lambda i: gr.replay(), 1, max(3, int(30 / (nb * 0.05)))) / nb
+        print("obs n=%d T=%d: %.4f ms/launch  %.0f GB/s (%.1f%%)" % (n, T, ms, n * T * 206 / ms / 1e6, n * T * 206 / ms / 1e6 / 65.341), flush=True)
+        del g, bufs, lay, acts, gr
 
 
 if __name__ == "__main__":
-    what = sys.argv[1:] or ["step", "ring", "obs"]
+    what = sys.argv[1:] or ["step", "obs"]
     if "step" in what: step_probe()
-    if "ring" in what: ring_probe()
     if "obs" in what: obs_probe()
 
 
@@ -137,10 +105,8 @@ if __name__ == "__main__" and "tsweep" in sys.argv[1:]:
 def stg_sweep():
     """Small batches: launch time against steps per launch (slope = per-step time, intercept = fixed cost per launch),
     with and without episode tracking, for the 64-env tile build and the STG lane kernel."""
-    for mode, env in (("tile64", dict(CX_AGENT_LANE_N="0", CX_AGENT_SMALL_N="0", CX_AGENT_WT="64")), ("stg", dict(CX_AGENT_LANE_N=str(1 << 40)))):
-        for k in ("CX_AGENT_SMALL_N", "CX_AGENT_WT", "CX_OBS_RING", "CX_AGENT_LANE_N"):
-            os.environ.pop(k, None)
-        os.environ.update(env)
+    for mode, route in (("tile64", "tile64"), ("stg", "lane")):
+        os.environ["CX_ROUTE"] = route
         for track in (True, False):
             for n in (4096, 65536):
                 for T in (8, 16, 32, 64, 128):
@@ -154,8 +120,7 @@ def stg_sweep():
                     print("%s track=%d n=%d T=%d: %.2f us/launch  %.3f us/step  %.0f GB/s (%.1f%%)" % (
                         mode, track, n, T, ms * 1e3, ms * 1e3 / T, n * T * 31.44 / ms / 1e6, n * T * 31.44 / ms / 1e6 / 65.341), flush=True)
                     del g, bufs, acts, gr
-    for k in ("CX_AGENT_SMALL_N", "CX_AGENT_WT", "CX_OBS_RING", "CX_AGENT_LANE_N"):
-        os.environ.pop(k, None)
+    os.environ.pop("CX_ROUTE", None)
 
 
 if __name__ == "__main__":
@@ -166,14 +131,11 @@ if __name__ == "__main__":
 def big_sweep():
     """Large batches: kernel build x steps per launch (boat_race, the bench workload)."""
     for n in (1 << 19, 1 << 20):
-        for mode, env in (("tile64", dict(CX_AGENT_WT="64")), ("tile128", dict(CX_AGENT_WT="128")), ("tile256", dict(CX_AGENT_WT="256")), ("stg", dict(CX_AGENT_LANE_N=str(1 << 40)))):
+        for mode, route in (("tile64", "tile64"), ("tile128", "tile128"), ("tile256", "tile256"), ("stg", "lane")):
             if os.environ.get("PROBE_MODES") and mode not in os.environ["PROBE_MODES"].split(","):
                 continue
             for T in (12, 16, 20, 24, 32, 48):
-                for k in ("CX_AGENT_SMALL_N", "CX_AGENT_WT", "CX_OBS_RING", "CX_AGENT_LANE_N", "CX_AGENT_SUBT"):
-                    os.environ.pop(k, None)
-                os.environ.update(env)
-                os.environ["CX_AGENT_SUBT"] = "0"
+                os.environ["CX_ROUTE"] = route
                 g = NativeGame(expected_spec("boat_race", max_episode_steps=100, track_returns=True), n)
                 nb = max(2, int(1300e6 // (n * T * 31)) + 1)
                 bufs = [g.alloc_outputs(T) for _ in range(nb)]
@@ -186,8 +148,7 @@ def big_sweep():
                 print("boat_race n=%d T=%d %s: %.4f ms/launch  %.3e env-steps/s  %.0f GB/s (%.1f%%)" % (
                     n, T, mode, ms, n * T / ms * 1e3, alg / ms / 1e6, alg / ms / 1e6 / 65.341), flush=True)
                 del g, bufs, acts
-    for k in ("CX_AGENT_SMALL_N", "CX_AGENT_WT", "CX_OBS_RING", "CX_AGENT_LANE_N", "CX_AGENT_SUBT"):
-        os.environ.pop(k, None)
+    os.environ.pop("CX_ROUTE", None)
 
 
 if __name__ == "__main__":
@@ -195,12 +156,11 @@ if __name__ == "__main__":
 
 
 def lane_knobs():
-    """k_agent_rollout_lane at BASELINE config 1 (Demo 1, 65,536 envs): warps per CTA, steps per launch."""
-    for wpc in (os.environ.get("LANEKNOB_MODES", "1").split(",")):
-        os.environ.pop("CX_AGENT_PDL", None); os.environ.pop("CX_AGENT_LANE_N", None); os.environ.pop("CX_AGENT_SMALL_N", None); os.environ.pop("CX_AGENT_WT", None)
-        if wpc.startswith("wt"): os.environ.update(CX_AGENT_LANE_N="0", CX_AGENT_SMALL_N="0", CX_AGENT_WT=wpc[2:])
-        if wpc.endswith("pdl0"): os.environ["CX_AGENT_PDL"] = "0"
-        if wpc.startswith("tile64"): os.environ.update(CX_AGENT_LANE_N="0", CX_AGENT_SMALL_N="0", CX_AGENT_WT="64")
+    """k_agent_rollout_lane at BASELINE config 1 (Demo 1, 65,536 envs) by batch size and steps per launch, against the
+    routes LANEKNOB_MODES names (auto or CX_ROUTE values, e.g. auto,tile64)."""
+    for mode in (os.environ.get("LANEKNOB_MODES", "auto").split(",")):
+        os.environ.pop("CX_ROUTE", None)
+        if mode != "auto": os.environ["CX_ROUTE"] = mode
         for n in [int(x) for x in os.environ.get("LANEKNOB_SIZES", "4096,16384,32768,65536,131072,262144").split(",")]:
             for T in (32, 100):
                 g = NativeGame(expected_spec("demo1", max_episode_steps=100, track_returns=True), n)
@@ -212,9 +172,9 @@ def lane_knobs():
                 timed(lambda i: gr.replay(), 0, max(3, int(100 / per)))
                 ms = timed(lambda i: gr.replay(), 1, max(6, int(60 / per))) / max(nb, 8)
                 alg = n * (T * 31 + 14)
-                print("lane wpc=%s n=%d T=%d: %.2f us/launch  %.0f GB/s (%.1f%%)" % (wpc, n, T, ms * 1e3, alg / ms / 1e6, alg / ms / 1e6 / 65.341), flush=True)
+                print("lane %s n=%d T=%d: %.2f us/launch  %.0f GB/s (%.1f%%)" % (mode, n, T, ms * 1e3, alg / ms / 1e6, alg / ms / 1e6 / 65.341), flush=True)
                 del g, bufs, acts, gr
-    for k in ("CX_AGENT_PDL", "CX_AGENT_LANE_N", "CX_AGENT_SMALL_N", "CX_AGENT_WT"): os.environ.pop(k, None)
+    os.environ.pop("CX_ROUTE", None)
 
 
 if __name__ == "__main__":
@@ -224,12 +184,9 @@ if __name__ == "__main__":
 def t_small():
     """Large batches, few steps per launch: which tile build?"""
     for n in (1 << 19, 1 << 20):
-        for mode, env in (("tile64", dict(CX_AGENT_WT="64")), ("tile128", dict(CX_AGENT_WT="128")), ("tile256", dict(CX_AGENT_WT="256"))):
+        for mode in ("tile64", "tile128", "tile256"):   # single steps of these batches skip the step composer
             for T in (1, 2, 4, 8):
-                for k in ("CX_AGENT_SMALL_N", "CX_AGENT_WT", "CX_AGENT_LANE_N", "CX_AGENT_STEP_FLAT"):
-                    os.environ.pop(k, None)
-                os.environ.update(env)
-                os.environ["CX_AGENT_STEP_FLAT"] = "0"
+                os.environ["CX_ROUTE"] = mode
                 g = NativeGame(expected_spec("boat_race", max_episode_steps=100, track_returns=True), n)
                 nb = max(2, int(400e6 // (n * T * 31)) + 1)
                 bufs = [g.alloc_outputs(T) for _ in range(nb)]
@@ -240,8 +197,7 @@ def t_small():
                 alg = n * (T * 31 + 14)
                 print("boat_race n=%d T=%d %s: %.2f us/launch  %.0f GB/s (%.1f%%)" % (n, T, mode, ms * 1e3, alg / ms / 1e6, alg / ms / 1e6 / 65.341), flush=True)
                 del g, bufs, acts, gr
-    for k in ("CX_AGENT_SMALL_N", "CX_AGENT_WT", "CX_AGENT_LANE_N", "CX_AGENT_STEP_FLAT"):
-        os.environ.pop(k, None)
+    os.environ.pop("CX_ROUTE", None)
 
 
 if __name__ == "__main__":

@@ -1,4 +1,5 @@
-"""Development aid: k_agent_rollout (256 envs per warp) against the lane-per-env kernel (CX_AGENT_SMALL_N) by batch size."""
+"""Development aid: k_agent_rollout (256 envs per warp) against the lane-per-env kernel by batch size: run it under
+CX_ROUTE=tile256 and CX_ROUTE=obs."""
 import sys, os
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from scripts.quick_time import run

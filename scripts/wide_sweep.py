@@ -1,5 +1,6 @@
-"""Development aid: single-agent worlds of several board sizes by batch size and kernel route (stg = k_agent_rollout_lane,
-tma = lane-per-env TMA kernel / tile builds with CX_AGENT_LANE_N=0)."""
+"""Development aid: single-agent worlds of several board sizes by batch size and kernel route (CX_ROUTE: lane =
+k_agent_rollout_lane, obs = lane-per-env TMA kernel, tile64 = k_agent_rollout; boards above 96 cells run on the obs
+kernel under tile64 as well)."""
 import sys, os
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
@@ -10,9 +11,7 @@ from examples.worlds import Walker
 from tests.test_gpu_generic_worlds import _random_art
 
 def run(rows, cols, n, T, route):
-    os.environ.pop("CX_AGENT_LANE_N", None)
-    if route == "stg": os.environ["CX_AGENT_LANE_N"] = str(1 << 40)
-    if route == "tma": os.environ["CX_AGENT_LANE_N"] = "0"
+    os.environ["CX_ROUTE"] = route
     art = _random_art(np.random.Generator(np.random.PCG64(rows * cols)), rows, cols, 0.2, 0.2)
     game = ascii_art_to_game(art, ' ', drapes={'A': Partial(Walker, walls='#', treasures='*'),
                                                '#': things.FixedDrape, '*': things.FixedDrape},
@@ -39,5 +38,5 @@ def run(rows, cols, n, T, route):
 if __name__ == "__main__":
     for rows, cols in ((5, 5), (8, 12), (10, 12), (15, 16)):
         for n in (16384, 65536, 1 << 18, 1 << 20):
-            for route in ("stg", "tma"):
+            for route in ("lane", "obs", "tile64"):
                 run(rows, cols, n, 16, route)

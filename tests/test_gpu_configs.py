@@ -143,19 +143,19 @@ def test_one_wave_build_matches_the_standard_build(n):
 
 def test_register_state_kernel_builds_agree(monkeypatch):
     """The three builds of the register-state generic kernel (5 CTAs x 96 registers, 6 x 80, two fat CTAs x 72) are the
-    same source under different launch bounds; cx_launch_generic_rollout picks one by batch size.  Forced through the
-    development knob CX_GEN_BUILD they must produce identical rollouts and final states."""
+    same source under different launch bounds; cx_launch_generic_rollout picks one by batch size.  Forced through
+    CX_ROUTE=gen96 / gen80 / gen_wave they must produce identical rollouts and final states."""
     n, T = 1024, 40
     results = []
-    for build in ("1", "2", "3"):
-        monkeypatch.setenv("CX_GEN_BUILD", build)
+    for build in ("gen96", "gen80", "gen_wave"):
+        monkeypatch.setenv("CX_ROUTE", build)
         game = make_world("hello", num_envs=n, max_episode_steps=11, track_returns=True, verify=False)
         game.its_showtime()
         acts = game.native.fill_actions(T, seed=5)
         boards, rewards, discounts, flags = game.rollout(acts)
         game.native.fold_stats()   # partial statistics blocks follow the launch geometry
         results.append((boards.clone(), rewards.clone(), flags.clone(), game.native.state.clone(), game.episode_stats()))
-    monkeypatch.delenv("CX_GEN_BUILD")
+    monkeypatch.delenv("CX_ROUTE")
     for other in results[1:]:
         for x, y in zip(results[0][:4], other[:4]):
             assert torch.equal(x, y)

@@ -137,23 +137,15 @@ def test_hidden_sprite_behind_the_first_drape_stops_stamping():
 
 
 @pytest.mark.parametrize("world", O.GOAL_WORLDS)
-@pytest.mark.parametrize("route", ["auto", "wt64", "wt128", "lane", "stg", "tiles_for_single_steps"])
+@pytest.mark.parametrize("route", ["auto", "wt64", "wt128", "obs", "stg", "tiles_for_single_steps"])
 def test_reach_the_goal_worlds(golden_dir, world, route, monkeypatch):
     """terminate_episode that depends on the cell the agent reached (ADVICE r1): reference-recorded episodes as envs
     of a fused rollout, then random rollouts with auto reset against the oracle, step-by-step play() included.
     `goal` is a single-agent game (transition table with per-cell termination and discount, every kernel build),
     `goal2` runs on the generic kernels (directives replayed per step in update order)."""
-    if route.startswith("wt"):
-        monkeypatch.setenv("CX_AGENT_LANE_N", "0")
-        monkeypatch.setenv("CX_AGENT_SMALL_N", "0")
-        monkeypatch.setenv("CX_AGENT_WT", route[2:])
-    elif route == "lane":
-        monkeypatch.setenv("CX_AGENT_LANE_N", "0")
-        monkeypatch.setenv("CX_AGENT_SMALL_N", str(1 << 40))
-    elif route == "stg":
-        monkeypatch.setenv("CX_AGENT_LANE_N", str(1 << 40))
-    elif route == "tiles_for_single_steps":
-        monkeypatch.setenv("CX_AGENT_STEP_FLAT", "0")
+    if route != "auto":
+        monkeypatch.setenv("CX_ROUTE", {"wt64": "tile64", "wt128": "tile128", "obs": "obs", "stg": "lane",
+                                        "tiles_for_single_steps": "no_step_composer"}[route])
     with open(os.path.join(golden_dir, "generality_" + world + ".json")) as f:
         eps = json.load(f)["episodes"]
     T = max(len(e["actions"]) for e in eps)

@@ -17,17 +17,16 @@ WORLDS = ["boat_race", "demo1", "demo2", "demo3", "demo4", "hello"]
 
 @pytest.fixture(autouse=True, params=["auto", "wt64", "wt128", "wt256", "stg"])
 def agent_kernel(request, monkeypatch):
-    """Single-agent worlds run on several kernels: tiny batches take the lane-per-env kernel (cx_rollout's default),
-    larger ones k_agent_rollout in one of three builds (64 / 128 / 256 envs per warp; 256 is the bench kernel), single
-    steps the stateless composer.  Every test of this module runs on all of them: CX_AGENT_SMALL_N=0 sends small
-    batches to k_agent_rollout as well and CX_AGENT_WT picks its build; "stg" sends every batch of whole warps to the
-    small-batch kernel (k_agent_rollout_lane: lane = env, STG.128 tile copies)."""
+    """Single-agent worlds run on several kernels: tiny batches take the lane-per-env kernels (cx_rollout's default),
+    larger ones k_agent_rollout in one of three builds (64 / 128 / 256 envs per warp; 64 is what large multi-step
+    rollouts take), single steps the stateless composer.  Every test of this module runs on all of them:
+    CX_ROUTE=tile64 / tile128 / tile256 sends small batches to k_agent_rollout as well, in that build; "stg"
+    (CX_ROUTE=lane) sends every batch of whole warps to the small-batch kernel (k_agent_rollout_lane: lane = env,
+    STG.128 tile copies)."""
     if request.param == "stg":
-        monkeypatch.setenv("CX_AGENT_LANE_N", str(1 << 40))
+        monkeypatch.setenv("CX_ROUTE", "lane")
     elif request.param != "auto":
-        monkeypatch.setenv("CX_AGENT_LANE_N", "0")
-        monkeypatch.setenv("CX_AGENT_SMALL_N", "0")
-        monkeypatch.setenv("CX_AGENT_WT", request.param[2:])
+        monkeypatch.setenv("CX_ROUTE", "tile" + request.param[2:])
     return request.param
 
 

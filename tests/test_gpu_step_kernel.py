@@ -1,8 +1,8 @@
 """GPU parity of the single-step composer (`k_agent_step_flat`: cx_step / cx_step_observations on single-agent
 games) and of `cx_sample_actions`.
 
-The composer must agree with (a) the tile kernels it replaces for T = 1 (`CX_AGENT_STEP_FLAT=0` routes single steps
-through them again), (b) `cx_layers_from_board[_f32]` on the board it wrote, for every element type, ragged batch
+The composer must agree with (a) the tile kernels it replaces for T = 1 (`CX_ROUTE=no_step_composer` routes single
+steps through them again), (b) `cx_layers_from_board[_f32]` on the board it wrote, for every element type, ragged batch
 sizes included, and (c) the CPU oracle.  The reference encoding of the float planes is
 `board.layered_board.view(-1).float()` (examples/actor_critic.py:147,173)."""
 import numpy as np
@@ -40,15 +40,27 @@ def test_single_step_composer_equals_tile_kernels(world, n, kw, monkeypatch):
     acts[3, ::7] = 9                                                    # a few actions outside the action set
     oa, ob = a.alloc_outputs(discount=True), b.alloc_outputs(discount=True)
     for t in range(T):
-        monkeypatch.setenv("CX_AGENT_STEP_FLAT", "1")
+        monkeypatch.delenv("CX_ROUTE", raising=False)
         a.step(acts[t].contiguous(), *oa)
-        monkeypatch.setenv("CX_AGENT_STEP_FLAT", "0")
+        monkeypatch.setenv("CX_ROUTE", "no_step_composer")
         b.step(acts[t].contiguous(), *ob)
         for x, y, what in zip(oa, ob, ("board", "reward", "flags", "discount")):
             assert torch.equal(x, y), (world, n, t, what)
     a.fold_stats(), b.fold_stats()
     assert torch.equal(a.state, b.state)
     assert a.stats() == b.stats()
+
+
+def test_unknown_route_fails_the_call(monkeypatch):
+    """CX_ROUTE names one kernel route; a name it does not know fails the call instead of running the automatic
+    choice."""
+    g = _game("boat_race", 64)
+    acts = g.fill_actions(4, seed=1)
+    monkeypatch.setenv("CX_ROUTE", "tile32")
+    with pytest.raises(ValueError, match="unknown CX_ROUTE 'tile32'"):
+        g.step(acts[0].contiguous(), *g.alloc_outputs())
+    with pytest.raises(ValueError, match="unknown CX_ROUTE 'tile32'"):
+        g.rollout(acts, *g.alloc_outputs(4))
 
 
 @pytest.mark.parametrize("world", AGENT_WORLDS)
