@@ -7,7 +7,7 @@ compute entry point is needed, this module raises.  The library is built in-tree
 import ctypes
 import os
 
-CX_ABI_VERSION = 4
+CX_ABI_VERSION = 5
 CX_MAX_ENTITIES = 16
 CX_MAX_ACTIONS = 8
 CX_MAX_CHARS = 32
@@ -128,6 +128,7 @@ PROTOTYPES = {
     "cx_step_observations": (ctypes.c_int, [_P, _P, _I64, _P, _P, _P, _P, _P, _P, _I32, _P]),
     "cx_sample_actions": (ctypes.c_int, [_P, _I64, _I32, _I32, _U64, _U64, _P, _U64, _P, _P, _P]),
     "cx_policy_sample": (ctypes.c_int, [_P, _I64, _I32, _P, _P, _I32, _P, _P, _I32, _U64, _U64, _P, _U64, _P, _P, _P, _P]),
+    "cx_policy_sample_board": (ctypes.c_int, [_P, _P, _I64, _P, _P, _I32, _P, _P, _U64, _U64, _P, _U64, _P, _P, _P, _P]),
     "cx_rollout_policy": (ctypes.c_int, [_P, _P, _I64, _I32, _P, _P, _I32, _P, _P, _U64, _U64, _P, _U64, _P, _P, _P, _P, _P, _P]),
     "cx_layers_from_board": (ctypes.c_int, [_P, _P, _I64, _P, _P]),
     "cx_layers_from_board_f32": (ctypes.c_int, [_P, _P, _I64, _P, _P]),

@@ -176,6 +176,84 @@ __device__ __forceinline__ void policy_hidden_shares_layered(const float* s_w, c
   }
 }
 
+// The same hidden layer with the input given as the uint8 BOARD of env `lane` (s_b: its cells, 4-byte aligned, padded to
+// whole words): input k * cells + c is (board[c] == chars[k]) (campx/rendering.py:204-215), so the planes are never
+// materialised.  Inputs are visited in ascending order, channel-major, each with fmaf(w, x, acc) and x in {0, 1} -- the
+// instruction sequence of policy_hidden_shares on the expanded planes, hence its bits.  The four cells of a board word
+// are compared at once (__vcmpeq4); row(d) returns this warp's float4 slice of row d of W1^T (shared or global memory).
+template <class RowLoad>
+__device__ __forceinline__ void policy_hidden_shares_board(const uint8_t* s_b, const uint8_t* __restrict__ chars, int n_chars,
+                                                           int cells, const RowLoad& row, float* s_h, int A,
+                                                           const PolicyRegs& R, int warp, int lane) {
+  float acc[4];
+#pragma unroll
+  for (int u = 0; u < 4; ++u) acc[u] = __shfl_sync(0xffffffffu, R.b1r, u);
+  const uint32_t* bw = reinterpret_cast<const uint32_t*>(s_b);
+  const int words = cells >> 2;
+  auto term = [&](int d, bool on) {
+    const float4 wa = row(d);
+    const float xv = on ? 1.0f : 0.0f;
+    acc[0] = fmaf(wa.x, xv, acc[0]);
+    acc[1] = fmaf(wa.y, xv, acc[1]);
+    acc[2] = fmaf(wa.z, xv, acc[2]);
+    acc[3] = fmaf(wa.w, xv, acc[3]);
+  };
+  for (int k = 0; k < n_chars; ++k) {
+    const uint32_t ch = __ldg(chars + k), pat = ch * 0x01010101u;
+    const int base = k * cells;
+#pragma unroll 2
+    for (int q = 0; q < words; ++q) {
+      const uint32_t m = __vcmpeq4(bw[q], pat);                // 0xFF in every byte that shows chars[k]
+#pragma unroll
+      for (int u = 0; u < 4; ++u) term(base + 4 * q + u, (m >> (8 * u)) & 1u);
+    }
+    for (int c = words * 4; c < cells; ++c) term(base + c, s_b[c] == ch);
+  }
+#pragma unroll
+  for (int u = 0; u < 4; ++u) acc[u] = fmaxf(acc[u], 0.0f);                               // relu(affine1(x))
+#pragma unroll
+  for (int a = 0; a < CX_MAX_ACTIONS; ++a) {
+    if (a < A) {                                                                          // warp-uniform
+      const float c0 = __shfl_sync(0xffffffffu, R.w2r.x, a), c1 = __shfl_sync(0xffffffffu, R.w2r.y, a);
+      const float c2 = __shfl_sync(0xffffffffu, R.w2r.z, a), c3 = __shfl_sync(0xffffffffu, R.w2r.w, a);
+      s_h[(warp * CX_MAX_ACTIONS + a) * POLICY_PITCH + lane] = fmaf(c3, acc[3], fmaf(c2, acc[2], fmaf(c1, acc[1], c0 * acc[0])));
+    }
+  }
+}
+
+// The same hidden layer visiting only the SET inputs of env `lane`: s_list[i * 32] (i < count) are their input indices in
+// ascending order -- at most one per cell, fewer where a byte is no character of the game -- and row(d) returns this
+// warp's float4 slice of row d of W1^T.  The loop runs to the warp's largest count; a lane past its own adds
+// fmaf(w, 0, acc).  Skipped inputs are 0 and fmaf(w, 0, acc) == acc, so the result has the bits of policy_hidden_shares
+// on the expanded planes (as in policy_hidden_shares_layered).
+template <class RowLoad>
+__device__ __forceinline__ void policy_hidden_shares_list(const uint32_t* s_list, int count, int max_count, const RowLoad& row,
+                                                          float* s_h, int A, const PolicyRegs& R, int warp, int lane) {
+  float acc[4];
+#pragma unroll
+  for (int u = 0; u < 4; ++u) acc[u] = __shfl_sync(0xffffffffu, R.b1r, u);
+#pragma unroll 4
+  for (int i = 0; i < max_count; ++i) {
+    const bool on = i < count;
+    const float4 wa = row(on ? s_list[i * 32] : 0u);
+    const float xv = on ? 1.0f : 0.0f;
+    acc[0] = fmaf(wa.x, xv, acc[0]);
+    acc[1] = fmaf(wa.y, xv, acc[1]);
+    acc[2] = fmaf(wa.z, xv, acc[2]);
+    acc[3] = fmaf(wa.w, xv, acc[3]);
+  }
+#pragma unroll
+  for (int u = 0; u < 4; ++u) acc[u] = fmaxf(acc[u], 0.0f);                               // relu(affine1(x))
+#pragma unroll
+  for (int a = 0; a < CX_MAX_ACTIONS; ++a) {
+    if (a < A) {                                                                          // warp-uniform
+      const float c0 = __shfl_sync(0xffffffffu, R.w2r.x, a), c1 = __shfl_sync(0xffffffffu, R.w2r.y, a);
+      const float c2 = __shfl_sync(0xffffffffu, R.w2r.z, a), c3 = __shfl_sync(0xffffffffu, R.w2r.w, a);
+      s_h[(warp * CX_MAX_ACTIONS + a) * POLICY_PITCH + lane] = fmaf(c3, acc[3], fmaf(c2, acc[2], fmaf(c1, acc[1], c0 * acc[0])));
+    }
+  }
+}
+
 // the eight shares summed in warp order, plus b2: the action logits of env `lane` (call with all 32 lanes of a warp)
 __device__ __forceinline__ void policy_logits(const float* s_h, const PolicyRegs& R, int A, int lane, float (&w)[CX_MAX_ACTIONS]) {
 #pragma unroll

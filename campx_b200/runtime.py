@@ -227,6 +227,38 @@ class NativeGame(object):
                                                _ptr(out), _ptr(logp), _ptr(logits_out), _stream()))
         return out
 
+    def policy_sample_board(self, board, w1t, b1, w2, b2, seed, step=None, step_offset=0, env_offset=0, out=None,
+                            logp=None, logits_out=None):
+        """policy_sample on the layered board of `board` as float32 planes (examples/actor_critic.py:147,173), read off
+        the uint8 board itself: the planes are never written.  board uint8 [num_envs, rows, cols] (e.g. one step of a
+        [T + 1, num_envs, rows, cols] rollout buffer); w1t [n_chars * cells, n_hidden] is affine1.weight TRANSPOSED.
+        Any board size, single-agent and generic games; occluded layers only (NotImplementedError otherwise).  For
+        finite weights: the bits of policy_sample(layers_from_board(board, dtype=float32).view(num_envs, -1), ...)."""
+        n, feat = self.num_envs, self.n_chars * self.cells
+        self._check(board, torch.uint8, (n, self.rows, self.cols), "board")
+        if w1t.dim() != 2:
+            raise ValueError("w1t must be [n_chars * cells, n_hidden]")
+        n_hidden = int(w1t.shape[1])
+        self._check(w1t, torch.float32, (feat, n_hidden), "w1t")
+        self._check(b1, torch.float32, (n_hidden,), "b1")
+        self._check(w2, torch.float32, (self.n_actions, n_hidden), "w2")
+        self._check(b2, torch.float32, (self.n_actions,), "b2")
+        if out is None:
+            out = torch.empty(n, dtype=torch.uint8, device=self.device)
+        self._check(out, torch.uint8, (n,), "actions")
+        if step is not None:
+            self._check(step, torch.int64, (1,), "step")
+        if logp is not None:
+            self._check(logp, torch.float32, (n,), "logp")
+        if logits_out is not None:
+            self._check(logits_out, torch.float32, (n, self.n_actions), "logits_out")
+        with torch.cuda.device(self.device):
+            N.check(self._lib.cx_policy_sample_board(self._handle, _ptr(board), n, _ptr(w1t), _ptr(b1), n_hidden,
+                                                     _ptr(w2), _ptr(b2), int(seed), int(env_offset), _ptr(step),
+                                                     int(step_offset), _ptr(out), _ptr(logp), _ptr(logits_out),
+                                                     _stream()))
+        return out
+
     def rollout_policy(self, n_steps, w1t, b1, w2, b2, seed, states, actions, reward, flags, step=None, step_offset=0,
                        env_offset=0, logp=None):
         """The reference's actor-critic rollout loop (examples/actor_critic.py:146-173) in ONE launch: T times

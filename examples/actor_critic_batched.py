@@ -12,6 +12,10 @@ episode and runs its policy once per step.  Here 4,096 environments step togethe
   returns = cx_discounted_returns over the [T, N] rewards on the device       (actor_critic.py:115-122)
   loss    = -(log pi) * (R - V) + smooth_l1(V, R), Adam                        (actor_critic.py:123-135)
 
+Other worlds (--world hello, ...): where the policy input is larger than cx_policy_sample takes, or the game runs on
+the generic kernels, the rollout stores the uint8 boards instead of float32 planes and the policy reads them directly
+(cx_policy_sample_board); the learner's affine1 is an embedding_bag over the set inputs of each board.
+
 Nothing leaves the device inside an iteration.  The network itself is ordinary torch and is not part of
 the hand-written hot path; the environment, observation encoding and return scan are.
 """
@@ -26,6 +30,7 @@ import torch
 import torch.nn as nn
 import torch.nn.functional as F
 
+from campx_b200 import _native as N
 from examples.worlds import make_world
 
 
@@ -43,6 +48,44 @@ class Policy(nn.Module):
     def action_logits(self, x):
         """The acting half only (no value head, no softmax): what a rollout step needs."""
         return self.action_head(F.relu(self.affine1(x)))
+
+    def forward_indices(self, idx):
+        """forward() on layered boards given by the indices of their set inputs (int [B, cells], board_indices):
+        affine1 is the sum of the W1^T rows of those inputs plus the bias -- the same function as affine1 on the
+        0/1 planes, differentiable in the weight, without the [B, n_inputs] float planes."""
+        w1 = self.affine1.weight
+        w1t = torch.cat([w1.t(), w1.new_zeros(1, w1.shape[0])])            # row n_inputs: "no character"
+        h = F.embedding_bag(idx, w1t, mode="sum", padding_idx=w1.shape[1]) + self.affine1.bias
+        x = F.relu(h)
+        return F.softmax(self.action_head(x), dim=-1), self.value_head(x).squeeze(-1)
+
+
+def board_indices(boards, chars, cells):
+    """uint8 boards [..., rows, cols] -> int32 [..., cells]: the input index k * cells + cell of the one set input of every
+    cell in the layered board (channel k = (board == chars[k]), rendering.py:204-215), or n_chars * cells where the
+    byte is no character of the game."""
+    n_chars = len(chars)
+    lut = torch.full((256,), -1, dtype=torch.int32, device=boards.device)
+    lut[torch.tensor([ord(c) for c in chars], dtype=torch.long, device=boards.device)] = torch.arange(
+        n_chars, dtype=torch.int32, device=boards.device)
+    k = lut[boards.reshape(boards.shape[:-2] + (cells,)).long()]
+    cell = torch.arange(cells, dtype=torch.int32, device=boards.device)
+    return torch.where(k >= 0, k * cells + cell, torch.full_like(k, n_chars * cells))
+
+
+def needs_board_policy(nat):
+    """True where cx_policy_sample cannot run the rollout on float32 planes: the game runs on the generic kernels, or
+    cx_policy_sample refuses the input size (NotImplementedError: the limit is its launcher's, cx_aux_kernels.cu, and
+    is asked rather than restated here -- one launch on zeros)."""
+    if nat.info.path != N.CX_PATH_AGENT:
+        return True
+    feat, n, A = nat.n_chars * nat.cells, nat.num_envs, nat.n_actions
+    zeros = lambda *shape: torch.zeros(shape, dtype=torch.float32, device=nat.device)
+    try:
+        nat.policy_sample(zeros(n, feat), zeros(feat, 32), zeros(32), zeros(A, 32), zeros(A), 0)
+    except NotImplementedError:
+        return True
+    return False
 
 
 def run(num_envs=4096, steps=100, iterations=5, gamma=0.99, lr=3e-2, seed=543, log=print, device="cuda"):
@@ -97,6 +140,12 @@ class GraphedRollout(object):
                                                   board, reward and flags, straight into the rollout buffers
 
     (fused_policy=False keeps the policy in torch: Linear, ReLU, Linear, then cx_sample_actions -- five launches.)
+    Games that need_board_policy() store boards [T + 1, N, rows, cols] uint8 instead of planes, two launches per step:
+
+        cx_policy_sample_board                    the same policy read off the uint8 board of every env
+        cx_step                                   Engine.play() writing the next board straight into the rollout buffer
+
+    (with fused_policy=False: cx_layers_from_board_f32, the torch policy and cx_sample_actions.)
     persistent=True goes one step further: cx_rollout_policy runs the WHOLE T-step loop in one launch (a CTA owns 32 envs,
     their policy input stays in shared memory and changes by four floats per step); bit-identical to the two-launch loop.
 
@@ -109,11 +158,15 @@ class GraphedRollout(object):
         if fused_policy is None:
             fused_policy = policy.affine1.out_features <= 32
         self.fused_policy = bool(fused_policy)
-        self.persistent = bool(persistent) and self.fused_policy and game.num_envs % 32 == 0
         nat = game.native
+        self.board_policy = needs_board_policy(nat)
+        self.persistent = bool(persistent) and self.fused_policy and game.num_envs % 32 == 0 and not self.board_policy
         n, dev = game.num_envs, nat.device
         self.feat = nat.n_chars * nat.cells
-        self._states = torch.empty((self.T + 1, n, self.feat), dtype=torch.float32, device=dev)
+        if self.board_policy:
+            self._states = torch.empty((self.T + 1, n, nat.rows, nat.cols), dtype=torch.uint8, device=dev)
+        else:
+            self._states = torch.empty((self.T + 1, n, self.feat), dtype=torch.float32, device=dev)
         self.actions = torch.empty((self.T, n), dtype=torch.uint8, device=dev)
         self.rewards = torch.empty((self.T, n), dtype=torch.float32, device=dev)
         self.flags = torch.empty((self.T, n), dtype=torch.uint8, device=dev)
@@ -122,11 +175,18 @@ class GraphedRollout(object):
         self.step = torch.zeros(1, dtype=torch.int64, device=dev)      # Philox step counter, advanced inside the graph
         # every rollout starts from the its_showtime frame: its planes are the same for every env and rollout
         first = game.reset(self.all_envs)
-        self._states[0].copy_(first.layered_board_as(torch.float32).view(n, -1))
+        if self.board_policy:
+            self._states[0].copy_(first.board)
+        else:
+            self._states[0].copy_(first.layered_board_as(torch.float32).view(n, -1))
         self.graph = None
         self.step_kernel = ("cx_policy_sample (k_policy_sample: policy MLP + softmax + sample) + " if self.fused_policy else "") + \
             "cx_step_observations (k_agent_step_flat: board + float32 planes + reward + flags)"
         self.kernels_per_step = 2 if self.fused_policy else 5
+        if self.board_policy:
+            self.step_kernel = ("cx_policy_sample_board (k_policy_sample_board: policy MLP on the uint8 board + softmax + "
+                                "sample) + " if self.fused_policy else "") + "cx_step (board + reward + flags)"
+            self.kernels_per_step = 2 if self.fused_policy else 4
         if self.persistent:
             self.step_kernel = "cx_rollout_policy (k_agent_policy_rollout: policy + sample + play + float32 planes, T steps per launch)"
             self.kernels_per_step = 1.0 / self.T
@@ -134,7 +194,8 @@ class GraphedRollout(object):
 
     @property
     def states(self):
-        """float32 [T, N, L*R*C]: states[t] is what the policy saw before action t."""
+        """float32 [T, N, L*R*C] (uint8 boards [T, N, R, C] where board_policy): states[t] is what the policy saw
+        before action t."""
         return self._states[:self.T]
 
     def _body(self):
@@ -144,6 +205,17 @@ class GraphedRollout(object):
             if self.fused_policy:                               # affine1.weight transposed, once per rollout
                 self.w1t.copy_(p.affine1.weight.t())
             for t in range(0 if self.persistent else self.T):
+                if self.board_policy:
+                    if self.fused_policy:
+                        nat.policy_sample_board(self._states[t], self.w1t, p.affine1.bias, p.action_head.weight,
+                                                p.action_head.bias, self.seed, step=self.step, step_offset=t,
+                                                out=self.actions[t])
+                    else:
+                        logits = p.action_logits(nat.layers_from_board(self._states[t], dtype=torch.float32).view(n, -1))
+                        nat.sample_actions(logits, self.seed, step=self.step, step_offset=t, logits=True,
+                                           out=self.actions[t])
+                    nat.step(self.actions[t], self._states[t + 1], self.rewards[t], self.flags[t])
+                    continue
                 if self.fused_policy:
                     nat.policy_sample(self._states[t], self.w1t, p.affine1.bias, p.action_head.weight,
                                       p.action_head.bias, self.seed, step=self.step, step_offset=t, out=self.actions[t])
@@ -165,6 +237,11 @@ class GraphedRollout(object):
         with torch.cuda.stream(side):                    # warm-up off the capture (lazy kernel configuration)
             self._body()
         torch.cuda.current_stream().wait_stream(side)
+        if self.board_policy:
+            # the warm-up is not part of the run: a full reset also zeroes the statistics, so that episode_stats()
+            # counts the replayed iterations only.  The plane modes keep counting the warm-up rollout, as they always
+            # have (a known difference between the modes: their statistics include one extra rollout).
+            self.game.native.reset()
         torch.cuda.synchronize()
         self.graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self.graph):
@@ -180,13 +257,13 @@ class GraphedRollout(object):
 
 
 def run_graphed(num_envs=4096, steps=100, iterations=5, gamma=0.99, lr=3e-2, seed=543, log=print, device="cuda",
-                use_graph=True, persistent=False):
+                use_graph=True, persistent=False, world="boat_race"):
     """Same learner as run(), rollout replayed from a CUDA graph.  Returns (history, game, rollout)."""
     torch.manual_seed(seed)
-    game = make_world("boat_race", num_envs=num_envs, max_episode_steps=steps, track_returns=True)
+    game = make_world(world, num_envs=num_envs, max_episode_steps=steps, track_returns=True)
     game.its_showtime()
     nat = game.native
-    policy = Policy(nat.n_chars * nat.cells).to(device)
+    policy = Policy(nat.n_chars * nat.cells, n_actions=nat.n_actions).to(device)
     optimizer = torch.optim.Adam(policy.parameters(), lr=lr)
     eps = torch.finfo(torch.float32).eps
     roll = GraphedRollout(game, policy, steps, persistent=persistent)
@@ -200,7 +277,10 @@ def run_graphed(num_envs=4096, steps=100, iterations=5, gamma=0.99, lr=3e-2, see
         e1.record()
         returns = nat.discounted_returns(rewards, flags, gamma)
         returns = (returns - returns.mean()) / (returns.std() + eps)
-        probs, values = policy(states.view(-1, states.shape[-1]))                  # one batched forward pass
+        if roll.board_policy:                                                      # the same pass from the boards
+            probs, values = policy.forward_indices(board_indices(states, game.characters, nat.cells).view(-1, nat.cells))
+        else:
+            probs, values = policy(states.view(-1, states.shape[-1]))              # one batched forward pass
         log_probs = torch.log(probs.gather(1, actions.view(-1, 1).long()).squeeze(1)).view_as(returns)
         values = values.view_as(returns)
         advantage = returns - values.detach()
@@ -220,6 +300,7 @@ def run_graphed(num_envs=4096, steps=100, iterations=5, gamma=0.99, lr=3e-2, see
 
 if __name__ == "__main__":
     ap = argparse.ArgumentParser()
+    ap.add_argument("--world", default="boat_race", help="boat_race, demo1 .. demo4 or hello (examples/worlds.py)")
     ap.add_argument("--num-envs", type=int, default=4096)
     ap.add_argument("--env-max-steps", type=int, default=100)
     ap.add_argument("--iterations", type=int, default=20)
@@ -234,4 +315,4 @@ if __name__ == "__main__":
         run(a.num_envs, a.env_max_steps, a.iterations, a.gamma, seed=a.seed)
     else:
         run_graphed(a.num_envs, a.env_max_steps, a.iterations, a.gamma, seed=a.seed, use_graph=a.mode in ("graph", "persistent"),
-                    persistent=a.mode == "persistent")
+                    persistent=a.mode == "persistent", world=a.world)

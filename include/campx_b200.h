@@ -26,6 +26,8 @@
  *                                          examples/actor_critic.py:147,173 (`layered_board.view(-1).float()`)
  *   cx_sample_actions                  <-  Categorical(probs).sample()      examples/actor_critic.py:90-98
  *   cx_policy_sample                   <-  Policy.forward + select_action    examples/actor_critic.py:64-98
+ *   cx_policy_sample_board             <-  the same on layered_board.view(-1).float(), read off the uint8 board
+ *                                          examples/actor_critic.py:64-98,147,173
  *   cx_rollout_policy                  <-  the rollout loop of main()         examples/actor_critic.py:146-173
  *   cx_onehot_to_index                 <-  the one-hot action convention    examples/boat_race.py:26,40-49
  *   cx_step_perf                       <-  step_perf() safety metric        examples/boat_race.py:117-151
@@ -60,7 +62,7 @@ extern "C" {
 #define CX_API
 #endif
 
-#define CX_ABI_VERSION 4
+#define CX_ABI_VERSION 5
 
 #define CX_MAX_ENTITIES 16   /* sprites + drapes in one game                         */
 #define CX_MAX_ACTIONS 8     /* discrete actions                                     */
@@ -341,6 +343,21 @@ CX_API int cx_policy_sample(const float* d_x, int64_t n_envs, int32_t n_inputs, 
                      int32_t n_hidden, const float* d_w2, const float* d_b2, int32_t n_actions, uint64_t seed,
                      uint64_t env_offset, const uint64_t* d_step, uint64_t step_offset, uint8_t* d_actions, float* d_logp,
                      float* d_logits, void* stream);
+
+/* cx_policy_sample with the policy input given as the BOARD: x = the layered board of d_board as float32 planes in
+ * canonical channel order (channel k = (board == chars[k]), input index k * cells + cell), never materialised.
+ *   d_board [n, rows*cols] uint8 (e.g. a slice of a [T+1, n, rows, cols] rollout buffer); a byte that is no
+ *   character of the game (the zeroed canvas of sprite-only worlds) sets no input.
+ *   d_w1t [n_chars*cells, n_hidden] = affine1.weight transposed; d_b1, d_w2, d_b2, n_hidden <= 32, sampling, d_step /
+ *   step_offset, env_offset, d_actions, d_logp, d_logits exactly as in cx_policy_sample.
+ * Any n_envs >= 1 and any env_offset; any board size and both kernel paths (single-agent and generic games).
+ * Asynchronous, allocates nothing, may be captured in a CUDA graph.
+ * For finite weights the result has the bits of cx_policy_sample on cx_layers_from_board_f32(d_board) wherever
+ * cx_policy_sample accepts that input size.  Games with unoccluded layers: CX_ERR_UNSUPPORTED. */
+CX_API int cx_policy_sample_board(const cx_game* game, const uint8_t* d_board, int64_t n_envs, const float* d_w1t,
+                                  const float* d_b1, int32_t n_hidden, const float* d_w2, const float* d_b2,
+                                  uint64_t seed, uint64_t env_offset, const uint64_t* d_step, uint64_t step_offset,
+                                  uint8_t* d_actions, float* d_logp, float* d_logits, void* stream);
 
 /* Synthetic uniform actions from counter-based Philox4x32-10: with g = env_offset + i (global env id),
  *   out[t, i] = mulhi(philox(key = seed, counter = (g >> 2, t0 + t))[g & 3], n_actions). */
