@@ -1,6 +1,6 @@
 // Device helpers shared by the single-agent kernels (cx_agent_kernels.cu, cx_agent_obs_kernels.cu).
 #pragma once
-#include "cx_internal.cuh"
+#include "cx_episode.cuh"
 
 namespace {
 
@@ -74,16 +74,6 @@ __device__ __forceinline__ void st_f32xg(float* p, int64_t i, int64_t end, const
     if (i + k < end) p[i + k] = v[k];
 }
 
-__device__ __forceinline__ double warp_sum(double v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  return v;
-}
-__device__ __forceinline__ float warp_max(float v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
-  return v;
-}
 // ---- bulk asynchronous copy shared -> global (TMA engine, no tensor map: the tile is a flat byte range) ----
 __device__ __forceinline__ uint64_t l2_evict_first_policy() {
   uint64_t pol;
@@ -105,38 +95,5 @@ __device__ __forceinline__ void bulk_wait_read_pending() {
 }
 // make this thread's generic-proxy shared-memory writes visible to the async proxy (the TMA engine)
 __device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-
-// atomic max on a double that is only ever raised (stats slots start at -inf)
-__device__ __forceinline__ void atomic_max_double(double* addr, double v) {
-  unsigned long long* a = reinterpret_cast<unsigned long long*>(addr);
-  unsigned long long old = *a;
-  while (__longlong_as_double((long long)old) < v) {
-    const unsigned long long assumed = old;
-    old = atomicCAS(a, assumed, (unsigned long long)__double_as_longlong(v));
-    if (old == assumed) break;
-  }
-}
-
-// Episode bookkeeping of one lane.  Lives in shared memory (touched only when an episode ends, about
-// once per hundred steps) so that it costs no registers in the step loop; folded into the global
-// statistics once per launch.
-struct LaneStats {
-  double sum, sumsq;
-  uint32_t cnt, len;
-  float mx, negmn;
-  __device__ __forceinline__ void clear() {
-    sum = sumsq = 0.0;
-    cnt = len = 0;
-    mx = negmn = -INFINITY;
-  }
-  __device__ __forceinline__ void episode(float ret, uint32_t steps) {
-    cnt += 1;
-    len += steps;
-    sum += (double)ret;
-    sumsq += (double)ret * (double)ret;
-    mx = fmaxf(mx, ret);
-    negmn = fmaxf(negmn, -ret);
-  }
-};
 
 }  // namespace

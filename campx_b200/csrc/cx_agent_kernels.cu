@@ -227,30 +227,15 @@ k_agent_rollout(const __grid_constant__ AgentParams P) {
           float r = s_tr[idx];
           if (want_discount) dc[i] = s_td[H.td_per_cell ? idx : a];
           if (TRACK && (ts[j][i] & CX_OVER_BIT)) {  // auto_reset == 0 and the episode ended: frozen env
-            e = cellv[j][i] | (was << 8) | ((CX_FLAG_ALREADY_OVER | CX_FLAG_REWARD_NONE) << 16);
+            e = cellv[j][i] | (was << 8) | (CX_FROZEN_FLAGS << 16);
             r = 0.0f;
             dc[i] = 0.0f;
           }
           uint32_t p = e & 0xFF;
           const uint32_t show = (e >> 8) & 0xFF;   // terminal board on a terminal step
           uint32_t f = e >> 16;
-          if (TRACK && !(f & (CX_FLAG_BAD_ACTION | CX_FLAG_ALREADY_OVER))) {
-            // 15-bit counter saturates (bit 15 = OVER); A/B on one box against the unsaturated counter: 0.186 = 0.185 ms
-            const uint32_t steps = min(ts[j][i] + 1u, (uint32_t)CX_STEP_MAX);
-            rt[j][i] += r;
-            if (!(f & CX_FLAG_TERMINATED) && steps >= max_steps) f |= CX_FLAG_TRUNCATED;  // time limit (SURVEY H4)
-            ts[j][i] = steps;
-            if (f & (CX_FLAG_TERMINATED | CX_FLAG_TRUNCATED)) {
-              stats.episode(rt[j][i], steps);
-              if (auto_reset) {  // the next play() starts from the its_showtime state
-                p = init_cell;
-                ts[j][i] = 0;
-                rt[j][i] = 0.0f;
-              } else {
-                ts[j][i] |= CX_OVER_BIT;
-              }
-            }
-          }
+          // the saturating step counter: A/B on one box against the unsaturated counter: 0.186 = 0.185 ms
+          if (TRACK && cx_episode_step(f, r, ts[j][i], rt[j][i], stats, max_steps, auto_reset)) p = init_cell;
           rw[i] = r;
           fl |= f << (8 * i);
           shw |= show << (8 * i);
@@ -348,23 +333,7 @@ k_agent_rollout(const __grid_constant__ AgentParams P) {
       }
     }
   }
-  if (TRACK) {
-    const double cnt = warp_sum((double)stats.cnt), len = warp_sum((double)stats.len);
-    const double sum = warp_sum(stats.sum), sumsq = warp_sum(stats.sumsq);
-    const float mx = warp_max(stats.mx), ngmn = warp_max(stats.negmn);
-    if (lane == 0) {
-      double* sp = cx_stat_stripe(P.stats, (uint32_t)(blockIdx.x * WARPS + warp));
-      if (cnt > 0.0) {
-        atomicAdd(sp + CX_STAT_EPISODES, cnt);
-        atomicAdd(sp + CX_STAT_RETURN_SUM, sum);
-        atomicAdd(sp + CX_STAT_RETURN_SUMSQ, sumsq);
-        atomicAdd(sp + CX_STAT_LENGTH_SUM, len);
-        atomic_max_double(sp + CX_STAT_RETURN_MAX, (double)mx);
-        atomic_max_double(sp + CX_STAT_NEG_RETURN_MIN, (double)ngmn);
-      }
-      atomicAdd(sp + CX_STAT_ENV_STEPS, (double)nenv * (double)P.T);
-    }
-  }
+  if (TRACK) cx_flush_stats(stats, P.stats, (uint32_t)(blockIdx.x * WARPS + warp), (uint32_t)nenv, P.T);
 }
 
 template <bool TRACK, bool VEC, bool SYNTH, int NG, int GW>

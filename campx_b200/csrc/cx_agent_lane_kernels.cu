@@ -193,26 +193,11 @@ __global__ void __launch_bounds__(LANE_MAX_WARPS * 32) k_agent_rollout_lane(cons
           if (ts & CX_OVER_BIT) {  // auto_reset == 0 and the episode ended: frozen env
             p = cell;
             show = drawn[(u + 1) & 1];   // where the last frame drew it
-            f = CX_FLAG_ALREADY_OVER | CX_FLAG_REWARD_NONE;
+            f = CX_FROZEN_FLAGS;
             rw = 0.0f;
             dc = 0.0f;
           }
-          if (!(f & (CX_FLAG_BAD_ACTION | CX_FLAG_ALREADY_OVER))) {
-            const uint32_t st = min(steps, (uint32_t)CX_STEP_MAX);
-            rt += rw;
-            if (!(f & CX_FLAG_TERMINATED) && st >= max_steps) f |= CX_FLAG_TRUNCATED;
-            ts = st;
-            if (f & (CX_FLAG_TERMINATED | CX_FLAG_TRUNCATED)) {
-              stats.episode(rt, st);
-              if (H.auto_reset) {
-                p = H.init_cell;
-                ts = 0;
-                rt = 0.0f;
-              } else {
-                ts |= CX_OVER_BIT;
-              }
-            }
-          }
+          if (cx_episode_step(f, rw, ts, rt, stats, max_steps, H.auto_reset)) p = H.init_cell;
         }
       }
       cell = p;
@@ -254,21 +239,7 @@ __global__ void __launch_bounds__(LANE_MAX_WARPS * 32) k_agent_rollout_lane(cons
     } else {
       stats.clear();   // whatever the empty mask of a lane without an env "played"
     }
-    const double cnt = warp_sum((double)stats.cnt), len = warp_sum((double)stats.len);
-    const double sum = warp_sum(stats.sum), sumsq = warp_sum(stats.sumsq);
-    const float mx = warp_max(stats.mx), ngmn = warp_max(stats.negmn);
-    if (lane == 0) {
-      double* sp = cx_stat_stripe(P.stats, (uint32_t)(blockIdx.x * WARPS + warp));
-      if (cnt > 0.0) {
-        atomicAdd(sp + CX_STAT_EPISODES, cnt);
-        atomicAdd(sp + CX_STAT_RETURN_SUM, sum);
-        atomicAdd(sp + CX_STAT_RETURN_SUMSQ, sumsq);
-        atomicAdd(sp + CX_STAT_LENGTH_SUM, len);
-        atomic_max_double(sp + CX_STAT_RETURN_MAX, (double)mx);
-        atomic_max_double(sp + CX_STAT_NEG_RETURN_MIN, (double)ngmn);
-      }
-      atomicAdd(sp + CX_STAT_ENV_STEPS, (double)nenv * (double)P.T);
-    }
+    cx_flush_stats(stats, P.stats, (uint32_t)(blockIdx.x * WARPS + warp), (uint32_t)nenv, P.T);
   }
 }
 

@@ -51,7 +51,7 @@ constexpr int OBS_WARPS = 4;
 constexpr int OBS_THREADS = OBS_WARPS * 32;
 constexpr int OBS_TILE = 32;  // envs per warp: lane = env
 
-// RING: tiles per warp.  A warp may not touch a tile again before the bulk store that shipped it has READ it; with one
+// RING: tiles per warp, 1 or 2.  A warp may not touch a tile again before the bulk store that shipped it has READ it; with one
 // tile that wait (TMA issue -> shared-memory read, ~1 us) sits on every step's critical path, which is what bounds
 // small batches (65,536 envs = 14 warps per SM: there is nothing else to run meanwhile).  With RING tiles used round
 // robin the warp waits for the store issued RING steps ago (`cp.async.bulk.wait_group.read RING-1`), i.e. almost
@@ -193,7 +193,7 @@ __global__ void __launch_bounds__(OBS_THREADS) k_agent_rollout_obs(const __grid_
       float rw = s_tr[idx];
       float dc = want_discount ? s_td[H.td_per_cell ? idx : a] : 1.0f;
       if (TRACK && (ts & CX_OVER_BIT)) {
-        e = cell | (shown << 8) | ((CX_FLAG_ALREADY_OVER | CX_FLAG_REWARD_NONE) << 16);
+        e = cell | (shown << 8) | (CX_FROZEN_FLAGS << 16);
         rw = 0.0f;
         dc = 0.0f;
       }
@@ -201,22 +201,7 @@ __global__ void __launch_bounds__(OBS_THREADS) k_agent_rollout_obs(const __grid_
       const uint32_t show = mine ? (e >> 8) & 0xFF : none;
       const uint32_t stood = mine ? p : none;   // the agent's cell in this step's frame (before any auto reset)
       uint32_t f = e >> 16;
-      if (TRACK && mine && !(f & (CX_FLAG_BAD_ACTION | CX_FLAG_ALREADY_OVER))) {
-        const uint32_t steps = min(ts + 1u, (uint32_t)CX_STEP_MAX);   // 15-bit counter saturates (bit 15 = OVER)
-        rt += rw;
-        if (!(f & CX_FLAG_TERMINATED) && steps >= max_steps) f |= CX_FLAG_TRUNCATED;
-        ts = steps;
-        if (f & (CX_FLAG_TERMINATED | CX_FLAG_TRUNCATED)) {
-          stats.episode(rt, steps);
-          if (auto_reset) {
-            p = H.init_cell;
-            ts = 0;
-            rt = 0.0f;
-          } else {
-            ts |= CX_OVER_BIT;
-          }
-        }
-      }
+      if (TRACK && mine && cx_episode_step(f, rw, ts, rt, stats, max_steps, auto_reset)) p = H.init_cell;
       if (mine) {
         cell = p;
         __stcs(P.reward + row + lane, rw);
@@ -273,23 +258,8 @@ __global__ void __launch_bounds__(OBS_THREADS) k_agent_rollout_obs(const __grid_
       P.ret[env] = rt;
     }
   }
-  if (TRACK) {  // all 32 lanes reduce (lanes without an env contribute empty statistics)
-    const double cnt = warp_sum((double)stats.cnt), len = warp_sum((double)stats.len);
-    const double sum = warp_sum(stats.sum), sumsq = warp_sum(stats.sumsq);
-    const float mx = warp_max(stats.mx), ngmn = warp_max(stats.negmn);
-    if (lane == 0) {
-      double* sp = cx_stat_stripe(P.stats, (uint32_t)(blockIdx.x * OBS_WARPS + warp));
-      if (cnt > 0.0) {
-        atomicAdd(sp + CX_STAT_EPISODES, cnt);
-        atomicAdd(sp + CX_STAT_RETURN_SUM, sum);
-        atomicAdd(sp + CX_STAT_RETURN_SUMSQ, sumsq);
-        atomicAdd(sp + CX_STAT_LENGTH_SUM, len);
-        atomic_max_double(sp + CX_STAT_RETURN_MAX, (double)mx);
-        atomic_max_double(sp + CX_STAT_NEG_RETURN_MIN, (double)ngmn);
-      }
-      atomicAdd(sp + CX_STAT_ENV_STEPS, (double)nenv * (double)P.T);
-    }
-  }
+  if (TRACK)  // all 32 lanes reduce (lanes without an env contribute empty statistics)
+    cx_flush_stats(stats, P.stats, (uint32_t)(blockIdx.x * OBS_WARPS + warp), (uint32_t)nenv, P.T);
 }
 
 size_t obs_smem_bytes(const cx_game* g, bool layers, int ring = 1) {
@@ -322,9 +292,7 @@ int launch_obs(const ObsParams& P, unsigned grid, size_t smem, cudaStream_t s) {
 
 template <bool TRACK>
 int launch_obs_ring(int ring, const ObsParams& P, unsigned grid, size_t smem, cudaStream_t s) {
-  if (ring >= 4) return launch_obs<TRACK, 4>(P, grid, smem, s);
-  if (ring >= 2) return launch_obs<TRACK, 2>(P, grid, smem, s);
-  return launch_obs<TRACK, 1>(P, grid, smem, s);
+  return ring >= 2 ? launch_obs<TRACK, 2>(P, grid, smem, s) : launch_obs<TRACK, 1>(P, grid, smem, s);
 }
 
 }  // namespace

@@ -213,27 +213,12 @@ __global__ void __launch_bounds__(ROLLOUT_THREADS) k_agent_policy_rollout(const 
       const uint32_t show = frozen ? s_drawn[lane] : (e >> 8) & 0xFF;
       s_drawn[lane] = show;                                 // all the next hidden layer waits for
       if (frozen) {
-        e = cell | (show << 8) | ((CX_FLAG_ALREADY_OVER | CX_FLAG_REWARD_NONE) << 16);
+        e = cell | (show << 8) | (CX_FROZEN_FLAGS << 16);
         rw = 0.0f;
       }
       uint32_t p = e & 0xFF;
       uint32_t f = e >> 16;
-      if (H.track && !(f & (CX_FLAG_BAD_ACTION | CX_FLAG_ALREADY_OVER))) {
-        const uint32_t steps = min(ts + 1u, (uint32_t)CX_STEP_MAX);
-        rt += rw;
-        if (!(f & CX_FLAG_TERMINATED) && steps >= max_steps) f |= CX_FLAG_TRUNCATED;
-        ts = steps;
-        if (f & (CX_FLAG_TERMINATED | CX_FLAG_TRUNCATED)) {
-          stats.episode(rt, steps);
-          if (H.auto_reset) {
-            p = H.init_cell;
-            ts = 0;
-            rt = 0.0f;
-          } else {
-            ts |= CX_OVER_BIT;
-          }
-        }
-      }
+      if (H.track && cx_episode_step(f, rw, ts, rt, stats, max_steps, H.auto_reset)) p = H.init_cell;
       cell = p;
       owed = true;
       o_t = t;
@@ -253,21 +238,7 @@ __global__ void __launch_bounds__(ROLLOUT_THREADS) k_agent_policy_rollout(const 
     if (H.track) {
       P.tstep[env] = (uint16_t)ts;
       P.ret[env] = rt;
-      const double cnt = warp_sum((double)stats.cnt), len = warp_sum((double)stats.len);
-      const double sum = warp_sum(stats.sum), sumsq = warp_sum(stats.sumsq);
-      const float mx = warp_max(stats.mx), ngmn = warp_max(stats.negmn);
-      if (lane == 0) {
-        double* sp = cx_stat_stripe(P.stats, blockIdx.x);
-        if (cnt > 0.0) {
-          atomicAdd(sp + CX_STAT_EPISODES, cnt);
-          atomicAdd(sp + CX_STAT_RETURN_SUM, sum);
-          atomicAdd(sp + CX_STAT_RETURN_SUMSQ, sumsq);
-          atomicAdd(sp + CX_STAT_LENGTH_SUM, len);
-          atomic_max_double(sp + CX_STAT_RETURN_MAX, (double)mx);
-          atomic_max_double(sp + CX_STAT_NEG_RETURN_MIN, (double)ngmn);
-        }
-        atomicAdd(sp + CX_STAT_ENV_STEPS, 32.0 * (double)P.T);
-      }
+      cx_flush_stats(stats, P.stats, blockIdx.x, 32u, P.T);
     }
   }
 }

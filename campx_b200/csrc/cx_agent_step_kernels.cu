@@ -113,8 +113,7 @@ __global__ void __launch_bounds__(ST_THREADS) k_agent_step_flat(const __grid_con
       ts = P.tstep[env];
       rt = P.ret[env];
       if (ts & CX_OVER_BIT) {  // auto_reset == 0 and the episode ended: frozen env, board stays as it was drawn
-        e = cell | ((uint32_t)__ldg(P.blob + H.off_shown + cell) << 8) |
-            ((CX_FLAG_ALREADY_OVER | CX_FLAG_REWARD_NONE) << 16);
+        e = cell | ((uint32_t)__ldg(P.blob + H.off_shown + cell) << 8) | (CX_FROZEN_FLAGS << 16);
         r = 0.0f;
         dc = 0.0f;
       }
@@ -123,22 +122,7 @@ __global__ void __launch_bounds__(ST_THREADS) k_agent_step_flat(const __grid_con
     const uint32_t show = (e >> 8) & 0xFF;
     s_stood[el] = (uint8_t)p;    // before any auto reset: the frame shows the terminal state
     uint32_t f = e >> 16;
-    if (TRACK && !(f & (CX_FLAG_BAD_ACTION | CX_FLAG_ALREADY_OVER))) {
-      const uint32_t steps = min(ts + 1u, (uint32_t)CX_STEP_MAX);
-      rt += r;
-      if (!(f & CX_FLAG_TERMINATED) && steps >= max_steps) f |= CX_FLAG_TRUNCATED;
-      ts = steps;
-      if (f & (CX_FLAG_TERMINATED | CX_FLAG_TRUNCATED)) {
-        st.episode(rt, steps);
-        if (auto_reset) {
-          p = H.init_cell;
-          ts = 0;
-          rt = 0.0f;
-        } else {
-          ts |= CX_OVER_BIT;
-        }
-      }
-    }
+    if (TRACK && cx_episode_step(f, r, ts, rt, st, max_steps, auto_reset)) p = H.init_cell;
     P.cell[env] = (uint8_t)p;
     if (TRACK) {
       P.tstep[env] = (uint16_t)ts;
@@ -238,21 +222,9 @@ __global__ void __launch_bounds__(ST_THREADS) k_agent_step_flat(const __grid_con
   }
 
   if (TRACK && P.actions != nullptr) {
-    const double cnt = warp_sum((double)st.cnt);
-    if (cnt > 0.0) {  // warp-uniform: rare (an episode ended in this warp's envs)
-      const double len = warp_sum((double)st.len), sum = warp_sum(st.sum), sumsq = warp_sum(st.sumsq);
-      const float mx = warp_max(st.mx), ngmn = warp_max(st.negmn);
-      if ((tid & 31) == 0) {
-        double* sp = cx_stat_stripe(P.stats, (uint32_t)(blockIdx.x * (blockDim.x >> 5) + (tid >> 5)));
-        atomicAdd(sp + CX_STAT_EPISODES, cnt);
-        atomicAdd(sp + CX_STAT_RETURN_SUM, sum);
-        atomicAdd(sp + CX_STAT_RETURN_SUMSQ, sumsq);
-        atomicAdd(sp + CX_STAT_LENGTH_SUM, len);
-        atomic_max_double(sp + CX_STAT_RETURN_MAX, (double)mx);
-        atomic_max_double(sp + CX_STAT_NEG_RETURN_MIN, (double)ngmn);
-      }
-    }
+    // the env-steps of the whole grid are added once, by its first thread, not by every warp
     if (blockIdx.x == 0 && tid == 0) atomicAdd(cx_stat_stripe(P.stats, 0) + CX_STAT_ENV_STEPS, (double)P.n);
+    cx_flush_stats(st, P.stats, (uint32_t)(blockIdx.x * (blockDim.x >> 5) + (tid >> 5)), 0u, 0);
   }
 }
 

@@ -38,7 +38,7 @@
 // Per env-step HBM traffic is the observation contract only (board + reward + flags + discount + action);
 // entity state and the plane move once per launch.  Games with more than CX_MAX_LIN per-env masks, rolling
 // drapes wider than 64 columns, or unaligned buffers use the per-cell painter's algorithm instead.
-#include "cx_internal.cuh"
+#include "cx_episode.cuh"
 #include "cx_philox.cuh"
 
 namespace {
@@ -401,26 +401,6 @@ __device__ __forceinline__ void fast_load_state(const Ctx& X, const uint16_t* st
         sreg[d] = ((rc >> 8) << 16) | (rc & 255u);
       }
     }
-  }
-}
-
-__device__ __forceinline__ double warp_sum(double v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  return v;
-}
-__device__ __forceinline__ float warp_max(float v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
-  return v;
-}
-__device__ __forceinline__ void atomic_max_double(double* addr, double v) {
-  unsigned long long* a = reinterpret_cast<unsigned long long*>(addr);
-  unsigned long long old = *a;
-  while (__longlong_as_double((long long)old) < v) {
-    const unsigned long long assumed = old;
-    old = atomicCAS(a, assumed, (unsigned long long)__double_as_longlong(v));
-    if (old == assumed) break;
   }
 }
 
@@ -967,9 +947,9 @@ __global__ void __launch_bounds__(BLK, OCC) k_generic_rollout(const __grid_const
   uint32_t sreg[CX_MAX_DYN];
   if (FAST && mine) fast_load_state(X, dyn[lane], sreg);
 
-  uint32_t ep_cnt = 0, ep_len = 0;
-  double ep_sum = 0.0, ep_sumsq = 0.0;
-  float ep_max = -INFINITY, ep_negmin = -INFINITY;
+  LaneStats stats;
+  stats.clear();
+  const uint32_t max_steps = H.max_steps > 0 ? (uint32_t)H.max_steps : 0xFFFFFFFFu;
 
   uint32_t a_next = 0;  // this lane's action for the coming step, loaded one step ahead of its use
   if (mine && !P.synth) a_next = P.actions[env0 + lane];
@@ -990,7 +970,7 @@ __global__ void __launch_bounds__(BLK, OCC) k_generic_rollout(const __grid_const
       if (H.track && (ts & CX_OVER_BIT)) {
         rw = 0.0f;
         dc = 0.0f;
-        f = CX_FLAG_ALREADY_OVER | CX_FLAG_REWARD_NONE;
+        f = CX_FROZEN_FLAGS;
       } else {
         if (FAST)
           fast_env_step(X, a, sreg, dyn[lane], plane + lane * cells, rw, f, dc);
@@ -999,27 +979,8 @@ __global__ void __launch_bounds__(BLK, OCC) k_generic_rollout(const __grid_const
         else
           generic_env_step(X, a, dyn[lane], W.prev[lane], plane + lane * cells, rw, f, dc);
       }
-      if (H.track && !(f & (CX_FLAG_BAD_ACTION | CX_FLAG_ALREADY_OVER))) {
-        const uint32_t steps = min(ts + 1u, (uint32_t)CX_STEP_MAX);   // 15-bit counter saturates (bit 15 = OVER)
-        rt += rw;
-        if (!(f & CX_FLAG_TERMINATED) && H.max_steps > 0 && steps >= (uint32_t)H.max_steps) f |= CX_FLAG_TRUNCATED;
-        ts = steps;
-        if (f & (CX_FLAG_TERMINATED | CX_FLAG_TRUNCATED)) {
-          ep_cnt += 1;
-          ep_len += steps;
-          ep_sum += (double)rt;
-          ep_sumsq += (double)rt * (double)rt;
-          ep_max = fmaxf(ep_max, rt);
-          ep_negmin = fmaxf(ep_negmin, -rt);
-          if (H.auto_reset) {
-            reset_me = true;  // state is reset after this step's (terminal) board has been composed
-            ts = 0;
-            rt = 0.0f;
-          } else {
-            ts |= CX_OVER_BIT;
-          }
-        }
-      }
+      // a restarting env's state is reset after this step's (terminal) board has been composed
+      if (H.track) reset_me = cx_episode_step(f, rw, ts, rt, stats, max_steps, H.auto_reset);
       P.reward[row + lane] = rw;
       if (P.discount) P.discount[row + lane] = dc;
       P.flags[row + lane] = (uint8_t)f;
@@ -1074,23 +1035,7 @@ __global__ void __launch_bounds__(BLK, OCC) k_generic_rollout(const __grid_const
       for (int b = lane; b < nenv * cells; b += 32) P.dynbd[env0 * cells + b] = plane[b];
     }
   }
-  if (H.track) {
-    const double cnt = warp_sum((double)ep_cnt), len = warp_sum((double)ep_len);
-    const double sum = warp_sum(ep_sum), sumsq = warp_sum(ep_sumsq);
-    const float mx = warp_max(ep_max), ngmn = warp_max(ep_negmin);
-    if (lane == 0) {
-      double* sp = cx_stat_stripe(P.stats, (uint32_t)(blockIdx.x * wpc + warp));
-      if (cnt > 0.0) {
-        atomicAdd(sp + CX_STAT_EPISODES, cnt);
-        atomicAdd(sp + CX_STAT_RETURN_SUM, sum);
-        atomicAdd(sp + CX_STAT_RETURN_SUMSQ, sumsq);
-        atomicAdd(sp + CX_STAT_LENGTH_SUM, len);
-        atomic_max_double(sp + CX_STAT_RETURN_MAX, (double)mx);
-        atomic_max_double(sp + CX_STAT_NEG_RETURN_MIN, (double)ngmn);
-      }
-      atomicAdd(sp + CX_STAT_ENV_STEPS, (double)nenv * (double)P.T);
-    }
-  }
+  if (H.track) cx_flush_stats(stats, P.stats, (uint32_t)(blockIdx.x * wpc + warp), (uint32_t)nenv, P.T);
 }
 
 // Render the current state of every env (first frame after its_showtime / reset).
