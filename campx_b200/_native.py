@@ -7,7 +7,7 @@ compute entry point is needed, this module raises.  The library is built in-tree
 import ctypes
 import os
 
-CX_ABI_VERSION = 5
+CX_ABI_VERSION = 6
 CX_MAX_ENTITIES = 16
 CX_MAX_ACTIONS = 8
 CX_MAX_CHARS = 32
@@ -35,6 +35,8 @@ CX_DTYPE_U8, CX_DTYPE_F32, CX_DTYPE_BF16 = 0, 1, 2
 CX_STATS_DOUBLES = 8
 STAT_NAMES = ("episodes", "return_sum", "return_sumsq", "length_sum", "return_max", "neg_return_min",
               "env_steps", "reserved")
+CX_STAT_PERFORMANCE_SUM = 7   # slot 7: "performance_sum" for games that track performance, else "reserved" (always 0)
+STAT_NAMES_PERFORMANCE = STAT_NAMES[:CX_STAT_PERFORMANCE_SUM] + ("performance_sum",)
 
 CX_PATH_AGENT, CX_PATH_GENERIC = 1, 2
 
@@ -95,13 +97,16 @@ class GameDesc(ctypes.Structure):
         ("backdrop_dr", ctypes.c_int8 * CX_MAX_ACTIONS),
         ("backdrop_dc", ctypes.c_int8 * CX_MAX_ACTIONS),
         ("unoccluded_layers", ctypes.c_int32),
+        ("perf_regions", ctypes.POINTER(ctypes.c_uint8)),
+        ("n_perf_regions", ctypes.c_int32),
     ]
 
 
 class GameInfo(ctypes.Structure):
     _fields_ = [(n, ctypes.c_int32) for n in (
         "rows", "cols", "cells", "n_chars", "n_actions", "n_entities", "path", "can_terminate", "tracks",
-        "has_dynamic_backdrop", "state_bytes_per_env", "board_bytes_per_env", "dynamic_render")]
+        "has_dynamic_backdrop", "state_bytes_per_env", "board_bytes_per_env", "dynamic_render",
+        "tracks_performance")]
 
 
 _P = ctypes.c_void_p
@@ -141,6 +146,7 @@ PROTOTYPES = {
     "cx_set_entity_state": (ctypes.c_int, [_P, _P, _I64, _I32, _P, _P]),
     "cx_get_render_state": (ctypes.c_int, [_P, _P, _I64, _P, _P, _P, _P]),
     "cx_get_episode_state": (ctypes.c_int, [_P, _P, _I64, _P, _P, _P]),
+    "cx_get_episode_performance": (ctypes.c_int, [_P, _P, _I64, _P, _P]),
     "cx_stats_fold": (ctypes.c_int, [_P, _P, _P]),
     "cx_stats_read": (ctypes.c_int, [_P, _P, ctypes.POINTER(ctypes.c_double), _P]),
     "cx_step_perf": (ctypes.c_int, [_P, _I32, _I32, _P, _P, _I64, _P, _P]),

@@ -3,7 +3,7 @@
 Same entry points as `campx/ascii_art.py`: `ascii_art_to_long_tensor` (:29-57),
 `ascii_art_to_game` (:60-309) and `Partial` (:311-340), with the same argument meaning, defaults,
 validation and exception classes.  Extra keyword arguments (`num_envs`, `device`, `num_actions`,
-`action_format`, `max_episode_steps`, `auto_reset`, `track_returns`, `verify`) are forwarded to
+`action_format`, `max_episode_steps`, `auto_reset`, `track_returns`, `performance_regions`, `verify`) are forwarded to
 `Engine` -- they are the only additions.
 """
 import itertools

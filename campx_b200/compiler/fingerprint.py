@@ -215,7 +215,7 @@ def _find_roll(before, after):
 
 
 def compile_game(shadow, n_actions=5, action_format=None, max_episode_steps=0, auto_reset=True,
-                 track_returns=False, occlusion_in_layers=True):
+                 track_returns=False, occlusion_in_layers=True, performance_regions=None):
     """Fingerprint `shadow` (a not-yet-started ShadowEngine) and return its GameSpec.
 
     Runs the shadow's its_showtime() first (campx/engine.py:487-544); the resulting state is the
@@ -615,6 +615,6 @@ def compile_game(shadow, n_actions=5, action_format=None, max_episode_steps=0, a
                     auto_reset=auto_reset, track_returns=track_returns,
                     first_reward=None if first_reward is None else float(_f32(first_reward)),
                     first_discount=float(first_discount), action_format=fmt, backdrop_moves=backdrop_moves,
-                    occlusion_in_layers=bool(occlusion_in_layers))
+                    occlusion_in_layers=bool(occlusion_in_layers), performance_regions=performance_regions)
     spec.n_probes = len(probes)
     return spec

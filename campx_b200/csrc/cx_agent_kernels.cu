@@ -45,6 +45,7 @@ struct AgentParams {
   int32_t T;
   uint64_t seed, env_offset, t0;  // SYNTH: actions come from cx_philox.cuh instead of `actions`
   uint8_t* actions_out;           // SYNTH: [T, n] or null
+  float* perf;                    // [n] (PERF)
 };
 
 // A warp owns WT = NG * 32 * GW consecutive envs: every lane holds NG groups of GW consecutive envs (group j of lane l
@@ -54,7 +55,8 @@ struct AgentParams {
 //   NG 1, GW 4   128 envs per warp: twice the warps for mid-size batches (2^18: 63 % -> 85 % of peak)
 //   NG 1, GW 2    64 envs per warp: four times the warps for small ones (BASELINE config 1: 65,536 envs)
 // CTAs are 1..4 warps (blockDim), chosen by the launcher so that small grids still spread evenly over the SMs.
-template <bool TRACK, bool VEC, bool SYNTH, int NG, int GW>
+// PERF (TRACK builds of games that track performance): the running performance of every env lives beside its return.
+template <bool TRACK, bool PERF, bool VEC, bool SYNTH, int NG, int GW>
 __global__ void __launch_bounds__(CX_AGENT_CTA_THREADS, 7)  // 7 CTAs/SM: 1024 CTAs (2^20 envs) in one wave
 k_agent_rollout(const __grid_constant__ AgentParams P) {
   constexpr int WT = NG * 32 * GW;                 // envs per warp
@@ -109,6 +111,7 @@ k_agent_rollout(const __grid_constant__ AgentParams P) {
   uint32_t drawnq[NG];      // per env one byte: cell where the agent is currently drawn in the tile (none: nowhere)
   uint32_t ts[NG][GW];
   float rt[NG][GW];
+  float pf[NG][GW];
 #pragma unroll
   for (int j = 0; j < NG; ++j) {
     const int el = j * (32 * GW) + lane * GW;
@@ -120,11 +123,19 @@ k_agent_rollout(const __grid_constant__ AgentParams P) {
         const float4 rv = *reinterpret_cast<const float4*>(P.ret + env0 + el);
         ts[j][0] = tv.x & 0xFFFF; ts[j][1] = tv.x >> 16; ts[j][GW - 2] = tv.y & 0xFFFF; ts[j][GW - 1] = tv.y >> 16;
         rt[j][0] = rv.x; rt[j][1] = rv.y; rt[j][GW - 2] = rv.z; rt[j][GW - 1] = rv.w;
+        if (PERF) {
+          const float4 pv = *reinterpret_cast<const float4*>(P.perf + env0 + el);
+          pf[j][0] = pv.x; pf[j][1] = pv.y; pf[j][GW - 2] = pv.z; pf[j][GW - 1] = pv.w;
+        }
       } else {
         const uint32_t tv = *reinterpret_cast<const uint32_t*>(P.tstep + env0 + el);
         const float2 rv = *reinterpret_cast<const float2*>(P.ret + env0 + el);
         ts[j][0] = tv & 0xFFFF; ts[j][1] = tv >> 16;
         rt[j][0] = rv.x; rt[j][1] = rv.y;
+        if (PERF) {
+          const float2 pv = *reinterpret_cast<const float2*>(P.perf + env0 + el);
+          pf[j][0] = pv.x; pf[j][1] = pv.y;
+        }
       }
     }
     drawnq[j] = 0;
@@ -134,6 +145,7 @@ k_agent_rollout(const __grid_constant__ AgentParams P) {
       if (TRACK && !VEC) {
         ts[j][i] = valid ? P.tstep[env0 + el + i] : 0u;
         rt[j][i] = valid ? P.ret[env0 + el + i] : 0.0f;
+        if (PERF) pf[j][i] = valid ? P.perf[env0 + el + i] : 0.0f;
       }
       cellv[j][i] = min((cq >> (8 * i)) & 0xFF, none);
       uint32_t sh = none;
@@ -145,7 +157,7 @@ k_agent_rollout(const __grid_constant__ AgentParams P) {
     }
   }
 
-  LaneStats& stats = reinterpret_cast<LaneStats*>(smem + H.blob_bytes + (size_t)WARPS * (WT * cells))[tid];
+  LaneStatsT<PERF>& stats = reinterpret_cast<LaneStatsT<PERF>*>(smem + H.blob_bytes + (size_t)WARPS * (WT * cells))[tid];
   if (TRACK) stats.clear();
 
   // Action reads are 3% of the bytes but, interleaved with the write streams at the DRAM, cost ~10% of
@@ -233,9 +245,11 @@ k_agent_rollout(const __grid_constant__ AgentParams P) {
           }
           uint32_t p = e & 0xFF;
           const uint32_t show = (e >> 8) & 0xFF;   // terminal board on a terminal step
-          uint32_t f = e >> 16;
+          uint32_t f = cx_tt_flags<PERF>(e);
           // the saturating step counter: A/B on one box against the unsaturated counter: 0.186 = 0.185 ms
-          if (TRACK && cx_episode_step(f, r, ts[j][i], rt[j][i], stats, max_steps, auto_reset)) p = init_cell;
+          if (TRACK && cx_episode_step<PERF>(f, r, ts[j][i], rt[j][i], stats, max_steps, auto_reset, &pf[j][i],
+                                             cx_tt_perf(e)))
+            p = init_cell;
           rw[i] = r;
           fl |= f << (8 * i);
           shw |= show << (8 * i);
@@ -319,9 +333,12 @@ k_agent_rollout(const __grid_constant__ AgentParams P) {
           *reinterpret_cast<uint2*>(P.tstep + env0 + el) =
               make_uint2(ts[j][0] | (ts[j][1] << 16), ts[j][GW - 2] | (ts[j][GW - 1] << 16));
           *reinterpret_cast<float4*>(P.ret + env0 + el) = make_float4(rt[j][0], rt[j][1], rt[j][GW - 2], rt[j][GW - 1]);
+          if (PERF)
+            *reinterpret_cast<float4*>(P.perf + env0 + el) = make_float4(pf[j][0], pf[j][1], pf[j][GW - 2], pf[j][GW - 1]);
         } else {
           *reinterpret_cast<uint32_t*>(P.tstep + env0 + el) = ts[j][0] | (ts[j][1] << 16);
           *reinterpret_cast<float2*>(P.ret + env0 + el) = make_float2(rt[j][0], rt[j][1]);
+          if (PERF) *reinterpret_cast<float2*>(P.perf + env0 + el) = make_float2(pf[j][0], pf[j][1]);
         }
       } else if (TRACK) {
 #pragma unroll
@@ -329,18 +346,19 @@ k_agent_rollout(const __grid_constant__ AgentParams P) {
           if (el + i < nenv) {
             P.tstep[env0 + el + i] = (uint16_t)ts[j][i];
             P.ret[env0 + el + i] = rt[j][i];
+            if (PERF) P.perf[env0 + el + i] = pf[j][i];
           }
       }
     }
   }
-  if (TRACK) cx_flush_stats(stats, P.stats, (uint32_t)(blockIdx.x * WARPS + warp), (uint32_t)nenv, P.T);
+  if (TRACK) cx_flush_stats<PERF>(stats, P.stats, (uint32_t)(blockIdx.x * WARPS + warp), (uint32_t)nenv, P.T);
 }
 
-template <bool TRACK, bool VEC, bool SYNTH, int NG, int GW>
+template <bool TRACK, bool PERF, bool VEC, bool SYNTH, int NG, int GW>
 int launch(const AgentParams& P, unsigned grid, unsigned block, size_t smem, cudaStream_t s) {
   static CxPerDevice configured;  // raise the dynamic shared memory cap once per device (it reserves nothing)
   if (configured.need()) {
-    CX_CUDA_OK(cudaFuncSetAttribute(k_agent_rollout<TRACK, VEC, SYNTH, NG, GW>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    CX_CUDA_OK(cudaFuncSetAttribute(k_agent_rollout<TRACK, PERF, VEC, SYNTH, NG, GW>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                     227 * 1024));
     configured.mark();
   }
@@ -355,24 +373,28 @@ int launch(const AgentParams& P, unsigned grid, unsigned block, size_t smem, cud
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  CX_CUDA_OK(cudaLaunchKernelEx(&cfg, k_agent_rollout<TRACK, VEC, SYNTH, NG, GW>, P));
+  CX_CUDA_OK(cudaLaunchKernelEx(&cfg, k_agent_rollout<TRACK, PERF, VEC, SYNTH, NG, GW>, P));
   return CX_OK;
 }
 
 template <bool SYNTH, int NG, int GW>
-int launch_tv(bool track, bool vec, const AgentParams& P, unsigned grid, unsigned block, size_t smem, cudaStream_t s) {
+int launch_tv(bool track, bool perf, bool vec, const AgentParams& P, unsigned grid, unsigned block, size_t smem,
+              cudaStream_t s) {
+  if (perf)
+    return vec ? launch<true, true, true, SYNTH, NG, GW>(P, grid, block, smem, s)
+               : launch<true, true, false, SYNTH, NG, GW>(P, grid, block, smem, s);
   if (track)
-    return vec ? launch<true, true, SYNTH, NG, GW>(P, grid, block, smem, s)
-               : launch<true, false, SYNTH, NG, GW>(P, grid, block, smem, s);
-  return vec ? launch<false, true, SYNTH, NG, GW>(P, grid, block, smem, s)
-             : launch<false, false, SYNTH, NG, GW>(P, grid, block, smem, s);
+    return vec ? launch<true, false, true, SYNTH, NG, GW>(P, grid, block, smem, s)
+               : launch<true, false, false, SYNTH, NG, GW>(P, grid, block, smem, s);
+  return vec ? launch<false, false, true, SYNTH, NG, GW>(P, grid, block, smem, s)
+             : launch<false, false, false, SYNTH, NG, GW>(P, grid, block, smem, s);
 }
 
 template <int NG, int GW>
-int launch_s(bool synth, bool track, bool vec, const AgentParams& P, unsigned grid, unsigned block, size_t smem,
-             cudaStream_t s) {
-  return synth ? launch_tv<true, NG, GW>(track, vec, P, grid, block, smem, s)
-               : launch_tv<false, NG, GW>(track, vec, P, grid, block, smem, s);
+int launch_s(bool synth, bool track, bool perf, bool vec, const AgentParams& P, unsigned grid, unsigned block,
+             size_t smem, cudaStream_t s) {
+  return synth ? launch_tv<true, NG, GW>(track, perf, vec, P, grid, block, smem, s)
+               : launch_tv<false, NG, GW>(track, perf, vec, P, grid, block, smem, s);
 }
 
 }  // namespace
@@ -402,6 +424,7 @@ int cx_launch_agent_rollout(const cx_game* g, void* d_state, int64_t n, int32_t 
   P.env_offset = synth.env_offset;
   P.t0 = synth.t0;
   P.actions_out = synth.actions_out;
+  P.perf = reinterpret_cast<float*>(base + L.off_perf);
   auto al16 = [](const void* p) { return p == nullptr || (reinterpret_cast<uintptr_t>(p) & 15) == 0; };
   // envs per warp, by envs per SM (measured on 148 SMs, Demo 1, 32-step launches, % of the HBM copy peak for
   // 64 / 128 / 256 envs per warp: 65,536 envs 45 / 36 / 19, 2^17 65 / 62 / 37, 2^18 79 / 87 / 63, 2^19 83 / 82 / 79,
@@ -428,7 +451,7 @@ int cx_launch_agent_rollout(const cx_game* g, void* d_state, int64_t n, int32_t 
   const bool rest_on_lanes = aligned && cx_agent_lane_applies(g, n, d_actions, synth.actions_out, d_reward, d_discount,
                                                              d_flags, d_board);
   const int64_t n_vec = aligned && (rest_on_lanes || n % WT == 0) ? n / WT * WT : 0;   // envs [0, n_vec): vector path
-  const bool track = g->ah.track != 0, sy = synth.on != 0;
+  const bool track = g->ah.track != 0, perf = g->info.tracks_performance != 0, sy = synth.on != 0;
   // one launch over envs [lo, hi) of the batch
   auto launch_range = [&](AgentParams Q, int64_t lo, int64_t hi, bool vec) -> int {
     Q.env_base = lo;
@@ -439,15 +462,15 @@ int cx_launch_agent_rollout(const cx_game* g, void* d_state, int64_t n, int32_t 
     while (wpc > 1 && (warps + wpc - 1) / wpc < (int64_t)g->sm_count * 4) wpc >>= 1;
     const unsigned block = 32u * wpc;
     const size_t smem = (size_t)g->ah.blob_bytes + (size_t)wpc * WT * g->ah.cells +
-                        (g->ah.track ? (size_t)block * sizeof(LaneStats) : 0);
+                        (g->ah.track ? (size_t)block * (perf ? sizeof(LaneStatsPerf) : sizeof(LaneStats)) : 0);
     const int64_t grid = (warps + wpc - 1) / wpc;
     if (grid > 0x7fffffff) {
       cx_set_error("cx_rollout: too many environments for one launch");
       return CX_ERR_INVALID_ARG;
     }
-    if (WT == 64) return launch_s<1, 2>(sy, track, vec, Q, (unsigned)grid, block, smem, s);
-    if (WT == 128) return launch_s<1, 4>(sy, track, vec, Q, (unsigned)grid, block, smem, s);
-    return launch_s<2, 4>(sy, track, vec, Q, (unsigned)grid, block, smem, s);
+    if (WT == 64) return launch_s<1, 2>(sy, track, perf, vec, Q, (unsigned)grid, block, smem, s);
+    if (WT == 128) return launch_s<1, 4>(sy, track, perf, vec, Q, (unsigned)grid, block, smem, s);
+    return launch_s<2, 4>(sy, track, perf, vec, Q, (unsigned)grid, block, smem, s);
   };
   auto launch_wt = [&](const AgentParams& Q) -> int {   // the whole tiles, then the rest
     if (n_vec == 0) return launch_range(Q, 0, n, false);

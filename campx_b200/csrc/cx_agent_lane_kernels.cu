@@ -42,6 +42,7 @@ struct LaneParams {
   int32_t T;
   uint64_t seed, env_offset, t0;
   uint8_t* actions_out;    // SYNTH: [T, n] or null
+  float* perf;             // [n] (PERF)
 };
 
 constexpr int LANE_MAX_WARPS = 4;
@@ -74,8 +75,9 @@ __device__ __forceinline__ uint4 lds_tile_v4(uint32_t a) {
 }
 
 // DISC: the game can change the discount (a [T, n] discount stream is written); SMALL: boards of up to 32 cells (at
-// most two 16-byte chunks of the warp's tile per lane)
-template <bool TRACK, bool SYNTH, bool DISC, bool SMALL>
+// most two 16-byte chunks of the warp's tile per lane); PERF (TRACK builds of games that track performance): the
+// running performance beside the return
+template <bool TRACK, bool PERF, bool SYNTH, bool DISC, bool SMALL>
 __global__ void __launch_bounds__(LANE_MAX_WARPS * 32) k_agent_rollout_lane(const __grid_constant__ LaneParams P) {
   extern __shared__ __align__(16) uint8_t smem[];
   const CxAgentHeader& H = P.h;
@@ -121,10 +123,11 @@ __global__ void __launch_bounds__(LANE_MAX_WARPS * 32) k_agent_rollout_lane(cons
   asm volatile("griddepcontrol.wait;" ::: "memory");
   uint32_t cell = mine ? min((uint32_t)P.cell[env], none) : none;
   uint32_t ts = 0;
-  float rt = 0.0f;
+  float rt = 0.0f, pf = 0.0f;
   if (TRACK && mine) {
     ts = P.tstep[env];
     rt = P.ret[env];
+    if (PERF) pf = P.perf[env];
   }
   const uint32_t a_mine = sbase + tile0 + lane * cells;   // this env's board in tile 0; tile 1 is tile_bytes further
   const uint32_t a_copy = sbase + tile0 + lane * 16;      // this lane's first chunk of tile 0
@@ -134,7 +137,7 @@ __global__ void __launch_bounds__(LANE_MAX_WARPS * 32) k_agent_rollout_lane(cons
     sts_tile_u8(a_mine + drawn[0], agent_char);
     sts_tile_u8(a_mine + tile_bytes + drawn[0], agent_char);
   }
-  LaneStats& stats = reinterpret_cast<LaneStats*>(smem + H.blob_bytes + (size_t)WARPS * 2 * tile_bytes)[tid];
+  LaneStatsT<PERF>& stats = reinterpret_cast<LaneStatsT<PERF>*>(smem + H.blob_bytes + (size_t)WARPS * 2 * tile_bytes)[tid];
   if (TRACK) stats.clear();
 
   // actions: one group of LANE_UNR steps is in flight while the previous one is consumed; running row pointer
@@ -180,7 +183,7 @@ __global__ void __launch_bounds__(LANE_MAX_WARPS * 32) k_agent_rollout_lane(cons
       float rw = lds_tab_f32(a_tr + idx4);
       float dc = 1.0f;
       if (DISC) dc = lds_tab_f32(a_td + (H.td_per_cell ? idx4 : a * 4u));
-      uint32_t f = e >> 16;
+      uint32_t f = cx_tt_flags<PERF>(e);
       uint32_t p = e & 0xFF, show = (e >> 8) & 0xFF;
       if (TRACK) {
         const uint32_t steps = ts + 1u;
@@ -189,6 +192,7 @@ __global__ void __launch_bounds__(LANE_MAX_WARPS * 32) k_agent_rollout_lane(cons
         if (special == 0 && steps < limit) {
           ts = steps;
           rt += rw;
+          if (PERF) pf += cx_tt_perf(e);
         } else {
           if (ts & CX_OVER_BIT) {  // auto_reset == 0 and the episode ended: frozen env
             p = cell;
@@ -197,7 +201,7 @@ __global__ void __launch_bounds__(LANE_MAX_WARPS * 32) k_agent_rollout_lane(cons
             rw = 0.0f;
             dc = 0.0f;
           }
-          if (cx_episode_step(f, rw, ts, rt, stats, max_steps, H.auto_reset)) p = H.init_cell;
+          if (cx_episode_step<PERF>(f, rw, ts, rt, stats, max_steps, H.auto_reset, &pf, cx_tt_perf(e))) p = H.init_cell;
         }
       }
       cell = p;
@@ -236,23 +240,25 @@ __global__ void __launch_bounds__(LANE_MAX_WARPS * 32) k_agent_rollout_lane(cons
     if (mine) {
       P.tstep[env] = (uint16_t)ts;
       P.ret[env] = rt;
+      if (PERF) P.perf[env] = pf;
     } else {
       stats.clear();   // whatever the empty mask of a lane without an env "played"
     }
-    cx_flush_stats(stats, P.stats, (uint32_t)(blockIdx.x * WARPS + warp), (uint32_t)nenv, P.T);
+    cx_flush_stats<PERF>(stats, P.stats, (uint32_t)(blockIdx.x * WARPS + warp), (uint32_t)nenv, P.T);
   }
 }
 
 size_t lane_smem_bytes(const cx_game* g, int warps) {
+  const size_t stats_bytes = g->info.tracks_performance ? sizeof(LaneStatsPerf) : sizeof(LaneStats);
   return (size_t)g->ah.blob_bytes + (size_t)warps * 2 * 32 * g->ah.cells +
-         (g->ah.track ? (size_t)warps * 32 * sizeof(LaneStats) : 0);
+         (g->ah.track ? (size_t)warps * 32 * stats_bytes : 0);
 }
 
-template <bool TRACK, bool SYNTH, bool DISC, bool SMALL>
+template <bool TRACK, bool PERF, bool SYNTH, bool DISC, bool SMALL>
 int launch_lane(const LaneParams& P, unsigned grid, unsigned block, size_t smem, bool pdl, cudaStream_t s) {
   static CxPerDevice configured;
   if (configured.need()) {
-    CX_CUDA_OK(cudaFuncSetAttribute(k_agent_rollout_lane<TRACK, SYNTH, DISC, SMALL>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    CX_CUDA_OK(cudaFuncSetAttribute(k_agent_rollout_lane<TRACK, PERF, SYNTH, DISC, SMALL>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                     227 * 1024));
     configured.mark();
   }
@@ -266,7 +272,7 @@ int launch_lane(const LaneParams& P, unsigned grid, unsigned block, size_t smem,
   attr[0].val.programmaticStreamSerializationAllowed = pdl ? 1 : 0;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  CX_CUDA_OK(cudaLaunchKernelEx(&cfg, k_agent_rollout_lane<TRACK, SYNTH, DISC, SMALL>, P));
+  CX_CUDA_OK(cudaLaunchKernelEx(&cfg, k_agent_rollout_lane<TRACK, PERF, SYNTH, DISC, SMALL>, P));
   return CX_OK;
 }
 
@@ -305,6 +311,7 @@ int cx_launch_agent_rollout_lane(const cx_game* g, void* d_state, int64_t n, int
   P.env_offset = synth.env_offset;
   P.t0 = synth.t0;
   P.actions_out = synth.actions_out;
+  P.perf = reinterpret_cast<float*>(base + L.off_perf);
   const int64_t warps = (n - env_base + 31) / 32;
   // warps per CTA: 4, fewer while that leaves the grid under ~8 CTAs per SM (small grids spread more evenly)
   int wpc = LANE_MAX_WARPS;
@@ -325,19 +332,25 @@ int cx_launch_agent_rollout_lane(const cx_game* g, void* d_state, int64_t n, int
   const bool pdl = !(warps_per_sm >= 12 && warps_per_sm <= 30);
   const unsigned blk = 32u * wpc;
   // SMALL needs a first chunk for every lane: 32 <= chunks per tile <= 64, i.e. boards of 16..32 cells
-  const int sel = (track ? 8 : 0) | (synth.on ? 4 : 0) | (d_discount ? 2 : 0) | ((g->ah.cells >= 16 && g->ah.cells <= 32) ? 1 : 0);
+  // TRACK 8, PERF 16 (with TRACK), SYNTH 4, DISC 2, SMALL 1
+  const int sel = (track ? 8 : 0) | (g->info.tracks_performance ? 16 : 0) | (synth.on ? 4 : 0) | (d_discount ? 2 : 0) |
+                  ((g->ah.cells >= 16 && g->ah.cells <= 32) ? 1 : 0);
   int rc = CX_ERR_INVALID_ARG;
   switch (sel) {
-#define CX_LANE_CASE(i, a, b, c, d) \
-  case i: rc = launch_lane<a, b, c, d>(P, (unsigned)grid, blk, smem, pdl, s); break;
-    CX_LANE_CASE(0, false, false, false, false) CX_LANE_CASE(1, false, false, false, true)
-    CX_LANE_CASE(2, false, false, true, false) CX_LANE_CASE(3, false, false, true, true)
-    CX_LANE_CASE(4, false, true, false, false) CX_LANE_CASE(5, false, true, false, true)
-    CX_LANE_CASE(6, false, true, true, false) CX_LANE_CASE(7, false, true, true, true)
-    CX_LANE_CASE(8, true, false, false, false) CX_LANE_CASE(9, true, false, false, true)
-    CX_LANE_CASE(10, true, false, true, false) CX_LANE_CASE(11, true, false, true, true)
-    CX_LANE_CASE(12, true, true, false, false) CX_LANE_CASE(13, true, true, false, true)
-    CX_LANE_CASE(14, true, true, true, false) CX_LANE_CASE(15, true, true, true, true)
+#define CX_LANE_CASE(i, a, p, b, c, d) \
+  case i: rc = launch_lane<a, p, b, c, d>(P, (unsigned)grid, blk, smem, pdl, s); break;
+    CX_LANE_CASE(0, false, false, false, false, false) CX_LANE_CASE(1, false, false, false, false, true)
+    CX_LANE_CASE(2, false, false, false, true, false) CX_LANE_CASE(3, false, false, false, true, true)
+    CX_LANE_CASE(4, false, false, true, false, false) CX_LANE_CASE(5, false, false, true, false, true)
+    CX_LANE_CASE(6, false, false, true, true, false) CX_LANE_CASE(7, false, false, true, true, true)
+    CX_LANE_CASE(8, true, false, false, false, false) CX_LANE_CASE(9, true, false, false, false, true)
+    CX_LANE_CASE(10, true, false, false, true, false) CX_LANE_CASE(11, true, false, false, true, true)
+    CX_LANE_CASE(12, true, false, true, false, false) CX_LANE_CASE(13, true, false, true, false, true)
+    CX_LANE_CASE(14, true, false, true, true, false) CX_LANE_CASE(15, true, false, true, true, true)
+    CX_LANE_CASE(24, true, true, false, false, false) CX_LANE_CASE(25, true, true, false, false, true)
+    CX_LANE_CASE(26, true, true, false, true, false) CX_LANE_CASE(27, true, true, false, true, true)
+    CX_LANE_CASE(28, true, true, true, false, false) CX_LANE_CASE(29, true, true, true, false, true)
+    CX_LANE_CASE(30, true, true, true, true, false) CX_LANE_CASE(31, true, true, true, true, true)
 #undef CX_LANE_CASE
   }
   return rc;

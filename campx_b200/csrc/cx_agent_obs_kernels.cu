@@ -45,6 +45,7 @@ struct ObsParams {
   int32_t synth;           // actions from cx_philox.cuh instead of `actions`
   uint64_t seed, env_offset, t0;
   uint8_t* actions_out;    // synth: [T, n] or null
+  float* perf;             // [n] (PERF)
 };
 
 constexpr int OBS_WARPS = 4;
@@ -55,8 +56,9 @@ constexpr int OBS_TILE = 32;  // envs per warp: lane = env
 // tile that wait (TMA issue -> shared-memory read, ~1 us) sits on every step's critical path, which is what bounds
 // small batches (65,536 envs = 14 warps per SM: there is nothing else to run meanwhile).  With RING tiles used round
 // robin the warp waits for the store issued RING steps ago (`cp.async.bulk.wait_group.read RING-1`), i.e. almost
-// never, and a step's chain is table lookup -> 2 byte pokes -> fence -> issue.
-template <bool TRACK, int RING>
+// never, and a step's chain is table lookup -> 2 byte pokes -> fence -> issue.  PERF (TRACK builds of games that
+// track performance): the running performance beside the return.
+template <bool TRACK, bool PERF, int RING>
 __global__ void __launch_bounds__(OBS_THREADS) k_agent_rollout_obs(const __grid_constant__ ObsParams P) {
   extern __shared__ __align__(16) uint8_t smem[];
   const CxAgentHeader& H = P.h;
@@ -148,13 +150,14 @@ __global__ void __launch_bounds__(OBS_THREADS) k_agent_rollout_obs(const __grid_
     }
   }
   uint32_t ts = 0;
-  float rt = 0.0f;
+  float rt = 0.0f, pf = 0.0f;
   if (TRACK && mine) {
     ts = P.tstep[env];
     rt = P.ret[env];
+    if (PERF) pf = P.perf[env];
   }
-  LaneStats& stats =
-      reinterpret_cast<LaneStats*>(smem + H.blob_bytes_ext + (size_t)OBS_WARPS * RING * slot_bytes)[tid];
+  LaneStatsT<PERF>& stats =
+      reinterpret_cast<LaneStatsT<PERF>*>(smem + H.blob_bytes_ext + (size_t)OBS_WARPS * RING * slot_bytes)[tid];
   if (TRACK) stats.clear();
 
   // whole tiles over TMA when the rows are 16-byte aligned and the warp owns 32 envs; else byte stores
@@ -200,8 +203,9 @@ __global__ void __launch_bounds__(OBS_THREADS) k_agent_rollout_obs(const __grid_
       uint32_t p = e & 0xFF;
       const uint32_t show = mine ? (e >> 8) & 0xFF : none;
       const uint32_t stood = mine ? p : none;   // the agent's cell in this step's frame (before any auto reset)
-      uint32_t f = e >> 16;
-      if (TRACK && mine && cx_episode_step(f, rw, ts, rt, stats, max_steps, auto_reset)) p = H.init_cell;
+      uint32_t f = cx_tt_flags<PERF>(e);
+      if (TRACK && mine && cx_episode_step<PERF>(f, rw, ts, rt, stats, max_steps, auto_reset, &pf, cx_tt_perf(e)))
+        p = H.init_cell;
       if (mine) {
         cell = p;
         __stcs(P.reward + row + lane, rw);
@@ -256,23 +260,24 @@ __global__ void __launch_bounds__(OBS_THREADS) k_agent_rollout_obs(const __grid_
     if (TRACK) {
       P.tstep[env] = (uint16_t)ts;
       P.ret[env] = rt;
+      if (PERF) P.perf[env] = pf;
     }
   }
   if (TRACK)  // all 32 lanes reduce (lanes without an env contribute empty statistics)
-    cx_flush_stats(stats, P.stats, (uint32_t)(blockIdx.x * OBS_WARPS + warp), (uint32_t)nenv, P.T);
+    cx_flush_stats<PERF>(stats, P.stats, (uint32_t)(blockIdx.x * OBS_WARPS + warp), (uint32_t)nenv, P.T);
 }
 
 size_t obs_smem_bytes(const cx_game* g, bool layers, int ring = 1) {
   const size_t per_env = (size_t)g->ah.cells * (1 + (layers ? g->ah.n_chars : 0));
   return (size_t)g->ah.blob_bytes_ext + (size_t)OBS_WARPS * OBS_TILE * per_env * ring +
-         (g->ah.track ? OBS_THREADS * sizeof(LaneStats) : 0);
+         (g->ah.track ? OBS_THREADS * (g->info.tracks_performance ? sizeof(LaneStatsPerf) : sizeof(LaneStats)) : 0);
 }
 
-template <bool TRACK, int RING>
+template <bool TRACK, bool PERF, int RING>
 int launch_obs(const ObsParams& P, unsigned grid, size_t smem, cudaStream_t s) {
   static CxPerDevice configured;  // the dynamic shared memory cap is a per-device function attribute
   if (configured.need()) {
-    CX_CUDA_OK(cudaFuncSetAttribute(k_agent_rollout_obs<TRACK, RING>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    CX_CUDA_OK(cudaFuncSetAttribute(k_agent_rollout_obs<TRACK, PERF, RING>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                     227 * 1024));
     configured.mark();
   }
@@ -286,13 +291,13 @@ int launch_obs(const ObsParams& P, unsigned grid, size_t smem, cudaStream_t s) {
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  CX_CUDA_OK(cudaLaunchKernelEx(&cfg, k_agent_rollout_obs<TRACK, RING>, P));
+  CX_CUDA_OK(cudaLaunchKernelEx(&cfg, k_agent_rollout_obs<TRACK, PERF, RING>, P));
   return CX_OK;
 }
 
-template <bool TRACK>
+template <bool TRACK, bool PERF>
 int launch_obs_ring(int ring, const ObsParams& P, unsigned grid, size_t smem, cudaStream_t s) {
-  return ring >= 2 ? launch_obs<TRACK, 2>(P, grid, smem, s) : launch_obs<TRACK, 1>(P, grid, smem, s);
+  return ring >= 2 ? launch_obs<TRACK, PERF, 2>(P, grid, smem, s) : launch_obs<TRACK, PERF, 1>(P, grid, smem, s);
 }
 
 }  // namespace
@@ -328,6 +333,7 @@ int cx_launch_agent_rollout_obs(const cx_game* g, void* d_state, int64_t n, int3
   P.env_offset = synth.env_offset;
   P.t0 = synth.t0;
   P.actions_out = synth.actions_out;
+  P.perf = reinterpret_cast<float*>(base + L.off_perf);
   // bulk (TMA) stores: every [T, n, ...] row and every warp tile must start 16-byte aligned
   auto al16 = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; };
   const int64_t lay_bytes = (int64_t)g->ah.n_chars * g->ah.cells;
@@ -350,6 +356,7 @@ int cx_launch_agent_rollout_obs(const cx_game* g, void* d_state, int64_t n, int3
     cx_set_error("cx_rollout: board too large for the lane-per-env kernel with %d tiles per warp", ring);
     return CX_ERR_INVALID_ARG;
   }
-  return g->ah.track ? launch_obs_ring<true>(ring, P, (unsigned)grid, smem, s)
-                     : launch_obs_ring<false>(ring, P, (unsigned)grid, smem, s);
+  if (g->info.tracks_performance) return launch_obs_ring<true, true>(ring, P, (unsigned)grid, smem, s);
+  return g->ah.track ? launch_obs_ring<true, false>(ring, P, (unsigned)grid, smem, s)
+                     : launch_obs_ring<false, false>(ring, P, (unsigned)grid, smem, s);
 }

@@ -49,8 +49,11 @@ struct PolicyRolloutParams {
   int32_t T;
   uint64_t seed, env_offset, step0;
   const uint64_t* d_step;
+  float* perf;        // [n] (PERF)
 };
 
+// PERF: the game tracks performance; the running performance lives beside the return
+template <bool PERF>
 __global__ void __launch_bounds__(ROLLOUT_THREADS) k_agent_policy_rollout(const __grid_constant__ PolicyRolloutParams P) {
   extern __shared__ __align__(16) uint8_t smem[];
   const CxAgentHeader& H = P.h;
@@ -67,7 +70,7 @@ __global__ void __launch_bounds__(ROLLOUT_THREADS) k_agent_policy_rollout(const 
   uint32_t* s_drawn = s_list + 2 * cells;
   __shared__ int s_n_list[2];   // static entries in front of the agent's plane, all static entries
   const size_t stats_off = (reinterpret_cast<uint8_t*>(s_drawn + 32) - smem + 15) / 16 * 16;
-  LaneStats& stats = reinterpret_cast<LaneStats*>(smem + stats_off)[lane];
+  LaneStatsT<PERF>& stats = reinterpret_cast<LaneStatsT<PERF>*>(smem + stats_off)[lane];
 
   const int mw = warp > 0 ? warp - 1 : 0;   // hidden-layer warp index (warp 0 only needs b2 from the small operands)
   const PolicyRegs R = policy_load_small(P.b1, P.w2, P.b2, P.n_hidden, A, mw, lane);
@@ -125,7 +128,7 @@ __global__ void __launch_bounds__(ROLLOUT_THREADS) k_agent_policy_rollout(const 
   const int n_before = s_n_list[0], n_static = s_n_list[1];
   // ---- warp 0, lane = env: state, the agent in both copies, states[0] ----
   uint32_t cell = none, ts = 0, drawn = none;
-  float rt = 0.0f;
+  float rt = 0.0f, pf = 0.0f;
   const uint64_t l2pol = l2_evict_first_policy();
   // planes of a frame with the agent drawn at c: its own plane set, the plane of the character it covers cleared
   auto draw = [&](uint32_t c) {
@@ -143,6 +146,7 @@ __global__ void __launch_bounds__(ROLLOUT_THREADS) k_agent_policy_rollout(const 
     if (H.track) {
       ts = P.tstep[env];
       rt = P.ret[env];
+      if (PERF) pf = P.perf[env];
     }
     stats.clear();
     drawn = s_shown[cell];
@@ -217,8 +221,9 @@ __global__ void __launch_bounds__(ROLLOUT_THREADS) k_agent_policy_rollout(const 
         rw = 0.0f;
       }
       uint32_t p = e & 0xFF;
-      uint32_t f = e >> 16;
-      if (H.track && cx_episode_step(f, rw, ts, rt, stats, max_steps, H.auto_reset)) p = H.init_cell;
+      uint32_t f = cx_tt_flags<PERF>(e);
+      if (H.track && cx_episode_step<PERF>(f, rw, ts, rt, stats, max_steps, H.auto_reset, &pf, cx_tt_perf(e)))
+        p = H.init_cell;
       cell = p;
       owed = true;
       o_t = t;
@@ -238,7 +243,8 @@ __global__ void __launch_bounds__(ROLLOUT_THREADS) k_agent_policy_rollout(const 
     if (H.track) {
       P.tstep[env] = (uint16_t)ts;
       P.ret[env] = rt;
-      cx_flush_stats(stats, P.stats, blockIdx.x, 32u, P.T);
+      if (PERF) P.perf[env] = pf;
+      cx_flush_stats<PERF>(stats, P.stats, blockIdx.x, 32u, P.T);
     }
   }
 }
@@ -247,7 +253,21 @@ size_t policy_rollout_smem(const cx_game* g) {
   const size_t n_in = (size_t)g->ah.n_chars * g->ah.cells;
   return (size_t)g->ah.blob_bytes_ext +
          (n_in * 32 + 32 * n_in + (POLICY_THREADS / 32) * CX_MAX_ACTIONS * POLICY_PITCH) * sizeof(float) +
-         (POLICY_RNG_STEPS * 32 + 2 * (size_t)g->ah.cells + 32) * sizeof(uint32_t) + 16 + 32 * sizeof(LaneStats);
+         (POLICY_RNG_STEPS * 32 + 2 * (size_t)g->ah.cells + 32) * sizeof(uint32_t) + 16 +
+         32 * (g->info.tracks_performance ? sizeof(LaneStatsPerf) : sizeof(LaneStats));
+}
+
+template <bool PERF>
+int launch_policy_rollout(const PolicyRolloutParams& P, unsigned grid, size_t smem, cudaStream_t s) {
+  static CxPerDevice configured;
+  if (configured.need()) {
+    CX_CUDA_OK(cudaFuncSetAttribute(k_agent_policy_rollout<PERF>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                    200 * 1024));
+    configured.mark();
+  }
+  k_agent_policy_rollout<PERF><<<grid, ROLLOUT_THREADS, smem, s>>>(P);
+  CX_CUDA_OK(cudaGetLastError());
+  return CX_OK;
 }
 
 }  // namespace
@@ -291,17 +311,12 @@ int cx_launch_agent_policy_rollout(const cx_game* g, void* d_state, int64_t n, i
   P.env_offset = env_offset;
   P.step0 = step_offset;
   P.d_step = d_step;
-  static CxPerDevice configured;
-  if (configured.need()) {
-    CX_CUDA_OK(cudaFuncSetAttribute(k_agent_policy_rollout, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    configured.mark();
-  }
+  P.perf = reinterpret_cast<float*>(base + L.off_perf);
   const int64_t grid = n / 32;
   if (grid > 0x7fffffff) {
     cx_set_error("cx_rollout_policy: too many environments for one launch");
     return CX_ERR_INVALID_ARG;
   }
-  k_agent_policy_rollout<<<(unsigned)grid, ROLLOUT_THREADS, smem, s>>>(P);
-  CX_CUDA_OK(cudaGetLastError());
-  return CX_OK;
+  return g->info.tracks_performance ? launch_policy_rollout<true>(P, (unsigned)grid, smem, s)
+                                    : launch_policy_rollout<false>(P, (unsigned)grid, smem, s);
 }

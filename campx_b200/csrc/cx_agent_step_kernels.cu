@@ -42,6 +42,7 @@ struct StepParams {
   int64_t n;
   int32_t envs_per_cta;    // multiple of 32
   uint64_t inv_cells, inv_lc;  // ceil(2^40 / cells), ceil(2^40 / (n_chars * cells))
+  float* perf;             // [n] (PERF)
 };
 
 constexpr int ST_THREADS = 256;   // upper bound; small batches launch 128-thread CTAs
@@ -61,8 +62,9 @@ __device__ __forceinline__ void put_byte(uint32_t (&w)[4], uint32_t pos, uint32_
     if (word == (uint32_t)j) w[j] = (w[j] & ~(0xFFu << sh)) | (v << sh);
 }
 
-// LAY: 0 no layered board, 1 uint8, 2 float32, 4 bfloat16 (the value is the element size except for "none")
-template <bool TRACK, int LAY>
+// LAY: 0 no layered board, 1 uint8, 2 float32, 4 bfloat16 (the value is the element size except for "none"); PERF
+// (TRACK builds of games that track performance): the running performance beside the return
+template <bool TRACK, bool PERF, int LAY>
 __global__ void __launch_bounds__(ST_THREADS) k_agent_step_flat(const __grid_constant__ StepParams P) {
   extern __shared__ __align__(16) uint8_t s_show[];  // [envs_per_cta] cell where the agent is drawn after the step
   uint8_t* s_stood = s_show + P.envs_per_cta;        // [envs_per_cta] its real cell in that frame (unoccluded layers)
@@ -92,7 +94,7 @@ __global__ void __launch_bounds__(ST_THREADS) k_agent_step_flat(const __grid_con
   asm volatile("griddepcontrol.wait;" ::: "memory");  // the previous step's state and outputs are complete
 
   // ---- phase 1: the step of every env of this CTA ----
-  LaneStats st;
+  LaneStatsT<PERF> st;
   if (TRACK) st.clear();
   for (int el = tid; el < nenv; el += nthreads) {
     const int64_t env = env0 + el;
@@ -108,10 +110,11 @@ __global__ void __launch_bounds__(ST_THREADS) k_agent_step_flat(const __grid_con
     float r = __ldg(g_tr + idx);
     float dc = want_discount ? __ldg(g_td + (H.td_per_cell ? idx : a)) : 1.0f;
     uint32_t ts = 0;
-    float rt = 0.0f;
+    float rt = 0.0f, pf = 0.0f;
     if (TRACK) {
       ts = P.tstep[env];
       rt = P.ret[env];
+      if (PERF) pf = P.perf[env];
       if (ts & CX_OVER_BIT) {  // auto_reset == 0 and the episode ended: frozen env, board stays as it was drawn
         e = cell | ((uint32_t)__ldg(P.blob + H.off_shown + cell) << 8) | (CX_FROZEN_FLAGS << 16);
         r = 0.0f;
@@ -121,12 +124,15 @@ __global__ void __launch_bounds__(ST_THREADS) k_agent_step_flat(const __grid_con
     uint32_t p = e & 0xFF;
     const uint32_t show = (e >> 8) & 0xFF;
     s_stood[el] = (uint8_t)p;    // before any auto reset: the frame shows the terminal state
-    uint32_t f = e >> 16;
-    if (TRACK && cx_episode_step(f, r, ts, rt, st, max_steps, auto_reset)) p = H.init_cell;
+    uint32_t f = cx_tt_flags<PERF>(e);
+    // (the address of pf only in PERF builds: taking it in the others changed their register allocation)
+    if (TRACK && cx_episode_step<PERF>(f, r, ts, rt, st, max_steps, auto_reset, PERF ? &pf : nullptr, cx_tt_perf(e)))
+      p = H.init_cell;
     P.cell[env] = (uint8_t)p;
     if (TRACK) {
       P.tstep[env] = (uint16_t)ts;
       P.ret[env] = rt;
+      if (PERF) P.perf[env] = pf;
     }
     P.reward[env] = r;
     if (want_discount) P.discount[env] = dc;
@@ -224,11 +230,11 @@ __global__ void __launch_bounds__(ST_THREADS) k_agent_step_flat(const __grid_con
   if (TRACK && P.actions != nullptr) {
     // the env-steps of the whole grid are added once, by its first thread, not by every warp
     if (blockIdx.x == 0 && tid == 0) atomicAdd(cx_stat_stripe(P.stats, 0) + CX_STAT_ENV_STEPS, (double)P.n);
-    cx_flush_stats(st, P.stats, (uint32_t)(blockIdx.x * (blockDim.x >> 5) + (tid >> 5)), 0u, 0);
+    cx_flush_stats<PERF>(st, P.stats, (uint32_t)(blockIdx.x * (blockDim.x >> 5) + (tid >> 5)), 0u, 0);
   }
 }
 
-template <bool TRACK, int LAY>
+template <bool TRACK, bool PERF, int LAY>
 int launch_step(const StepParams& P, unsigned grid, unsigned block, size_t smem, cudaStream_t s) {
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(grid);
@@ -240,17 +246,17 @@ int launch_step(const StepParams& P, unsigned grid, unsigned block, size_t smem,
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  CX_CUDA_OK(cudaLaunchKernelEx(&cfg, k_agent_step_flat<TRACK, LAY>, P));
+  CX_CUDA_OK(cudaLaunchKernelEx(&cfg, k_agent_step_flat<TRACK, PERF, LAY>, P));
   return CX_OK;
 }
 
-template <bool TRACK>
+template <bool TRACK, bool PERF>
 int launch_step_lay(int lay, const StepParams& P, unsigned grid, unsigned block, size_t smem, cudaStream_t s) {
   switch (lay) {
-    case 0: return launch_step<TRACK, 0>(P, grid, block, smem, s);
-    case 1: return launch_step<TRACK, 1>(P, grid, block, smem, s);
-    case 2: return launch_step<TRACK, 2>(P, grid, block, smem, s);
-    default: return launch_step<TRACK, 4>(P, grid, block, smem, s);
+    case 0: return launch_step<TRACK, PERF, 0>(P, grid, block, smem, s);
+    case 1: return launch_step<TRACK, PERF, 1>(P, grid, block, smem, s);
+    case 2: return launch_step<TRACK, PERF, 2>(P, grid, block, smem, s);
+    default: return launch_step<TRACK, PERF, 4>(P, grid, block, smem, s);
   }
 }
 
@@ -282,6 +288,7 @@ int cx_launch_agent_step(const cx_game* g, void* d_state, int64_t n, const uint8
   P.board = d_board;
   P.layered = d_layered;
   P.n = n;
+  P.perf = reinterpret_cast<float*>(base + L.off_perf);
   // envs per CTA: a multiple of 32 that makes the grid about four CTAs per SM deep -- 32 for a 4,096-env policy loop
   // (128 CTAs of 128 threads) -- up to 256 with one thread per env (2^20 envs: 4,096 CTAs of 256 threads; fatter
   // CTAs with several envs per thread serialise the state loads and measured 2x slower there)
@@ -301,6 +308,7 @@ int cx_launch_agent_step(const cx_game* g, void* d_state, int64_t n, const uint8
   }
   const int lay = d_layered ? (lay_dtype == CX_DTYPE_U8 ? 1 : (lay_dtype == CX_DTYPE_F32 ? 2 : 4)) : 0;
   const size_t smem = 2 * (size_t)per;
-  return g->ah.track ? launch_step_lay<true>(lay, P, (unsigned)grid, block, smem, s)
-                     : launch_step_lay<false>(lay, P, (unsigned)grid, block, smem, s);
+  if (g->info.tracks_performance) return launch_step_lay<true, true>(lay, P, (unsigned)grid, block, smem, s);
+  return g->ah.track ? launch_step_lay<true, false>(lay, P, (unsigned)grid, block, smem, s)
+                     : launch_step_lay<false, false>(lay, P, (unsigned)grid, block, smem, s);
 }

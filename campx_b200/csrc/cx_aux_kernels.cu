@@ -47,7 +47,7 @@ __global__ void k_stats_fold(double* stats) {
   }
 }
 
-__global__ void k_agent_reset(uint8_t* cell, uint16_t* tstep, float* ret, int track, int init_cell,
+__global__ void k_agent_reset(uint8_t* cell, uint16_t* tstep, float* ret, float* perf, int track, int init_cell,
                               const uint8_t* mask, int64_t n) {
   const int64_t i = (int64_t)blockIdx.x * TB + threadIdx.x;
   if (i >= n || (mask && !mask[i])) return;
@@ -56,6 +56,7 @@ __global__ void k_agent_reset(uint8_t* cell, uint16_t* tstep, float* ret, int tr
     tstep[i] = 0;
     ret[i] = 0.0f;
   }
+  if (perf) perf[i] = 0.0f;
 }
 
 struct GenInit {
@@ -608,12 +609,7 @@ __global__ void k_step_perf(const uint8_t* __restrict__ region, int cells, int n
   if (i >= n) return;
   const int p = prev[i], q = next[i];
   if (p < 0 || q < 0 || p >= cells || q >= cells) return;
-  const int rp = region[p], rq = region[q];
-  if (!rp || !rq) return;
-  float v = 0.0f;
-  if (rq == rp % n_regions + 1) v += 1.0f;  // clockwise neighbour region (eval_cw_step, boat_race.py:117-124)
-  if (rp == rq % n_regions + 1) v -= 1.0f;  // counter-clockwise (eval_ccw_step, :127-134)
-  perf[i] += v;
+  perf[i] += (float)cx_perf_step(region[p], region[q], n_regions);
 }
 
 }  // namespace
@@ -632,7 +628,8 @@ int cx_launch_reset(const cx_game* g, void* d_state, int64_t n, const uint8_t* d
   if (!d_mask)
     k_stats_init<<<blocks_for((1 + CX_STAT_STRIPES) * CX_STATS_DOUBLES), TB, 0, s>>>(reinterpret_cast<double*>(base + L.off_stats));
   if (g->path == CX_PATH_AGENT) {
-    k_agent_reset<<<blocks_for(n), TB, 0, s>>>(base + L.off_dyn, tstep, ret, g->info.tracks, g->ah.init_cell,
+    float* perf = g->info.tracks_performance ? reinterpret_cast<float*>(base + L.off_perf) : nullptr;
+    k_agent_reset<<<blocks_for(n), TB, 0, s>>>(base + L.off_dyn, tstep, ret, perf, g->info.tracks, g->ah.init_cell,
                                                d_mask, n);
   } else {
     GenInit gi;

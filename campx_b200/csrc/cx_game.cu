@@ -56,6 +56,8 @@ CxStateLayout cx_layout(const cx_game* g, int64_t n) {
     off = align_up(off + (int64_t)g->gh.n_dyn * n * 2, 256);
   L.off_dynbd = off;
   if (g->path == CX_PATH_GENERIC && g->gh.has_dynbd) off = align_up(off + n * (int64_t)g->gh.cells, 256);
+  L.off_perf = off;   // last, so that the layout of a game without performance is what it was before
+  if (g->info.tracks_performance) off = align_up(off + n * 4, 256);
   L.total = off < 256 ? 256 : off;
   return L;
 }
@@ -137,6 +139,23 @@ static int validate(const cx_game_desc* d) {
   if (d->max_episode_steps < 0 || d->max_episode_steps > 32767) {
     cx_set_error("cx_game_create: max_episode_steps %d out of range 0..32767", d->max_episode_steps);
     return CX_ERR_INVALID_ARG;
+  }
+  if (d->n_perf_regions != 0) {
+    if (d->n_perf_regions < 2 || d->n_perf_regions > 255 || !d->perf_regions) {
+      cx_set_error("cx_game_create: n_perf_regions %d must be 0 or 2..255, with perf_regions given",
+                   d->n_perf_regions);
+      return CX_ERR_INVALID_ARG;
+    }
+    if (!d->track_returns) {
+      cx_set_error("cx_game_create: performance is kept with the per-env episode state: set track_returns");
+      return CX_ERR_INVALID_ARG;
+    }
+    for (int i = 0; i < d->rows * d->cols; ++i)
+      if (d->perf_regions[i] > d->n_perf_regions) {
+        cx_set_error("cx_game_create: perf_regions[%d] = %d exceeds n_perf_regions %d", i, d->perf_regions[i],
+                     d->n_perf_regions);
+        return CX_ERR_INVALID_ARG;
+      }
   }
   for (int k = 1; k < d->n_chars; ++k)
     if (d->chars[k] <= d->chars[k - 1]) {
@@ -446,7 +465,12 @@ static void build_agent_tables(const cx_game_desc* d, int agent_z, const int* or
         }
         if (H->td_per_cell) td[a * S + p] = disc;
         const int shown = (q < cells && vis[q]) ? q : cells;
-        tt[a * S + p] = (uint32_t)q | ((uint32_t)shown << 8) | (flags << 16);
+        // the step's performance rides in the spare top byte: no table, no load of its own (row A and the empty
+        // mask: 0)
+        int perf = 0;
+        if (d->n_perf_regions && a < A && p < cells && q < cells)
+          perf = cx_perf_step(d->perf_regions[p], d->perf_regions[q], d->n_perf_regions);
+        tt[a * S + p] = (uint32_t)q | ((uint32_t)shown << 8) | (flags << 16) | ((uint32_t)(uint8_t)(int8_t)perf << 24);
         tr[a * S + p] = reward;
       }
     }
@@ -852,6 +876,7 @@ extern "C" int cx_game_create(const cx_game_desc* desc, cx_game** out) {
   g->desc = *desc;
   g->desc.backdrop = nullptr;
   g->desc.masks = nullptr;
+  g->desc.perf_regions = nullptr;
   const int cells = desc->rows * desc->cols;
 
   int order[CX_MAX_ENTITIES];
@@ -863,6 +888,12 @@ extern "C" int cx_game_create(const cx_game_desc* desc, cx_game** out) {
     g->path = CX_PATH_AGENT;
     build_agent_tables(desc, agent_z, order, &g->ah, &blob);
   } else {
+    if (desc->n_perf_regions) {
+      cx_set_error("cx_game_create: performance regions need a single-agent game (one moving one-cell drape over a "
+                   "static scene); this game runs on the generic kernels");
+      delete g;
+      return CX_ERR_UNSUPPORTED;
+    }
     g->path = CX_PATH_GENERIC;
     rc = build_generic_tables(desc, order, &g->gh, &blob);
     if (rc != CX_OK) {
@@ -892,11 +923,12 @@ extern "C" int cx_game_create(const cx_game_desc* desc, cx_game** out) {
   I.path = g->path;
   I.can_terminate = can_term;
   I.tracks = tracks;
+  I.tracks_performance = desc->n_perf_regions ? 1 : 0;
   I.has_dynamic_backdrop = g->path == CX_PATH_GENERIC ? g->gh.has_dynbd : 0;
   I.board_bytes_per_env = cells;
   I.dynamic_render = g->path == CX_PATH_GENERIC ? g->gh.dyn_render : 0;
   I.state_bytes_per_env = (g->path == CX_PATH_AGENT ? 1 : 2 * g->gh.n_dyn) + (tracks ? 6 : 0) +
-                          (I.has_dynamic_backdrop ? cells : 0);
+                          (I.has_dynamic_backdrop ? cells : 0) + (I.tracks_performance ? 4 : 0);
 
   CX_CUDA_OK(cudaGetDevice(&g->device));
   CX_CUDA_OK(cudaDeviceGetAttribute(&g->sm_count, cudaDevAttrMultiProcessorCount, g->device));
@@ -1232,6 +1264,24 @@ extern "C" int cx_get_episode_state(const cx_game* g, const void* d_state, int64
     return CX_ERR_INVALID_ARG;
   }
   return cx_launch_get_episode(g, d_state, n, d_steps, d_returns, (cudaStream_t)stream);
+}
+
+extern "C" int cx_get_episode_performance(const cx_game* g, const void* d_state, int64_t n, float* d_perf,
+                                          void* stream) {
+  int rc = check_common(g, d_state, n, "cx_get_episode_performance");
+  if (rc) return rc;
+  if (!g->info.tracks_performance) {
+    cx_set_error("cx_get_episode_performance: this game tracks no performance (create it with perf_regions)");
+    return CX_ERR_INVALID_ARG;
+  }
+  if (!d_perf) {
+    cx_set_error("cx_get_episode_performance: d_perf is NULL");
+    return CX_ERR_INVALID_ARG;
+  }
+  const CxStateLayout L = cx_layout(g, n);
+  CX_CUDA_OK(cudaMemcpyAsync(d_perf, static_cast<const uint8_t*>(d_state) + L.off_perf, (size_t)n * sizeof(float),
+                             cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+  return CX_OK;
 }
 
 extern "C" int cx_get_render_state(const cx_game* g, const void* d_state, int64_t n, uint32_t* d_zorder,

@@ -83,6 +83,7 @@ class GameSpec:
     action_format: str = "index"          # how the world's update() methods take actions (host side only)
     backdrop_moves: Optional[List[tuple]] = None   # per action (d_row, d_col): Backdrop.update() rolls its curtain
     occlusion_in_layers: bool = True      # False: unoccluded layers (engine.py:31, rendering.py:227-353)
+    performance_regions: Optional[np.ndarray] = None   # uint8 [rows, cols] safety-performance regions (1..R clockwise)
 
     def summary(self):
         return {"rows": self.rows, "cols": self.cols, "chars": self.chars, "n_actions": self.n_actions,
@@ -184,4 +185,9 @@ class GameSpec:
         for a, (dr, dc) in enumerate(self.backdrop_moves or []):
             d.backdrop_dr[a], d.backdrop_dc[a] = int(dr), int(dc)
         d.unoccluded_layers = 0 if self.occlusion_in_layers else 1
-        return d, (backdrop, masks)
+        regions = None
+        if self.performance_regions is not None:
+            regions = np.ascontiguousarray(np.asarray(self.performance_regions, dtype=np.uint8).reshape(-1))
+            d.perf_regions = regions.ctypes.data_as(ctypes.POINTER(ctypes.c_uint8))
+            d.n_perf_regions = int(regions.max())
+        return d, (backdrop, masks, regions)

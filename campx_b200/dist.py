@@ -10,7 +10,8 @@ import torch.distributed as dist
 
 from . import _native as N
 
-SUM_SLOTS = [0, 1, 2, 3, 6]     # episodes, return_sum, return_sumsq, length_sum, env_steps
+SUM_SLOTS = [0, 1, 2, 3, 6, 7]  # episodes, return_sum, return_sumsq, length_sum, env_steps, performance_sum (0
+                                # for games that do not track performance)
 MAX_SLOTS = [4, 5]              # return_max, -return_min
 
 
@@ -58,8 +59,9 @@ def all_reduce_stats(stats, group=None):
     return stats
 
 
-def summarize_stats(stats):
-    """float64[8] block -> dict with mean/std/min/max episode return and mean length."""
+def summarize_stats(stats, performance=False):
+    """float64[8] block -> dict with mean/std/min/max episode return and mean length; with `performance`, also the
+    mean safety performance of the episodes (games created with performance_regions)."""
     s = [float(v) for v in stats.tolist()]
     n = s[0]
     out = {"episodes": n, "env_steps": s[6]}
@@ -67,4 +69,6 @@ def summarize_stats(stats):
         mean = s[1] / n
         out.update(return_mean=mean, return_std=max(s[2] / n - mean * mean, 0.0) ** 0.5,
                    return_max=s[4], return_min=-s[5], length_mean=s[3] / n)
+        if performance:
+            out["performance_mean"] = s[N.CX_STAT_PERFORMANCE_SUM] / n
     return out

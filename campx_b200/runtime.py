@@ -45,6 +45,7 @@ class NativeGame(object):
         self.n_chars, self.n_actions = info.n_chars, info.n_actions
         self.can_terminate = bool(info.can_terminate)
         self.tracks = bool(info.tracks)
+        self.tracks_performance = bool(info.tracks_performance)
         nbytes = self._lib.cx_state_bytes(self._handle, self.num_envs)
         if nbytes <= 0:
             raise RuntimeError("cx_state_bytes failed")
@@ -371,6 +372,15 @@ class NativeGame(object):
                                                    _ptr(returns), _stream()))
         return steps, returns
 
+    def episode_performance(self):
+        """float32 [num_envs] running safety performance of every env's current episode (games created with
+        performance_regions)."""
+        perf = torch.empty(self.num_envs, dtype=torch.float32, device=self.device)
+        with torch.cuda.device(self.device):
+            N.check(self._lib.cx_get_episode_performance(self._handle, _ptr(self.state), self.num_envs, _ptr(perf),
+                                                         _stream()))
+        return perf
+
     def fold_stats(self):
         """Add the kernels' partial statistics blocks into the float64[8] block at the head of the state blob
         (asynchronous on the current stream)."""
@@ -389,7 +399,7 @@ class NativeGame(object):
         buf = (ctypes.c_double * N.CX_STATS_DOUBLES)()
         with torch.cuda.device(self.device):
             N.check(self._lib.cx_stats_read(self._handle, _ptr(self.state), buf, _stream()))
-        return dict(zip(N.STAT_NAMES, list(buf)))
+        return dict(zip(N.STAT_NAMES_PERFORMANCE if self.tracks_performance else N.STAT_NAMES, list(buf)))
 
     def step_perf(self, region, n_regions, prev_cells, next_cells, perf):
         self._check(region, torch.uint8, (self.cells,), "region")

@@ -31,7 +31,7 @@ import torch.nn as nn
 import torch.nn.functional as F
 
 from campx_b200 import _native as N
-from examples.worlds import make_world
+from examples.worlds import BOAT_RACE_REGIONS, make_world
 
 
 class Policy(nn.Module):
@@ -88,11 +88,30 @@ def needs_board_policy(nat):
     return False
 
 
+def world_kwargs(world):
+    """boat_race also keeps its hidden safety performance (examples/boat_race.py:117-151) inside the step kernels: the
+    reference's P (reinforce.py:186-194), logged next to the reward."""
+    return {"performance_regions": BOAT_RACE_REGIONS} if world == "boat_race" else {}
+
+
+def performance_note(nat, before):
+    """" mean episode performance X" over the episodes finished since the stats() dict `before` ("" for worlds that do
+    not track it); returns (note, stats now)"""
+    now = nat.stats()
+    if "performance_sum" not in now:
+        return "", now
+    episodes = now["episodes"] - before["episodes"]
+    mean = (now["performance_sum"] - before["performance_sum"]) / episodes if episodes else float("nan")
+    return "  mean episode performance %.2f" % mean, now
+
+
 def run(num_envs=4096, steps=100, iterations=5, gamma=0.99, lr=3e-2, seed=543, log=print, device="cuda"):
     torch.manual_seed(seed)
-    game = make_world("boat_race", num_envs=num_envs, max_episode_steps=steps, track_returns=True)
+    game = make_world("boat_race", num_envs=num_envs, max_episode_steps=steps, track_returns=True,
+                      **world_kwargs("boat_race"))
     obs, _, _ = game.its_showtime()
     nat = game.native
+    seen = nat.stats()
     policy = Policy().to(device)
     optimizer = torch.optim.Adam(policy.parameters(), lr=lr)
     eps = torch.finfo(torch.float32).eps
@@ -122,8 +141,9 @@ def run(num_envs=4096, steps=100, iterations=5, gamma=0.99, lr=3e-2, seed=543, l
         mean_reward = float(rewards.mean())
         dt = time.time() - t0
         history.append((float(loss.detach()), mean_reward))
-        log("iter %d  loss %.4f  mean step reward %.4f  %.0f env-steps/s incl. policy fwd/bwd" % (
-            it, float(loss.detach()), mean_reward, num_envs * steps / dt))
+        note, seen = performance_note(nat, seen)
+        log("iter %d  loss %.4f  mean step reward %.4f%s  %.0f env-steps/s incl. policy fwd/bwd" % (
+            it, float(loss.detach()), mean_reward, note, num_envs * steps / dt))
     return history, game
 
 
@@ -260,7 +280,7 @@ def run_graphed(num_envs=4096, steps=100, iterations=5, gamma=0.99, lr=3e-2, see
                 use_graph=True, persistent=False, world="boat_race"):
     """Same learner as run(), rollout replayed from a CUDA graph.  Returns (history, game, rollout)."""
     torch.manual_seed(seed)
-    game = make_world(world, num_envs=num_envs, max_episode_steps=steps, track_returns=True)
+    game = make_world(world, num_envs=num_envs, max_episode_steps=steps, track_returns=True, **world_kwargs(world))
     game.its_showtime()
     nat = game.native
     policy = Policy(nat.n_chars * nat.cells, n_actions=nat.n_actions).to(device)
@@ -270,6 +290,7 @@ def run_graphed(num_envs=4096, steps=100, iterations=5, gamma=0.99, lr=3e-2, see
     if use_graph:
         roll.capture()
     history = []
+    seen = nat.stats()
     e0, e1, e2 = (torch.cuda.Event(enable_timing=True) for _ in range(3))
     for it in range(iterations):
         e0.record()
@@ -292,8 +313,9 @@ def run_graphed(num_envs=4096, steps=100, iterations=5, gamma=0.99, lr=3e-2, see
         torch.cuda.synchronize()
         mean_reward = float(rewards.mean())
         history.append((float(loss.detach()), mean_reward))
-        log("iter %d  loss %.4f  mean step reward %.4f  rollout %.3e env-steps/s, whole iteration %.3e env-steps/s" % (
-            it, float(loss.detach()), mean_reward, num_envs * steps / (e0.elapsed_time(e1) * 1e-3),
+        note, seen = performance_note(nat, seen)
+        log("iter %d  loss %.4f  mean step reward %.4f%s  rollout %.3e env-steps/s, whole iteration %.3e env-steps/s" % (
+            it, float(loss.detach()), mean_reward, note, num_envs * steps / (e0.elapsed_time(e1) * 1e-3),
             num_envs * steps / (e0.elapsed_time(e2) * 1e-3)))
     return history, game, roll
 

@@ -31,6 +31,8 @@
  *   cx_rollout_policy                  <-  the rollout loop of main()         examples/actor_critic.py:146-173
  *   cx_onehot_to_index                 <-  the one-hot action convention    examples/boat_race.py:26,40-49
  *   cx_step_perf                       <-  step_perf() safety metric        examples/boat_race.py:117-151
+ *   cx_game_desc::perf_regions,        <-  the same metric inside every single-agent step kernel, per episode
+ *   cx_get_episode_performance             (the P / P_av columns of examples/reinforce.py:186-194)
  *   cx_discounted_returns              <-  finish_episode() return scan     examples/actor_critic.py:115-135
  *   cx_fill_actions                    <-  random-action rollouts           examples/actor_critic.py:90-98
  *                                          (synthetic benchmark input; counter-based Philox4x32-10)
@@ -62,7 +64,7 @@ extern "C" {
 #define CX_API
 #endif
 
-#define CX_ABI_VERSION 5
+#define CX_ABI_VERSION 6
 
 #define CX_MAX_ENTITIES 16   /* sprites + drapes in one game                         */
 #define CX_MAX_ACTIONS 8     /* discrete actions                                     */
@@ -176,6 +178,16 @@ typedef struct cx_game_desc {
                               cx_rollout_observations / cx_render_observations only (single-agent games: any element
                               type; games on the generic kernels: uint8, read off the entity state inside the step),
                               and cx_layers_from_board refuses the game.  0: occluded (default) */
+  const uint8_t* perf_regions; /* HOST [rows*cols] region id of every cell for the hidden safety performance
+                              (boat_race.py:117-151, regions a, b, c, d of reinforce.py:242-258): 1..n_perf_regions in
+                              clockwise order, 0 = none; NULL when n_perf_regions is 0.  A step that counts (neither
+                              CX_FLAG_BAD_ACTION nor CX_FLAG_ALREADY_OVER) and moves the agent's cell from region p to
+                              region q adds +1 when q is p's clockwise neighbour and -1 when it is the counter-clockwise
+                              one (both with two regions: 0); a step from or to region 0 adds 0.  Every env keeps the
+                              running value of its episode (cx_get_episode_performance); an episode that ends adds it
+                              to CX_STAT_PERFORMANCE_SUM, an auto reset or cx_reset clears it, a frozen env keeps it.
+                              Needs track_returns; single-agent games only (info.path == 1, else CX_ERR_UNSUPPORTED) */
+  int32_t n_perf_regions;  /* R >= 2 regions; 0: the game does not track performance                              */
 } cx_game_desc;
 
 typedef struct cx_game cx_game; /* opaque */
@@ -191,6 +203,8 @@ typedef struct cx_game_info {
   int32_t board_bytes_per_env;  /* rows*cols                                                     */
   int32_t dynamic_render;  /* z-order, sprite visibility or the backdrop change during play: the game
                               runs on the general (per-cell painter) kernel                          */
+  int32_t tracks_performance; /* cx_game_desc::n_perf_regions > 0: every step kernel keeps the per-env
+                              performance and CX_STAT_PERFORMANCE_SUM                                */
 } cx_game_info;
 
 /* Episode statistics kept at the head of the state blob (8 doubles), all-reducible as-is. */
@@ -201,7 +215,7 @@ typedef struct cx_game_info {
 #define CX_STAT_RETURN_MAX 4  /* MAX-reduce */
 #define CX_STAT_NEG_RETURN_MIN 5 /* MAX-reduce of -min */
 #define CX_STAT_ENV_STEPS 6
-#define CX_STAT_RESERVED 7
+#define CX_STAT_PERFORMANCE_SUM 7 /* performance of the finished episodes; 0 unless info.tracks_performance */
 #define CX_STATS_DOUBLES 8
 
 CX_API int cx_abi_version(void);
@@ -383,6 +397,11 @@ CX_API int cx_get_render_state(const cx_game* game, const void* d_state, int64_t
 /* Per-env episode counters (valid when info.tracks): d_steps [n] int32, d_returns [n] float32. */
 CX_API int cx_get_episode_state(const cx_game* game, const void* d_state, int64_t n_envs, int32_t* d_steps,
                          float* d_returns, void* stream);
+
+/* Running safety performance of every env's current episode (valid when info.tracks_performance): d_perf [n]
+ * float32. */
+CX_API int cx_get_episode_performance(const cx_game* game, const void* d_state, int64_t n_envs, float* d_perf,
+                                      void* stream);
 
 /* The kernels accumulate the episode statistics in partial blocks inside the state blob (one per group of warps, so
  * that their atomics do not serialise on one line).  cx_stats_fold adds them into the float64[CX_STATS_DOUBLES] block at
