@@ -7,7 +7,7 @@ compute entry point is needed, this module raises.  The library is built in-tree
 import ctypes
 import os
 
-CX_ABI_VERSION = 6
+CX_ABI_VERSION = 7
 CX_MAX_ENTITIES = 16
 CX_MAX_ACTIONS = 8
 CX_MAX_CHARS = 32
@@ -21,7 +21,8 @@ CX_ERR_UNSUPPORTED = -2
 CX_ERR_CUDA = -3
 CX_ERR_NOMEM = -4
 
-CX_KIND_STATIC, CX_KIND_CELL, CX_KIND_ROLL, CX_KIND_SPRITE = 0, 1, 2, 3
+CX_KIND_STATIC, CX_KIND_CELL, CX_KIND_ROLL, CX_KIND_SPRITE, CX_KIND_PICKUP = 0, 1, 2, 3, 4
+CX_MAX_PICKUPS = 64          # item cells of all pickup drapes of one game
 CX_VIS_KEEP, CX_VIS_SHOW, CX_VIS_HIDE, CX_VIS_TOGGLE = 0, 1, 2, 3
 
 CX_FLAG_TERMINATED = 0x01
@@ -73,6 +74,8 @@ class EntityDesc(ctypes.Structure):
         ("n_zdirs", ctypes.c_uint8 * CX_MAX_ACTIONS),
         ("z_move", (ctypes.c_int8 * CX_MAX_ZDIRS) * CX_MAX_ACTIONS),
         ("z_front", (ctypes.c_int8 * CX_MAX_ZDIRS) * CX_MAX_ACTIONS),
+        ("terminate_emptied", ctypes.c_uint8),
+        ("emptied_value", ctypes.c_float),
     ]
 
 
@@ -106,7 +109,7 @@ class GameInfo(ctypes.Structure):
     _fields_ = [(n, ctypes.c_int32) for n in (
         "rows", "cols", "cells", "n_chars", "n_actions", "n_entities", "path", "can_terminate", "tracks",
         "has_dynamic_backdrop", "state_bytes_per_env", "board_bytes_per_env", "dynamic_render",
-        "tracks_performance")]
+        "tracks_performance", "n_pickups")]
 
 
 _P = ctypes.c_void_p
@@ -147,6 +150,7 @@ PROTOTYPES = {
     "cx_get_render_state": (ctypes.c_int, [_P, _P, _I64, _P, _P, _P, _P]),
     "cx_get_episode_state": (ctypes.c_int, [_P, _P, _I64, _P, _P, _P]),
     "cx_get_episode_performance": (ctypes.c_int, [_P, _P, _I64, _P, _P]),
+    "cx_get_pickups": (ctypes.c_int, [_P, _P, _I64, _P, _P]),
     "cx_stats_fold": (ctypes.c_int, [_P, _P, _P]),
     "cx_stats_read": (ctypes.c_int, [_P, _P, ctypes.POINTER(ctypes.c_double), _P]),
     "cx_step_perf": (ctypes.c_int, [_P, _I32, _I32, _P, _P, _I64, _P, _P]),

@@ -18,9 +18,12 @@ Probe set
 
   * for sprites that change `_visible`: every action from the other visibility state;
   * for a Backdrop whose update() changes its curtain: every action from a few pre-rolled curtains.
+  * for a pickup drape (collectible items): every probe above that took an item again with that item already
+    taken, and with that item as the drape's last one.
 
 Fitted per entity (see include/campx_b200.h `cx_entity_desc`)
-  kind, per-action toroidal move, blocker characters (one-cell drapes), per-action step reward,
+  kind (a drape that only ever loses the cell its watched entity stands on is a pickup), per-action toroidal move,
+  blocker characters (one-cell drapes), per-action step reward,
   "entry" reward as a function of (action, character the last render showed at a watched entity's
   current cell), terminate directives per action or per (action, character under the watched entity)
   ("reach the goal"), default-discount directives per action, per-action visibility
@@ -134,7 +137,9 @@ def _teleport(shadow, base_masks, ch, where):
             ent._visible = bool(where[2])
         return
     cur = ent.curtain
-    if where[0] == "cell":
+    if where[0] == "mask":                  # ("mask", uint8 [rows, cols]): a pickup drape with some items taken
+        cur.copy_(torch.from_numpy(np.asarray(where[1], dtype=np.uint8)).to(cur.dtype))
+    elif where[0] == "cell":
         cur.zero_()
         if where[1] is not None:
             cur[where[1] // cols, where[1] % cols] = 1
@@ -289,6 +294,8 @@ def compile_game(shadow, n_actions=5, action_format=None, max_episode_steps=0, a
         changed = [not np.array_equal(pr.post[ch][1], m0) for pr in s0_probes]
         if not any(changed):
             kind[ch] = N.CX_KIND_STATIC
+        elif all(_cleared_only(m0, pr.post[ch][1]) for pr in s0_probes):
+            kind[ch] = N.CX_KIND_PICKUP          # only ever loses cells: collectible items (fitted below)
         elif int(m0.sum()) == 1:
             kind[ch] = N.CX_KIND_CELL
         else:
@@ -398,6 +405,18 @@ def compile_game(shadow, n_actions=5, action_format=None, max_episode_steps=0, a
                                    "%s but update() gave %s" % (ch, p, a, mv[a], "".join(sorted(blk)), model, q))
         blockers[ch] = "".join(sorted(blk))
 
+    # ---- pickup drapes: items the agent collects ----------------------------------------------------------
+    # A drape that looked static from the initial state may still lose an item once the agent stands elsewhere.
+    for ch in z_chars:
+        if kind[ch] == N.CX_KIND_STATIC and any(
+                not np.array_equal(pr.post[ch][1], pr.pre[ch][1]) for pr in probes) and all(
+                _cleared_only(pr.pre[ch][1], pr.post[ch][1]) for pr in probes):
+            kind[ch] = N.CX_KIND_PICKUP
+    pickups = {}
+    if any(k == N.CX_KIND_PICKUP for k in kind.values()):
+        pickups = _fit_pickups(z_chars, kind, base_masks, base_snap, probes, probe, rank, A, rows, cols,
+                               len(base.update_groups), performance_regions, occlusion_in_layers)
+
     # ---- backdrop: static apart from the sprite stamps of quirk Q1, or rolled by Backdrop.update() ------------
     def first_drape_of(order_):
         return next((i for i, c in enumerate(order_) if kind[c] != N.CX_KIND_SPRITE), len(order_))
@@ -475,6 +494,12 @@ def compile_game(shadow, n_actions=5, action_format=None, max_episode_steps=0, a
 
     specs = []
     for z, ch in enumerate(z_chars):
+        if ch in pickups:
+            agent, reward, emptied = pickups[ch]
+            specs.append(EntitySpec(character=ch, kind=N.CX_KIND_PICKUP, mask=base_masks[ch], update_rank=rank[ch],
+                                    update_group=group_of[ch], watch=agent,
+                                    entry_reward={a: {ch: reward[a]} for a in range(A)}, terminate_emptied=emptied))
+            continue
         obs = []                                  # (probe, action, f32 reward or None)
         term, disc, zord = {}, {}, {}
         for pr in probes:
@@ -608,6 +633,10 @@ def compile_game(shadow, n_actions=5, action_format=None, max_episode_steps=0, a
             terminate=terminate or None, terminate_on=terminate_on or None, discount=discount or None,
             visible_op=visible_ops.get(ch), z_orders=z_orders or None))
 
+    if pickups:
+        _check_pickup_game(specs, pickups, base.backdrop.curtain.as_subclass(torch.Tensor).numpy(), backdrop_moves,
+                           rows, cols)
+
     # ---- whole-step consistency: the per-entity fits must add up to what play() returned --------------------
     spec = GameSpec(rows=rows, cols=cols, chars=chars, n_actions=A, entities=specs,
                     backdrop=base.backdrop.curtain.as_subclass(torch.Tensor).numpy().astype(np.uint8).copy(),
@@ -618,3 +647,132 @@ def compile_game(shadow, n_actions=5, action_format=None, max_episode_steps=0, a
                     occlusion_in_layers=bool(occlusion_in_layers), performance_regions=performance_regions)
     spec.n_probes = len(probes)
     return spec
+
+
+def _cleared_only(before, after):
+    """`after` is `before` with zero or more cells cleared (a binary curtain that only loses cells)."""
+    before, after = np.asarray(before).reshape(-1), np.asarray(after).reshape(-1)
+    return bool(np.isin(after, (0, 1)).all() and np.all(after <= (before != 0)))
+
+
+def _fit_pickups(z_chars, kind, base_masks, base_snap, probes, probe, rank, A, rows, cols, n_groups,
+                 performance_regions, occlusion_in_layers):
+    """Fit every CX_KIND_PICKUP candidate: when its update() runs and its curtain holds the watched agent's current
+    cell (the entry-reward query: the post-move cell if it updates after the agent, the pre-move cell otherwise), it
+    clears that one cell and calls add_reward(r[a]); if that emptied the curtain it may call terminate_episode(v);
+    nothing else.  Probes are added with the item already taken and with it as the last one.  Returns
+    {char: (agent char, [r[a]], v or None)}."""
+    chars = [c for c in z_chars if kind[c] == N.CX_KIND_PICKUP]
+    cells_ = [c for c in z_chars if kind[c] == N.CX_KIND_CELL]
+    for ch in chars:
+        if len(cells_) != 1 or any(kind[c] in (N.CX_KIND_SPRITE, N.CX_KIND_ROLL) for c in z_chars) or n_groups > 1 \
+                or rows * cols > 254:
+            raise CompileError("pickup drape %r needs a single-agent game (one moving one-cell drape over a static "
+                               "scene, one update group, at most 254 cells); this game would run on the generic "
+                               "kernels" % ch)
+        if performance_regions is not None:
+            raise CompileError("pickup drape %r together with performance_regions is not supported" % ch)
+        if not occlusion_in_layers:
+            raise CompileError("pickup drape %r needs occluded layers (occlusion_in_layers=True)" % ch)
+    agent = cells_[0]
+    z = {c: i for i, c in enumerate(z_chars)}
+    agent_cell = _cell_of(base_masks[agent])
+    owner, total = {}, 0
+    for ch in chars:
+        if z[ch] > z[agent]:
+            raise CompileError("pickup drape %r lies in front of the agent %r in z-order; it must be below it"
+                               % (ch, agent))
+        for c in np.flatnonzero(base_masks[ch].reshape(-1)):
+            if c in owner:
+                raise CompileError("pickup drapes %r and %r share cell %d" % (owner[c], ch, c))
+            if c == agent_cell:
+                raise CompileError("pickup drape %r has an item under the agent's initial cell" % ch)
+            owner[c] = ch
+            total += 1
+        if total > N.CX_MAX_PICKUPS:
+            raise CompileError("more than %d item cells in all (pickup drape %r)" % (N.CX_MAX_PICKUPS, ch))
+
+    def watched(pr, ch):
+        return _cell_of(pr.after[ch][agent][1])
+
+    out = {}
+    for ch in chars:
+        m0 = base_masks[ch].reshape(-1)
+        for pr in [pr for pr in probes if ch not in pr.teleports]:
+            c = watched(pr, ch)
+            if c is None or not m0[c]:
+                continue
+            taken, last = m0.copy(), np.zeros_like(m0)
+            taken[c], last[c] = 0, 1
+            for m in (taken, last):
+                probe(pr.action, dict(pr.teleports, **{ch: ("mask", m.reshape(rows, cols))}))
+        rewards, emptied = {}, set()
+        for pr in probes:
+            pre, post = pr.pre[ch][1].reshape(-1), pr.post[ch][1].reshape(-1)
+            c = watched(pr, ch)
+            hit = c is not None and pre[c] != 0
+            model = pre.copy()
+            if hit:
+                model[c] = 0
+            if not np.array_equal(post, model):
+                raise CompileError("drape %r changes its curtain in a way that is neither static nor a pickup "
+                                   "(clearing the cell %r stands on)" % (ch, agent))
+            events = pr.events.get(ch, ())
+            if not hit:
+                if events:
+                    raise CompileError("pickup drape %r calls %s in a step that takes no item"
+                                       % (ch, sorted({k for k, _ in events})))
+                continue
+            paid = [p for k, p in events if k == "reward"]
+            ends = [p for k, p in events if k == "terminate"]
+            if len(paid) != 1 or len(paid) + len(ends) != len(events):
+                raise CompileError("pickup drape %r must call add_reward exactly once when it takes an item, and "
+                                   "nothing but terminate_episode besides" % ch)
+            rewards.setdefault(pr.action, set()).add(float(_f32(paid[0])))
+            if model.any():
+                if ends:
+                    raise CompileError("pickup drape %r calls terminate_episode while items remain" % ch)
+            else:
+                emptied.add(float(ends[-1]) if ends else None)
+        values = set().union(*rewards.values())
+        if any(len(v) != 1 for v in rewards.values()) or (len(rewards) < A and len(values) != 1):
+            raise CompileError("the reward of pickup drape %r depends on something other than the action" % ch)
+        if len(emptied) != 1:
+            raise CompileError("pickup drape %r calls terminate_episode only sometimes when it takes its last item" % ch)
+        reward = [next(iter(rewards.get(a, values))) for a in range(A)]
+        out[ch] = (agent, reward, emptied.pop())
+    return out
+
+
+def _check_pickup_game(specs, pickups, backdrop, backdrop_moves, rows, cols):
+    """Refuse pickup games the single-agent kernels cannot run exactly: a changing render state, or another entity
+    that depends on whether an item is present (an item, or what lies under it, among its blockers, entry-reward or
+    terminate characters)."""
+    for e in specs:
+        if e.z_orders or (backdrop_moves and any(m != (0, 0) for m in backdrop_moves)):
+            raise CompileError("pickup drape %r needs a static render order and backdrop (%r changes it)"
+                               % (next(iter(pickups)), e.character))
+    present, absent = backdrop.reshape(-1).astype(np.int64), backdrop.reshape(-1).astype(np.int64)
+    for e in specs:
+        if e.kind in (N.CX_KIND_STATIC, N.CX_KIND_PICKUP):
+            m = np.asarray(e.mask).reshape(-1) != 0
+            present = np.where(m, ord(e.character), present)
+            if e.kind == N.CX_KIND_STATIC:
+                absent = np.where(m, ord(e.character), absent)
+    items = {}
+    for e in specs:
+        if e.kind == N.CX_KIND_PICKUP:
+            for c in np.flatnonzero(np.asarray(e.mask).reshape(-1)):
+                if present[c] != absent[c]:
+                    items.setdefault(e.character, set()).update((chr(present[c]), chr(absent[c])))
+    for e in specs:
+        if e.kind == N.CX_KIND_PICKUP:
+            continue
+        seen = set(e.blockers)
+        for table in list((e.entry_reward or {}).values()) + list((e.terminate_on or {}).values()):
+            seen.update(table)
+        for ch, shown in items.items():
+            if seen & shown:
+                raise CompileError("entity %r depends on whether an item of pickup drape %r is present (%r among its "
+                                   "blockers, entry-reward or terminate characters)"
+                                   % (e.character, ch, "".join(sorted(seen & shown))))

@@ -283,7 +283,7 @@ int launch_lane(const LaneParams& P, unsigned grid, unsigned block, size_t smem,
 bool cx_agent_lane_applies(const cx_game* g, int64_t n, const void* d_actions, const void* d_actions_out,
                            const void* d_reward, const void* d_discount, const void* d_flags, const void* d_board) {
   auto al16 = [](const void* p) { return p == nullptr || (reinterpret_cast<uintptr_t>(p) & 15) == 0; };
-  return g->path == CX_PATH_AGENT && n > 0 && n % 16 == 0 && lane_smem_bytes(g, 1) <= 64 * 1024 && al16(d_actions) &&
+  return g->path == CX_PATH_AGENT && !g->info.n_pickups && n > 0 && n % 16 == 0 && lane_smem_bytes(g, 1) <= 64 * 1024 && al16(d_actions) &&
          al16(d_actions_out) && al16(d_reward) && al16(d_discount) && al16(d_flags) && al16(d_board);
 }
 

@@ -21,6 +21,10 @@
 // are too large for k_agent_rollout's 256-env warp tiles (97..254 cells): at >= 100 bytes per env-step a
 // lane-per-env warp saturates HBM as well.  It also takes ragged batches (N not a multiple of 32) and
 // unaligned buffers (coalesced byte stores instead of the bulk stores) and in-kernel Philox actions.
+//
+// Games with collectible items (CX_KIND_PICKUP) run only here, in the PICK build: each lane keeps its env's u64 of
+// remaining items (CxPickHeader) and every ring slot remembers which items it shows; an item whose bit differs is
+// poked between its present and absent bytes (board and layered tile) when the slot comes up.
 #include "cx_agent_common.cuh"
 #include "cx_philox.cuh"
 
@@ -46,6 +50,8 @@ struct ObsParams {
   uint64_t seed, env_offset, t0;
   uint8_t* actions_out;    // synth: [T, n] or null
   float* perf;             // [n] (PERF)
+  uint64_t* pick;          // [n] items each env still holds (PICK)
+  CxPickHeader pk;         // (PICK)
 };
 
 constexpr int OBS_WARPS = 4;
@@ -57,8 +63,8 @@ constexpr int OBS_TILE = 32;  // envs per warp: lane = env
 // small batches (65,536 envs = 14 warps per SM: there is nothing else to run meanwhile).  With RING tiles used round
 // robin the warp waits for the store issued RING steps ago (`cp.async.bulk.wait_group.read RING-1`), i.e. almost
 // never, and a step's chain is table lookup -> 2 byte pokes -> fence -> issue.  PERF (TRACK builds of games that
-// track performance): the running performance beside the return.
-template <bool TRACK, bool PERF, int RING>
+// track performance): the running performance beside the return.  PICK: games with pickups (see the top of the file).
+template <bool TRACK, bool PERF, int RING, bool PICK>
 __global__ void __launch_bounds__(OBS_THREADS) k_agent_rollout_obs(const __grid_constant__ ObsParams P) {
   extern __shared__ __align__(16) uint8_t smem[];
   const CxAgentHeader& H = P.h;
@@ -70,6 +76,11 @@ __global__ void __launch_bounds__(OBS_THREADS) k_agent_rollout_obs(const __grid_
     const uint4* src = reinterpret_cast<const uint4*>(P.blob);
     uint4* dst = reinterpret_cast<uint4*>(smem);
     for (int i = tid; i < H.blob_bytes_ext / 16; i += OBS_THREADS) dst[i] = src[i];
+    if constexpr (PICK) {  // the item tables go right behind the extension
+      const uint4* psrc = reinterpret_cast<const uint4*>(P.blob + P.pk.off);
+      uint4* pdst = reinterpret_cast<uint4*>(smem + H.blob_bytes_ext);
+      for (int i = tid; i < P.pk.bytes / 16; i += OBS_THREADS) pdst[i] = psrc[i];
+    }
   }
   __syncthreads();  // the only block barrier
 
@@ -95,7 +106,8 @@ __global__ void __launch_bounds__(OBS_THREADS) k_agent_rollout_obs(const __grid_
   // per warp: RING x { [board tile 32*cells][layered tile 32*chars*cells (if wanted)] }, all multiples of 16 bytes
   const int per_env = cells + (layers ? lay_bytes : 0);
   const int slot_bytes = OBS_TILE * per_env;
-  uint8_t* wbase = smem + H.blob_bytes_ext + (size_t)warp * RING * slot_bytes;
+  const int tiles_at = H.blob_bytes_ext + (PICK ? P.pk.bytes : 0);
+  uint8_t* wbase = smem + tiles_at + (size_t)warp * RING * slot_bytes;
   for (int r = 0; r < RING; ++r) {                              // every lane stages its own env's static scene
     uint8_t* myb = wbase + r * slot_bytes + lane * cells;
     uint8_t* myl = wbase + r * slot_bytes + OBS_TILE * cells + lane * lay_bytes;
@@ -135,6 +147,49 @@ __global__ void __launch_bounds__(OBS_THREADS) k_agent_rollout_obs(const __grid_
     (wbase + r * slot_bytes + OBS_TILE * cells + lane * lay_bytes)[agent_k * cells + c] = v;
   };
 
+  // PICK: the static scene (basech / basek / baselay) shows every item; slot r shows the items in shown_items[r].
+  const uint8_t* __restrict__ s_item_at = smem + H.blob_bytes_ext + P.pk.item_at;
+  const CxPickItem* __restrict__ s_items = reinterpret_cast<const CxPickItem*>(smem + H.blob_bytes_ext + P.pk.items);
+  const CxPickDrape* __restrict__ s_drapes =
+      reinterpret_cast<const CxPickDrape*>(smem + H.blob_bytes_ext + P.pk.drapes);
+  uint64_t items = 0, shown_items[RING];
+  if constexpr (PICK) items = mine ? P.pick[env] : P.pk.all;
+  auto poke_item = [&](int r, uint32_t i, bool present) {  // item i of ring slot r (the agent is not drawn on it)
+    const CxPickItem it = s_items[i];
+    const uint32_t c = it.cell, kp = s_basek[c];
+    (wbase + r * slot_bytes + lane * cells)[c] = present ? s_basech[c] : it.under_ch;
+    if (layers) {
+      uint8_t* myl = wbase + r * slot_bytes + OBS_TILE * cells + lane * lay_bytes;
+      const uint32_t k_off = present ? it.under_k : kp, k_on = present ? kp : it.under_k;
+      if (k_off != 0xFF) myl[k_off * cells + c] = 0;
+      if (k_on != 0xFF) myl[k_on * cells + c] = 1;
+    }
+  };
+  auto sync_items = [&](int r, uint64_t want) {  // bring slot r to the items `want`
+    for (uint64_t m = shown_items[r] ^ want; m; m &= m - 1) {
+      const uint32_t i = __ffsll((long long)m) - 1;
+      poke_item(r, i, (want >> i) & 1);
+    }
+    shown_items[r] = want;
+  };
+  auto draw_agent = [&](int r, uint32_t c) {  // draw over the items slot r shows (a taken one left its under_k set)
+    draw(r, c);
+    if constexpr (PICK) {
+      const uint32_t i = s_item_at[c];
+      if (layers && i != CX_NO_ITEM && !((shown_items[r] >> i) & 1)) {
+        const uint32_t k = s_items[i].under_k;
+        if (k != 0xFF) (wbase + r * slot_bytes + OBS_TILE * cells + lane * lay_bytes)[k * cells + c] = 0;
+      }
+    }
+  };
+  auto erase_agent = [&](int r, uint32_t c) {  // erase, with the items slot r shows
+    erase(r, c);
+    if constexpr (PICK) {
+      const uint32_t i = s_item_at[c];
+      if (i != CX_NO_ITEM && !((shown_items[r] >> i) & 1)) poke_item(r, i, false);
+    }
+  };
+
   uint32_t cell = mine ? min((uint32_t)P.cell[env], none) : none;
   uint32_t shown = s_shown[cell];   // where the agent is drawn in the most recent frame
   uint32_t drawn[RING];             // ... and in each ring slot (a slot is RING frames behind when it comes up again)
@@ -143,7 +198,11 @@ __global__ void __launch_bounds__(OBS_THREADS) k_agent_rollout_obs(const __grid_
   for (int r = 0; r < RING; ++r) {
     drawn[r] = shown;
     lcell[r] = none;
-    if (shown != none) draw(r, shown);
+    if constexpr (PICK) {  // the items this env has already taken leave every slot
+      shown_items[r] = P.pk.all;
+      sync_items(r, items);
+    }
+    if (shown != none) draw_agent(r, shown);
     if (layers && unocc && cell != none) {
       agent_plane(r, cell, 1);
       lcell[r] = cell;
@@ -157,7 +216,7 @@ __global__ void __launch_bounds__(OBS_THREADS) k_agent_rollout_obs(const __grid_
     if (PERF) pf = P.perf[env];
   }
   LaneStatsT<PERF>& stats =
-      reinterpret_cast<LaneStatsT<PERF>*>(smem + H.blob_bytes_ext + (size_t)OBS_WARPS * RING * slot_bytes)[tid];
+      reinterpret_cast<LaneStatsT<PERF>*>(smem + tiles_at + (size_t)OBS_WARPS * RING * slot_bytes)[tid];
   if (TRACK) stats.clear();
 
   // whole tiles over TMA when the rows are 16-byte aligned and the warp owns 32 envs; else byte stores
@@ -204,8 +263,27 @@ __global__ void __launch_bounds__(OBS_THREADS) k_agent_rollout_obs(const __grid_
       const uint32_t show = mine ? (e >> 8) & 0xFF : none;
       const uint32_t stood = mine ? p : none;   // the agent's cell in this step's frame (before any auto reset)
       uint32_t f = cx_tt_flags<PERF>(e);
-      if (TRACK && mine && cx_episode_step<PERF>(f, rw, ts, rt, stats, max_steps, auto_reset, &pf, cx_tt_perf(e)))
+      uint64_t frame_items = 0;   // PICK: the items of this step's frame (before an auto reset)
+      if constexpr (PICK) {
+        // one look-up at the watched cell: the agent's cell after the move when the pickups update after it, before
+        // the move otherwise (the entry-reward query); a bad action or a frozen env takes nothing
+        const uint32_t i = s_item_at[P.pk.after ? p : cell];
+        if (mine && i != CX_NO_ITEM && ((items >> i) & 1) && !(f & (CX_FLAG_BAD_ACTION | CX_FLAG_ALREADY_OVER))) {
+          items &= ~(1ull << i);
+          const CxPickDrape& D = s_drapes[s_items[i].drape];
+          rw += D.reward[a];      // the table's sum of the entities before it, or 0 (REWARD_NONE)
+          f &= ~(uint32_t)CX_FLAG_REWARD_NONE;
+          if (D.terminates && !(items & D.items)) {
+            f |= CX_FLAG_TERMINATED;
+            dc = D.emptied_value;
+          }
+        }
+        frame_items = items;
+      }
+      if (TRACK && mine && cx_episode_step<PERF>(f, rw, ts, rt, stats, max_steps, auto_reset, &pf, cx_tt_perf(e))) {
         p = H.init_cell;
+        if constexpr (PICK) items = P.pk.all;   // an auto reset puts every item back
+      }
       if (mine) {
         cell = p;
         __stcs(P.reward + row + lane, rw);
@@ -219,7 +297,18 @@ __global__ void __launch_bounds__(OBS_THREADS) k_agent_rollout_obs(const __grid_
         if (lane == 0) bulk_wait_read_pending<RING - 1>();  // the store that last shipped slot r has read it
         __syncwarp();
       }
-      if (drawn[r] != show) {
+      if constexpr (PICK) {
+        if (shown_items[r] != frame_items) {   // the agent comes off first: pokes assume it is not drawn there
+          if (drawn[r] != none) erase_agent(r, drawn[r]);
+          drawn[r] = none;
+          sync_items(r, frame_items);
+        }
+        if (drawn[r] != show) {
+          if (drawn[r] != none) erase_agent(r, drawn[r]);
+          if (show != none) draw_agent(r, show);
+          drawn[r] = show;
+        }
+      } else if (drawn[r] != show) {
         if (drawn[r] != none) erase(r, drawn[r]);
         if (show != none) draw(r, show);
         drawn[r] = show;
@@ -262,6 +351,7 @@ __global__ void __launch_bounds__(OBS_THREADS) k_agent_rollout_obs(const __grid_
       P.ret[env] = rt;
       if (PERF) P.perf[env] = pf;
     }
+    if constexpr (PICK) P.pick[env] = items;
   }
   if (TRACK)  // all 32 lanes reduce (lanes without an env contribute empty statistics)
     cx_flush_stats<PERF>(stats, P.stats, (uint32_t)(blockIdx.x * OBS_WARPS + warp), (uint32_t)nenv, P.T);
@@ -269,15 +359,15 @@ __global__ void __launch_bounds__(OBS_THREADS) k_agent_rollout_obs(const __grid_
 
 size_t obs_smem_bytes(const cx_game* g, bool layers, int ring = 1) {
   const size_t per_env = (size_t)g->ah.cells * (1 + (layers ? g->ah.n_chars : 0));
-  return (size_t)g->ah.blob_bytes_ext + (size_t)OBS_WARPS * OBS_TILE * per_env * ring +
+  return (size_t)g->ah.blob_bytes_ext + (size_t)g->ph.bytes + (size_t)OBS_WARPS * OBS_TILE * per_env * ring +
          (g->ah.track ? OBS_THREADS * (g->info.tracks_performance ? sizeof(LaneStatsPerf) : sizeof(LaneStats)) : 0);
 }
 
-template <bool TRACK, bool PERF, int RING>
+template <bool TRACK, bool PERF, int RING, bool PICK>
 int launch_obs(const ObsParams& P, unsigned grid, size_t smem, cudaStream_t s) {
   static CxPerDevice configured;  // the dynamic shared memory cap is a per-device function attribute
   if (configured.need()) {
-    CX_CUDA_OK(cudaFuncSetAttribute(k_agent_rollout_obs<TRACK, PERF, RING>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    CX_CUDA_OK(cudaFuncSetAttribute(k_agent_rollout_obs<TRACK, PERF, RING, PICK>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                     227 * 1024));
     configured.mark();
   }
@@ -291,13 +381,13 @@ int launch_obs(const ObsParams& P, unsigned grid, size_t smem, cudaStream_t s) {
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  CX_CUDA_OK(cudaLaunchKernelEx(&cfg, k_agent_rollout_obs<TRACK, PERF, RING>, P));
+  CX_CUDA_OK(cudaLaunchKernelEx(&cfg, k_agent_rollout_obs<TRACK, PERF, RING, PICK>, P));
   return CX_OK;
 }
 
-template <bool TRACK, bool PERF>
+template <bool TRACK, bool PERF, bool PICK = false>
 int launch_obs_ring(int ring, const ObsParams& P, unsigned grid, size_t smem, cudaStream_t s) {
-  return ring >= 2 ? launch_obs<TRACK, PERF, 2>(P, grid, smem, s) : launch_obs<TRACK, PERF, 1>(P, grid, smem, s);
+  return ring >= 2 ? launch_obs<TRACK, PERF, 2, PICK>(P, grid, smem, s) : launch_obs<TRACK, PERF, 1, PICK>(P, grid, smem, s);
 }
 
 }  // namespace
@@ -334,6 +424,8 @@ int cx_launch_agent_rollout_obs(const cx_game* g, void* d_state, int64_t n, int3
   P.t0 = synth.t0;
   P.actions_out = synth.actions_out;
   P.perf = reinterpret_cast<float*>(base + L.off_perf);
+  P.pick = reinterpret_cast<uint64_t*>(base + L.off_pick);
+  P.pk = g->ph;
   // bulk (TMA) stores: every [T, n, ...] row and every warp tile must start 16-byte aligned
   auto al16 = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; };
   const int64_t lay_bytes = (int64_t)g->ah.n_chars * g->ah.cells;
@@ -357,6 +449,9 @@ int cx_launch_agent_rollout_obs(const cx_game* g, void* d_state, int64_t n, int3
     return CX_ERR_INVALID_ARG;
   }
   if (g->info.tracks_performance) return launch_obs_ring<true, true>(ring, P, (unsigned)grid, smem, s);
+  if (g->info.n_pickups)   // (never together with performance: cx_game_create refuses that)
+    return g->ah.track ? launch_obs_ring<true, false, true>(ring, P, (unsigned)grid, smem, s)
+                       : launch_obs_ring<false, false, true>(ring, P, (unsigned)grid, smem, s);
   return g->ah.track ? launch_obs_ring<true, false>(ring, P, (unsigned)grid, smem, s)
                      : launch_obs_ring<false, false>(ring, P, (unsigned)grid, smem, s);
 }

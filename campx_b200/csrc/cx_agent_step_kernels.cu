@@ -266,7 +266,7 @@ int launch_step_lay(int lay, const StepParams& P, unsigned grid, unsigned block,
 // because a CTA owns a multiple of 32 envs).  Callers fall back to the tile kernels otherwise.
 bool cx_agent_step_applies(const cx_game* g, const void* d_board, const void* d_layered) {
   auto al16 = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; };
-  return g->path == CX_PATH_AGENT && al16(d_board) && al16(d_layered);
+  return g->path == CX_PATH_AGENT && !g->info.n_pickups && al16(d_board) && al16(d_layered);
 }
 
 int cx_launch_agent_step(const cx_game* g, void* d_state, int64_t n, const uint8_t* d_actions, float* d_reward,

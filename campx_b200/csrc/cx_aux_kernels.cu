@@ -47,8 +47,8 @@ __global__ void k_stats_fold(double* stats) {
   }
 }
 
-__global__ void k_agent_reset(uint8_t* cell, uint16_t* tstep, float* ret, float* perf, int track, int init_cell,
-                              const uint8_t* mask, int64_t n) {
+__global__ void k_agent_reset(uint8_t* cell, uint16_t* tstep, float* ret, float* perf, uint64_t* pick,
+                              uint64_t all_items, int track, int init_cell, const uint8_t* mask, int64_t n) {
   const int64_t i = (int64_t)blockIdx.x * TB + threadIdx.x;
   if (i >= n || (mask && !mask[i])) return;
   cell[i] = (uint8_t)init_cell;
@@ -57,6 +57,7 @@ __global__ void k_agent_reset(uint8_t* cell, uint16_t* tstep, float* ret, float*
     ret[i] = 0.0f;
   }
   if (perf) perf[i] = 0.0f;
+  if (pick) pick[i] = all_items;   // every item back on the board
 }
 
 struct GenInit {
@@ -83,13 +84,20 @@ __global__ void k_dynbd_reset(uint8_t* dynbd, const uint8_t* backdrop, int cells
   dynbd[i] = backdrop[i - e * cells];
 }
 
+// pick (games with pickups, else null): the items each env holds; basech shows every item, a taken one shows its
+// under_ch (CxPickItem)
 __global__ void k_agent_render(const uint8_t* cell, const uint8_t* basech, const uint8_t* shown, int cells,
-                               int agent_char, uint8_t* board, int64_t n) {
+                               int agent_char, uint8_t* board, int64_t n, const uint64_t* pick,
+                               const uint8_t* item_at, const CxPickItem* items) {
   const int64_t i = (int64_t)blockIdx.x * TB + threadIdx.x;
   if (i >= n * cells) return;
   const int64_t e = i / cells;
   const int c = (int)(i - e * cells);
   uint8_t v = basech[c];
+  if (pick) {
+    const uint32_t k = item_at[c];
+    if (k != CX_NO_ITEM && !((pick[e] >> k) & 1)) v = items[k].under_ch;
+  }
   if (shown[cell[e]] == c) v = (uint8_t)agent_char;
   board[i] = v;
 }
@@ -629,8 +637,9 @@ int cx_launch_reset(const cx_game* g, void* d_state, int64_t n, const uint8_t* d
     k_stats_init<<<blocks_for((1 + CX_STAT_STRIPES) * CX_STATS_DOUBLES), TB, 0, s>>>(reinterpret_cast<double*>(base + L.off_stats));
   if (g->path == CX_PATH_AGENT) {
     float* perf = g->info.tracks_performance ? reinterpret_cast<float*>(base + L.off_perf) : nullptr;
-    k_agent_reset<<<blocks_for(n), TB, 0, s>>>(base + L.off_dyn, tstep, ret, perf, g->info.tracks, g->ah.init_cell,
-                                               d_mask, n);
+    uint64_t* pick = g->info.n_pickups ? reinterpret_cast<uint64_t*>(base + L.off_pick) : nullptr;
+    k_agent_reset<<<blocks_for(n), TB, 0, s>>>(base + L.off_dyn, tstep, ret, perf, pick, g->ph.all, g->info.tracks,
+                                               g->ah.init_cell, d_mask, n);
   } else {
     GenInit gi;
     memset(&gi, 0, sizeof(gi));
@@ -650,9 +659,11 @@ int cx_launch_render(const cx_game* g, const void* d_state, int64_t n, uint8_t* 
   if (g->path != CX_PATH_AGENT) return cx_launch_generic_render(g, d_state, n, d_board, s);
   const CxStateLayout L = cx_layout(g, n);
   const uint8_t* base = static_cast<const uint8_t*>(d_state);
-  k_agent_render<<<blocks_for(n * g->ah.cells), TB, 0, s>>>(base + L.off_dyn, g->d_blob + g->ah.off_basech,
-                                                            g->d_blob + g->ah.off_shown, g->ah.cells,
-                                                            g->ah.agent_char, d_board, n);
+  const uint8_t* pk = g->d_blob + g->ph.off;
+  k_agent_render<<<blocks_for(n * g->ah.cells), TB, 0, s>>>(
+      base + L.off_dyn, g->d_blob + g->ah.off_basech, g->d_blob + g->ah.off_shown, g->ah.cells, g->ah.agent_char, d_board,
+      n, g->info.n_pickups ? reinterpret_cast<const uint64_t*>(base + L.off_pick) : nullptr, pk + g->ph.item_at,
+      reinterpret_cast<const CxPickItem*>(pk + g->ph.items));
   CX_CUDA_OK(cudaGetLastError());
   return CX_OK;
 }
@@ -664,8 +675,8 @@ int cx_launch_get_entity(const cx_game* g, const void* d_state, int64_t n, int32
   const CxStateLayout L = cx_layout(g, n);
   const uint8_t* base = static_cast<const uint8_t*>(d_state);
   const int kind = g->desc.entities[z].kind;
-  if (kind == CX_KIND_STATIC) {
-    cx_set_error("cx_get_entity_state: entity %d is static", z);
+  if (kind == CX_KIND_STATIC || kind == CX_KIND_PICKUP) {
+    cx_set_error("cx_get_entity_state: entity %d is static or a pickup drape", z);
     return CX_ERR_INVALID_ARG;
   }
   if (g->path == CX_PATH_AGENT) {

@@ -58,6 +58,8 @@ CxStateLayout cx_layout(const cx_game* g, int64_t n) {
   if (g->path == CX_PATH_GENERIC && g->gh.has_dynbd) off = align_up(off + n * (int64_t)g->gh.cells, 256);
   L.off_perf = off;   // last, so that the layout of a game without performance is what it was before
   if (g->info.tracks_performance) off = align_up(off + n * 4, 256);
+  L.off_pick = off;   // behind everything else for the same reason
+  if (g->info.n_pickups) off = align_up(off + n * 8, 256);
   L.total = off < 256 ? 256 : off;
   return L;
 }
@@ -88,6 +90,7 @@ static void build_action_table(const cx_game_desc* d, const int* order, CxAction
     if (a < d->n_actions) {
       for (int i = 0; i < d->n_entities; ++i) {
         const cx_entity_desc& e = d->entities[order[i]];
+        if (e.kind == CX_KIND_PICKUP) continue;   // pays and terminates only when it takes an item (the kernel)
         if (e.reward_actions >> a & 1) any_reward = true;
         if (e.discount_actions >> a & 1) disc = e.discount_value[a];
         if (e.terminate_actions >> a & 1) {
@@ -181,7 +184,7 @@ static int validate(const cx_game_desc* d) {
         cx_set_error("cx_game_create: character %d used by two entities", e.character);  // engine.py:343-350
         return CX_ERR_INVALID_ARG;
       }
-    if (e.kind > CX_KIND_SPRITE) {
+    if (e.kind > CX_KIND_PICKUP) {
       cx_set_error("cx_game_create: entity %d has unknown kind %d", z, e.kind);
       return CX_ERR_INVALID_ARG;
     }
@@ -214,6 +217,10 @@ static int validate(const cx_game_desc* d) {
         cx_set_error("cx_game_create: blockers are only defined for CELL drapes (entity %d)", z);
         return CX_ERR_UNSUPPORTED;
       }
+    }
+    if (e.kind == CX_KIND_PICKUP && e.terminate_emptied && !(e.emptied_value >= 0.0f && e.emptied_value <= 1.0f)) {
+      cx_set_error("Pcontinue must be in range [0,1]");  // plot.py:176-177
+      return CX_ERR_INVALID_ARG;
     }
     if (e.kind == CX_KIND_CELL) {
       int first;
@@ -368,7 +375,7 @@ static AgentStep agent_step_host(const cx_game_desc* d, int agent_z, const int* 
   float summed = 0.0f;
   for (int i = 0; i < d->n_entities; ++i) {
     const cx_entity_desc& e = d->entities[order[i]];
-    if (!(e.reward_actions >> a & 1)) continue;
+    if (!(e.reward_actions >> a & 1) || e.kind == CX_KIND_PICKUP) continue;
     volatile float rr = e.step_reward[a];
     if (e.watch == agent_z) {
       const int k = (e.update_rank >= ag.update_rank) ? kn : ko;  // things['A'] is current sibling state
@@ -387,6 +394,7 @@ static AgentStep agent_step_host(const cx_game_desc* d, int agent_z, const int* 
   float disc = 1.0f;  // plot.py:100
   for (int i = 0; i < d->n_entities; ++i) {
     const cx_entity_desc& e = d->entities[order[i]];
+    if (e.kind == CX_KIND_PICKUP) continue;
     if (e.discount_actions >> a & 1) disc = e.discount_value[a];
     if (e.terminate_actions >> a & 1) {
       over = true;
@@ -408,7 +416,29 @@ static AgentStep agent_step_host(const cx_game_desc* d, int agent_z, const int* 
   return out;
 }
 
-static void build_agent_tables(const cx_game_desc* d, int agent_z, const int* order, CxAgentHeader* H, Blob* B) {
+// Static composition without the agent (painter's algorithm, engine.py:306-321) and where the agent is visible; pickup
+// drapes with all their items (items_present) or none.
+static void compose_static(const cx_game_desc* d, int agent_z, bool items_present, std::vector<uint8_t>* basech,
+                           std::vector<uint8_t>* vis) {
+  const int cells = d->rows * d->cols;
+  basech->assign(cells + 1, 0);
+  vis->assign(cells + 1, 0);
+  for (int c = 0; c < cells; ++c) {
+    (*basech)[c] = d->backdrop[c];
+    (*vis)[c] = 1;
+  }
+  for (int z = 0; z < d->n_entities; ++z) {
+    if (z == agent_z || (d->entities[z].kind == CX_KIND_PICKUP && !items_present)) continue;
+    const uint8_t* m = d->masks + (size_t)z * cells;
+    for (int c = 0; c < cells; ++c)
+      if (m[c]) {
+        (*basech)[c] = d->entities[z].character;
+        if (z > agent_z) (*vis)[c] = 0;  // painted after (in front of) the agent
+      }
+  }
+}
+
+static int build_agent_tables(const cx_game_desc* d, int agent_z, const int* order, CxAgentHeader* H, Blob* B) {
   const int R = d->rows, C = d->cols, cells = R * C, A = d->n_actions;
   const cx_entity_desc& ag = d->entities[agent_z];
   memset(H, 0, sizeof(*H));
@@ -424,20 +454,24 @@ static void build_agent_tables(const cx_game_desc* d, int agent_z, const int* or
   H->auto_reset = d->auto_reset;
   build_action_table(d, order, &H->act);
 
-  // static composition without the agent (painter's algorithm, engine.py:306-321) + agent visibility
-  std::vector<uint8_t> basech(cells + 1, 0), vis(cells + 1, 0);
-  for (int c = 0; c < cells; ++c) {
-    basech[c] = d->backdrop[c];
-    vis[c] = 1;
-  }
-  for (int z = 0; z < d->n_entities; ++z) {
-    if (z == agent_z) continue;
-    const uint8_t* m = d->masks + (size_t)z * cells;
-    for (int c = 0; c < cells; ++c)
-      if (m[c]) {
-        basech[c] = d->entities[z].character;
-        if (z > agent_z) vis[c] = 0;  // painted after (in front of) the agent
+  // The step tables are lowered with every item absent, the scene (basech and what derives from it) shows every item
+  // present.  Games without pickups: the two are the same.
+  std::vector<uint8_t> absent, vis, basech, unused;
+  compose_static(d, agent_z, false, &absent, &vis);
+  compose_static(d, agent_z, true, &basech, &unused);   // (pickups in front of the agent: build_pick_tables refuses)
+  for (int p = 0; p < cells; ++p) {
+    // nothing but the pickups' own reward and termination may depend on an item's presence: one Engine.play() from
+    // every cell under every action must not change when all items are put back
+    for (int a = 0; a < A; ++a) {
+      const AgentStep x = agent_step_host(d, agent_z, order, absent.data(), vis.data(), a, p);
+      const AgentStep y = agent_step_host(d, agent_z, order, basech.data(), vis.data(), a, p);
+      if (x.q != y.q || memcmp(&x.reward, &y.reward, 4) || x.over != y.over || memcmp(&x.discount, &y.discount, 4)) {
+        cx_set_error("cx_game_create: the step from cell %d under action %d depends on whether an item is present "
+                     "(an item or the character under it is a blocker, an entry-reward or a terminate character of "
+                     "another entity); only the pickup drape's own reward and termination may", p, a);
+        return CX_ERR_UNSUPPORTED;
       }
+    }
   }
   const int S = cells + 1;
   for (int z = 0; z < d->n_entities; ++z)
@@ -457,7 +491,7 @@ static void build_agent_tables(const cx_game_desc* d, int agent_z, const int* or
         float reward = 0.0f, disc = 1.0f;
         uint32_t flags = CX_FLAG_BAD_ACTION | CX_FLAG_REWARD_NONE;  // row A: env left untouched
         if (a < A) {
-          const AgentStep st = agent_step_host(d, agent_z, order, basech.data(), vis.data(), a, p);
+          const AgentStep st = agent_step_host(d, agent_z, order, absent.data(), vis.data(), a, p);
           q = st.q;
           reward = st.reward;
           disc = st.discount;
@@ -518,6 +552,110 @@ static void build_agent_tables(const cx_game_desc* d, int agent_z, const int* or
   for (int i = 0; i < L * cells + 24; ++i)
     B->bytes[H->off_baselay_wrap + i] = B->bytes[H->off_baselay + i % (L * cells)];
   B->pad();
+  return CX_OK;
+}
+
+// The CX_KIND_PICKUP region of a single-agent game (CxPickHeader), appended to the blob behind the agent tables.
+static int build_pick_tables(const cx_game_desc* d, int agent_z, CxPickHeader* P, Blob* B) {
+  const int cells = d->rows * d->cols;
+  memset(P, 0, sizeof(*P));
+  int n_drapes = 0, side = -1;
+  for (int z = 0; z < d->n_entities; ++z) n_drapes += d->entities[z].kind == CX_KIND_PICKUP;
+  if (!n_drapes) return CX_OK;
+  const cx_entity_desc& ag = d->entities[agent_z];
+  if (d->n_perf_regions) {
+    cx_set_error("cx_game_create: pickup drapes together with performance regions are not supported");
+    return CX_ERR_UNSUPPORTED;
+  }
+  if (d->unoccluded_layers) {
+    cx_set_error("cx_game_create: pickup drapes need occluded layers (occlusion_in_layers=True)");
+    return CX_ERR_UNSUPPORTED;
+  }
+  int agent_cell;
+  popcount_mask(d->masks + (size_t)agent_z * cells, cells, &agent_cell);
+  std::vector<uint8_t> absent, vis;
+  compose_static(d, agent_z, false, &absent, &vis);
+  std::vector<uint8_t> item_at(cells + 1, CX_NO_ITEM);
+  std::vector<CxPickItem> items;
+  std::vector<CxPickDrape> drapes;
+  for (int z = 0; z < d->n_entities; ++z) {
+    const cx_entity_desc& e = d->entities[z];
+    if (e.kind != CX_KIND_PICKUP) continue;
+    const int ch = e.character;
+    if (z > agent_z) {
+      cx_set_error("cx_game_create: pickup drape '%c' lies in front of the agent in z-order; pickup drapes must be below "
+                   "it", ch);
+      return CX_ERR_UNSUPPORTED;
+    }
+    const int after = e.update_rank > ag.update_rank ? 1 : 0;
+    if (side >= 0 && side != after) {
+      cx_set_error("cx_game_create: pickup drape '%c' updates on the other side of the agent than another pickup "
+                   "drape; all pickup drapes must update before it or all after it", ch);
+      return CX_ERR_UNSUPPORTED;
+    }
+    side = after;
+    for (int y = 0; y < d->n_entities; ++y) {
+      const cx_entity_desc& o = d->entities[y];
+      if (o.kind == CX_KIND_PICKUP || o.update_rank < e.update_rank) continue;
+      bool directs = o.reward_actions || o.terminate_actions || o.discount_actions;
+      for (int a = 0; a < d->n_actions; ++a) directs |= o.terminate_chars[a] != 0;
+      if (directs) {   // the kernel adds the item's reward last and lets its termination win
+        cx_set_error("cx_game_create: entity '%c' updates after pickup drape '%c' and calls add_reward, "
+                     "terminate_episode or change_default_discount; entities after a pickup drape may not", o.character,
+                     ch);
+        return CX_ERR_UNSUPPORTED;
+      }
+    }
+    if (e.watch != agent_z) {
+      cx_set_error("cx_game_create: pickup drape '%c' must watch the agent", ch);
+      return CX_ERR_UNSUPPORTED;
+    }
+    CxPickDrape pd;
+    memset(&pd, 0, sizeof(pd));
+    const int own = char_index(d, ch);
+    for (int a = 0; a < d->n_actions; ++a) pd.reward[a] = e.entry_reward[a][own];
+    pd.terminates = e.terminate_emptied ? 1 : 0;
+    pd.emptied_value = e.emptied_value;
+    const uint8_t* m = d->masks + (size_t)z * cells;
+    for (int c = 0; c < cells; ++c) {
+      if (!m[c]) continue;
+      if (item_at[c] != CX_NO_ITEM) {
+        cx_set_error("cx_game_create: pickup drape '%c' shares cell %d with another pickup drape", ch, c);
+        return CX_ERR_UNSUPPORTED;
+      }
+      if (c == agent_cell) {
+        cx_set_error("cx_game_create: pickup drape '%c' has an item under the agent's initial cell %d", ch, c);
+        return CX_ERR_UNSUPPORTED;
+      }
+      if ((int)items.size() >= CX_MAX_PICKUPS) {
+        cx_set_error("cx_game_create: more than %d item cells in all (pickup drape '%c')", CX_MAX_PICKUPS, ch);
+        return CX_ERR_UNSUPPORTED;
+      }
+      CxPickItem it;
+      it.cell = (uint8_t)c;
+      it.under_ch = absent[c];
+      const int k = char_index(d, absent[c]);
+      it.under_k = (uint8_t)(k < 0 ? 0xFF : k);
+      it.drape = (uint8_t)drapes.size();
+      pd.items |= 1ull << items.size();
+      item_at[c] = (uint8_t)items.size();
+      items.push_back(it);
+    }
+    drapes.push_back(pd);
+  }
+  P->n_items = (int32_t)items.size();
+  P->after = side > 0 ? 1 : 0;
+  P->all = P->n_items == 64 ? ~0ull : (1ull << P->n_items) - 1;
+  P->item_at = 0;
+  P->items = (cells + 1 + 15) / 16 * 16;
+  P->drapes = (P->items + (int32_t)(items.size() * sizeof(CxPickItem)) + 15) / 16 * 16;
+  P->bytes = (P->drapes + (int32_t)(drapes.size() * sizeof(CxPickDrape)) + 15) / 16 * 16;
+  P->off = B->reserve(P->bytes);
+  memcpy(&B->bytes[P->off + P->item_at], item_at.data(), cells + 1);
+  memcpy(&B->bytes[P->off + P->items], items.data(), items.size() * sizeof(CxPickItem));
+  memcpy(&B->bytes[P->off + P->drapes], drapes.data(), drapes.size() * sizeof(CxPickDrape));
+  B->pad();
+  return CX_OK;
 }
 
 static int build_generic_tables(const cx_game_desc* d, const int* order, CxGenHeader* H, Blob* B) {
@@ -884,10 +1022,23 @@ extern "C" int cx_game_create(const cx_game_desc* desc, cx_game** out) {
 
   Blob blob;
   int agent_z = -1;
+  bool pickups = false;
+  for (int z = 0; z < desc->n_entities; ++z) pickups |= desc->entities[z].kind == CX_KIND_PICKUP;
   if (agent_path_applies(desc, &agent_z)) {
     g->path = CX_PATH_AGENT;
-    build_agent_tables(desc, agent_z, order, &g->ah, &blob);
+    rc = build_agent_tables(desc, agent_z, order, &g->ah, &blob);
+    if (rc == CX_OK) rc = build_pick_tables(desc, agent_z, &g->ph, &blob);
+    if (rc != CX_OK) {
+      delete g;
+      return rc;
+    }
   } else {
+    if (pickups) {
+      cx_set_error("cx_game_create: pickup drapes need a single-agent game (one moving one-cell drape over a static "
+                   "scene); this game runs on the generic kernels");
+      delete g;
+      return CX_ERR_UNSUPPORTED;
+    }
     if (desc->n_perf_regions) {
       cx_set_error("cx_game_create: performance regions need a single-agent game (one moving one-cell drape over a "
                    "static scene); this game runs on the generic kernels");
@@ -907,6 +1058,8 @@ extern "C" int cx_game_create(const cx_game_desc* desc, cx_game** out) {
     can_term |= act.over[a] != 0;
     for (int z = 0; z < desc->n_entities; ++z) can_term |= desc->entities[z].terminate_chars[a] != 0;
   }
+  for (int z = 0; z < desc->n_entities; ++z)
+    can_term |= desc->entities[z].kind == CX_KIND_PICKUP && desc->entities[z].terminate_emptied;
   const int tracks = (can_term || desc->max_episode_steps > 0 || desc->track_returns) ? 1 : 0;
   if (g->path == CX_PATH_AGENT)
     g->ah.track = tracks;
@@ -927,8 +1080,10 @@ extern "C" int cx_game_create(const cx_game_desc* desc, cx_game** out) {
   I.has_dynamic_backdrop = g->path == CX_PATH_GENERIC ? g->gh.has_dynbd : 0;
   I.board_bytes_per_env = cells;
   I.dynamic_render = g->path == CX_PATH_GENERIC ? g->gh.dyn_render : 0;
+  I.n_pickups = g->path == CX_PATH_AGENT ? g->ph.n_items : 0;
   I.state_bytes_per_env = (g->path == CX_PATH_AGENT ? 1 : 2 * g->gh.n_dyn) + (tracks ? 6 : 0) +
-                          (I.has_dynamic_backdrop ? cells : 0) + (I.tracks_performance ? 4 : 0);
+                          (I.has_dynamic_backdrop ? cells : 0) + (I.tracks_performance ? 4 : 0) +
+                          (I.n_pickups ? 8 : 0);
 
   CX_CUDA_OK(cudaGetDevice(&g->device));
   CX_CUDA_OK(cudaDeviceGetAttribute(&g->sm_count, cudaDevAttrMultiProcessorCount, g->device));
@@ -1072,7 +1227,8 @@ static int rollout_common(const cx_game* g, void* d_state, int64_t n, int32_t T,
         cx_agent_lane_applies(g, n, d_actions, synth.actions_out, d_reward, d_discount, d_flags, d_board))
       return cx_launch_agent_rollout_lane(g, d_state, n, T, d_actions, synth, d_reward, d_discount, d_flags, d_board,
                                           (cudaStream_t)stream);
-    if (g->ah.cells > CX_AGENT_TILE_MAX_CELLS || n < small_n)  // large boards, small batches: lane-per-env kernel, board only
+    // games with pickups: always here (the PICK build), whatever the route
+    if (g->ah.cells > CX_AGENT_TILE_MAX_CELLS || n < small_n || g->info.n_pickups)  // large boards, small batches: lane-per-env kernel, board only
       return cx_launch_agent_rollout_obs(g, d_state, n, T, d_actions, synth, d_reward, d_discount, d_flags, d_board,
                                          nullptr, (cudaStream_t)stream);
     return cx_launch_agent_rollout(g, d_state, n, T, d_actions, synth, d_reward, d_discount, d_flags, d_board, route,
@@ -1154,6 +1310,11 @@ extern "C" int cx_rollout_policy(const cx_game* g, void* d_state, int64_t n, int
                                  uint8_t* d_actions, float* d_reward, uint8_t* d_flags, float* d_logp, void* stream) {
   int rc = check_common(g, d_state, n, "cx_rollout_policy");
   if (rc) return rc;
+  if (g->info.n_pickups) {
+    cx_set_error("cx_rollout_policy: games with pickup drapes are not supported; use cx_policy_sample_board and "
+                 "cx_step");
+    return CX_ERR_UNSUPPORTED;
+  }
   if (T < 1 || !d_w1t || !d_b1 || !d_w2 || !d_b2 || !d_states || !d_actions || !d_reward || !d_flags || n_hidden < 1 ||
       n_hidden > 32) {
     cx_set_error("cx_rollout_policy: bad argument (n_steps >= 1, n_hidden in 1..32, no NULL buffers)");
@@ -1236,6 +1397,10 @@ extern "C" int cx_get_entity_state(const cx_game* g, const void* d_state, int64_
     cx_set_error("cx_get_entity_state: bad z_index %d or NULL output", z);
     return CX_ERR_INVALID_ARG;
   }
+  if (g->desc.entities[z].kind == CX_KIND_PICKUP) {
+    cx_set_error("cx_get_entity_state: entity %d is a pickup drape (its items: cx_get_pickups)", z);
+    return CX_ERR_INVALID_ARG;
+  }
   return cx_launch_get_entity(g, d_state, n, z, d_cells, (cudaStream_t)stream);
 }
 
@@ -1247,8 +1412,8 @@ extern "C" int cx_set_entity_state(const cx_game* g, void* d_state, int64_t n, i
     cx_set_error("cx_set_entity_state: bad z_index %d or NULL input", z);
     return CX_ERR_INVALID_ARG;
   }
-  if (g->desc.entities[z].kind == CX_KIND_STATIC) {
-    cx_set_error("cx_set_entity_state: entity %d is static", z);
+  if (g->desc.entities[z].kind == CX_KIND_STATIC || g->desc.entities[z].kind == CX_KIND_PICKUP) {
+    cx_set_error("cx_set_entity_state: entity %d is static or a pickup drape", z);
     return CX_ERR_INVALID_ARG;
   }
   return cx_launch_set_entity(g, d_state, n, z, d_cells, (cudaStream_t)stream);
@@ -1280,6 +1445,19 @@ extern "C" int cx_get_episode_performance(const cx_game* g, const void* d_state,
   }
   const CxStateLayout L = cx_layout(g, n);
   CX_CUDA_OK(cudaMemcpyAsync(d_perf, static_cast<const uint8_t*>(d_state) + L.off_perf, (size_t)n * sizeof(float),
+                             cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+  return CX_OK;
+}
+
+extern "C" int cx_get_pickups(const cx_game* g, const void* d_state, int64_t n, uint64_t* d_bits, void* stream) {
+  int rc = check_common(g, d_state, n, "cx_get_pickups");
+  if (rc) return rc;
+  if (!g->info.n_pickups || !d_bits) {
+    cx_set_error("cx_get_pickups: the game has no pickup drapes, or d_bits is NULL");
+    return CX_ERR_INVALID_ARG;
+  }
+  const CxStateLayout L = cx_layout(g, n);
+  CX_CUDA_OK(cudaMemcpyAsync(d_bits, static_cast<const uint8_t*>(d_state) + L.off_pick, (size_t)n * sizeof(uint64_t),
                              cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
   return CX_OK;
 }

@@ -85,6 +85,39 @@ struct CxAgentHeader {
   CxActionTable act;        // host copy
 };
 
+// ---- collectible items (CX_KIND_PICKUP) of a single-agent game ----
+// The agent tables above are built with every item absent (cx_game_create checks that they equal the tables with
+// every item present), while basech / basek / baselay show every item present: the static scene of a fresh episode.
+// Each env keeps a u64 of the items it still holds (CxStateLayout::off_pick).  The PICK build of k_agent_rollout_obs
+// stages the region below after the observation extension and pokes an item's cell between its present and absent
+// bytes when the bit changes.
+#define CX_MAX_PICKUPS 64
+#define CX_NO_ITEM 0xFF
+struct CxPickItem {          // one item cell
+  uint8_t cell;
+  uint8_t under_ch;          // board character once the item is taken (the static scene without it)
+  uint8_t under_k;           // its channel in the canonical order (0xFF: not a game character)
+  uint8_t drape;             // index into the CxPickDrape array
+};
+struct CxPickDrape {         // one pickup drape
+  uint64_t items;            // bits of its items
+  float reward[CX_MAX_ACTIONS + 1];  // add_reward value of a step that takes one of them (entry_reward[a][own char])
+  float emptied_value;       // discount of the terminate_episode call once the last one is taken
+  int32_t terminates;        // cx_entity_desc::terminate_emptied
+  int32_t pad;
+};
+struct CxPickHeader {
+  int32_t n_items;           // 0: the game has no pickups
+  int32_t after;             // the pickups update after the agent: they see its post-move cell (else its pre-move cell)
+  int32_t off;               // byte offset of the staged region in the blob (16-byte aligned) ...
+  int32_t bytes;             // ... and its size (a multiple of 16)
+  int32_t item_at;           // region offsets: u8 [cells+1] item index of every cell (CX_NO_ITEM: none) ...
+  int32_t items;             // ... CxPickItem [n_items] ...
+  int32_t drapes;            // ... CxPickDrape [n_drapes] (8-byte aligned)
+  int32_t pad;
+  uint64_t all;              // every item present
+};
+
 // ---- generic path tables ----
 struct CxGenEntity {
   uint8_t ch, kind, visible, group;
@@ -195,6 +228,7 @@ struct CxStateLayout {
   int64_t off_dyn;     // agent path: u8 [n]; generic: u16 [n_dyn][n]
   int64_t off_dynbd;   // generic + Q1: u8 [n][cells]
   int64_t off_perf;    // games that track performance: f32 [n] running performance of the current episode
+  int64_t off_pick;    // games with pickups: u64 [n] items each env still holds (CxPickHeader)
   int64_t total;
 };
 
@@ -204,6 +238,7 @@ struct cx_game {
   cx_game_info info;
   CxAgentHeader ah;
   CxGenHeader gh;
+  CxPickHeader ph;         // single-agent games with CX_KIND_PICKUP drapes
   uint8_t* d_blob;         // device tables
   uint8_t* d_chars;        // device copy of chars[] for the layer kernels
   int device;

@@ -13,7 +13,7 @@ import numpy as np
 from . import _native as N
 
 KIND_NAMES = {N.CX_KIND_STATIC: "static", N.CX_KIND_CELL: "cell", N.CX_KIND_ROLL: "roll",
-              N.CX_KIND_SPRITE: "sprite"}
+              N.CX_KIND_SPRITE: "sprite", N.CX_KIND_PICKUP: "pickup"}
 
 
 @dataclasses.dataclass
@@ -36,11 +36,13 @@ class EntitySpec:
     discount: Optional[Dict[int, float]] = None           # action -> change_default_discount value
     visible_op: Optional[List[int]] = None                # sprites, per action: CX_VIS_* applied to Sprite.visible
     z_orders: Optional[Dict[int, List[tuple]]] = None     # action -> [(move_this, in_front_of_that or None), ...]
+    terminate_emptied: Optional[float] = None             # pickups: discount passed to terminate_episode by the step
+                                                          # that takes the last item (None: no such call)
 
     def summary(self):
         out = {"char": self.character, "kind": KIND_NAMES[self.kind], "rank": self.update_rank,
                "group": self.update_group}
-        if self.kind != N.CX_KIND_STATIC:
+        if self.kind not in (N.CX_KIND_STATIC, N.CX_KIND_PICKUP):
             out["moves"] = [tuple(m) for m in (self.moves or [])]
         if self.blockers:
             out["blockers"] = "".join(sorted(self.blockers))
@@ -63,6 +65,8 @@ class EntitySpec:
             out["visible_op"] = [("keep", "show", "hide", "toggle")[v] for v in self.visible_op]
         if self.z_orders:
             out["z_orders"] = {a: list(v) for a, v in sorted(self.z_orders.items())}
+        if self.terminate_emptied is not None:
+            out["terminate_emptied"] = self.terminate_emptied
         return out
 
 
@@ -173,6 +177,8 @@ class GameSpec:
                 for k, (move_this, front_of) in enumerate(zd):
                     c.z_move[a][k] = z_of[move_this]
                     c.z_front[a][k] = -1 if front_of is None else z_of[front_of]
+            if e.terminate_emptied is not None:
+                c.terminate_emptied, c.emptied_value = 1, float(e.terminate_emptied)
         backdrop = np.ascontiguousarray(np.asarray(self.backdrop, dtype=np.uint8).reshape(-1))
         masks = np.ascontiguousarray(masks)
         d.backdrop = backdrop.ctypes.data_as(ctypes.POINTER(ctypes.c_uint8))

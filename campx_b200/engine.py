@@ -367,7 +367,8 @@ class Engine(object):
 
     @property
     def never_rewards(self):
-        return all(e.step_reward is None or all(r is None for r in e.step_reward) for e in self._spec.entities)
+        return all((e.step_reward is None or all(r is None for r in e.step_reward)) and e.kind != N.CX_KIND_PICKUP
+                   for e in self._spec.entities)
 
     @property
     def the_plot(self):
@@ -397,6 +398,24 @@ class Engine(object):
     def positions(self, character):
         """int32 [num_envs] cell index (row*cols+col) of a moving entity; -1 = empty mask."""
         return self._native.entity_state(character)
+
+    def pickup_curtain(self, character):
+        """bool [num_envs, rows, cols]: the curtain of pickup drape `character` in every env -- the items it still
+        holds."""
+        spec = self._spec
+        z_of = {e.character: z for z, e in enumerate(spec.entities)}
+        if character not in z_of or spec.entities[z_of[character]].kind != N.CX_KIND_PICKUP:
+            raise ValueError('{} is not a pickup drape of this game'.format(repr(character)))
+        first = 0                                  # item numbering: pickup drapes in z-order, row-major cells
+        for e in spec.entities[:z_of[character]]:
+            if e.kind == N.CX_KIND_PICKUP:
+                first += int(np.count_nonzero(e.mask))
+        cells = np.flatnonzero(np.asarray(spec.entities[z_of[character]].mask).reshape(-1))
+        dev = self._native.device
+        held = (self._native.pickups()[:, None] >> torch.arange(first, first + len(cells), device=dev)) & 1
+        out = torch.zeros((self._num_envs, self._rows * self._cols), dtype=torch.bool, device=dev)
+        out[:, torch.from_numpy(cells).to(dev)] = held.bool()
+        return out.view(self._num_envs, self._rows, self._cols)
 
     def episode_stats(self):
         return self._native.stats()

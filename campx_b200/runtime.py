@@ -381,6 +381,14 @@ class NativeGame(object):
                                                          _stream()))
         return perf
 
+    def pickups(self):
+        """int64 [num_envs]: bit i set = item i is still on the board (games with pickup drapes).  Items are numbered
+        pickup drape by pickup drape in z-order, row-major within a drape (`Engine.pickup_curtain` unpacks them)."""
+        bits = torch.empty(self.num_envs, dtype=torch.int64, device=self.device)
+        with torch.cuda.device(self.device):
+            N.check(self._lib.cx_get_pickups(self._handle, _ptr(self.state), self.num_envs, _ptr(bits), _stream()))
+        return bits
+
     def fold_stats(self):
         """Add the kernels' partial statistics blocks into the float64[8] block at the head of the state blob
         (asynchronous on the current stream)."""

@@ -5,6 +5,7 @@ tensors.  They are behaviourally identical to the reference's worlds
     boat_race     examples/boat_race.py:16-115
     demo1..demo4  the `Demo 1..4` notebooks (game cells)
     hello         `Hello World Example.ipynb` cells 3-4
+    coins         a "collect the coins" maze (not a reference world): `Coin` is the plain collectible-item drape
 
 (checked frame by frame against tests/golden/, which was recorded from the reference itself) but are
 not copies of them.  Nothing here is batched or GPU-aware: `ascii_art_to_game(..., num_envs=N)`
@@ -46,6 +47,16 @@ HELLO_ART = ['                                    ',
              '     @ @ @ @   @ @   @ @    @   @   ',
              '      @@@   @@@  @   @  @@@ @@@@  4 ',
              '                                    ']
+
+
+COINS_ART = ['##########',
+             '#A $   $ #',
+             '# ##$##  #',
+             '#$ #  #$ #',
+             '#  $ ## $#',
+             '# ##  #  #',
+             '#$   $ $ #',
+             '##########']
 
 
 def _moved(mask, act):
@@ -147,6 +158,25 @@ class Slider(things.Sprite):
         self._position = self.Position(row, col)
 
 
+class Coin(things.Drape):
+    """Collectible items: a coin pays `value` once when the agent stands on it, then disappears; taking the last one
+    ends the episode with discount `pcontinue`."""
+
+    def __init__(self, curtain, character, value=1.0, pcontinue=0.0, agent='A'):
+        super(Coin, self).__init__(curtain, character)
+        self.value, self.pcontinue, self.agent = value, pcontinue, agent
+
+    def update(self, actions, board, layers, backdrop, all_things, the_plot):
+        if actions is None:
+            return
+        here = all_things[self.agent].curtain
+        if (self.curtain * here).sum():
+            self.curtain.set_(self.curtain * (1 - here))
+            the_plot.add_reward(self.value)
+            if not self.curtain.any():
+                the_plot.terminate_episode(self.pcontinue)
+
+
 def _ring_world(cw, ccw, toll, **engine_kwargs):
     def arrow(bonus):
         return Partial(Arrow, bonus=torch.FloatTensor(bonus), toll=toll)
@@ -162,7 +192,10 @@ def _ring_world(cw, ccw, toll, **engine_kwargs):
 
 
 def make_world(name, **engine_kwargs):
-    """Un-started Engine for one of: boat_race, demo1, demo2, demo3, demo4, hello."""
+    """Un-started Engine for one of: boat_race, demo1, demo2, demo3, demo4, hello, coins.
+
+    coins takes two more keywords: `update_schedule` (default 'A$#': the coins see the agent's cell after its move) and
+    `coins` (the Coin drape class, or a Partial of it, default Coin)."""
     if name == 'boat_race':
         return _ring_world(3, 1, -0.25, **engine_kwargs)
     if name == 'demo4':
@@ -184,6 +217,12 @@ def make_world(name, **engine_kwargs):
                                  sprites={'1': Partial(Slider, 0), '2': Partial(Slider, 1),
                                           '3': Partial(Slider, 2), '4': Partial(Slider, 3)},
                                  drapes={'@': Roller}, z_order='12@34', **engine_kwargs)
+    if name == 'coins':
+        schedule = engine_kwargs.pop('update_schedule', 'A$#')
+        coin = engine_kwargs.pop('coins', Coin)
+        return ascii_art_to_game(COINS_ART, ' ',
+                                 drapes={'A': Partial(Walker, walls='#'), '$': coin, '#': things.FixedDrape},
+                                 z_order='$A#', update_schedule=schedule, **engine_kwargs)
     raise KeyError(name)
 
 

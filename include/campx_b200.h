@@ -33,6 +33,8 @@
  *   cx_step_perf                       <-  step_perf() safety metric        examples/boat_race.py:117-151
  *   cx_game_desc::perf_regions,        <-  the same metric inside every single-agent step kernel, per episode
  *   cx_get_episode_performance             (the P / P_av columns of examples/reinforce.py:186-194)
+ *   CX_KIND_PICKUP, cx_get_pickups     <-  a collectible-item Drape (clears the agent's cell, add_reward, and
+ *                                          terminate_episode once empty: the "collect the coins" pattern)
  *   cx_discounted_returns              <-  finish_episode() return scan     examples/actor_critic.py:115-135
  *   cx_fill_actions                    <-  random-action rollouts           examples/actor_critic.py:90-98
  *                                          (synthetic benchmark input; counter-based Philox4x32-10)
@@ -64,7 +66,7 @@ extern "C" {
 #define CX_API
 #endif
 
-#define CX_ABI_VERSION 6
+#define CX_ABI_VERSION 7
 
 #define CX_MAX_ENTITIES 16   /* sprites + drapes in one game                         */
 #define CX_MAX_ACTIONS 8     /* discrete actions                                     */
@@ -86,7 +88,18 @@ typedef enum cx_kind {
   CX_KIND_STATIC = 0, /* Drape whose mask never changes (things.FixedDrape, hover-reward tiles) */
   CX_KIND_CELL = 1,   /* Drape with a one-cell mask that moves (AgentDrape, boat_race.py:28-59)  */
   CX_KIND_ROLL = 2,   /* Drape whose whole mask rolls toroidally (RollingDrape, Hello World)      */
-  CX_KIND_SPRITE = 3  /* Sprite: (row, col) position (SlidingSprite, Hello World)                 */
+  CX_KIND_SPRITE = 3, /* Sprite: (row, col) position (SlidingSprite, Hello World)                 */
+  CX_KIND_PICKUP = 4  /* Drape of collectible items (coins, keys, pellets): when its curtain holds the watched
+                         entity's current cell as it updates, it clears that one cell and calls
+                         add_reward(entry_reward[a][own char]); terminate_emptied: terminate_episode(emptied_value)
+                         when that emptied the curtain.  Nothing else.  Single-agent games only (info.path == 1),
+                         below the agent in z-order, at most 64 item cells in all, none under the agent's initial
+                         cell, no two pickup drapes on one cell, all pickup drapes on the same side of the agent in
+                         the update order and no entity after them calling add_reward / terminate_episode /
+                         change_default_discount, occluded layers, no perf_regions, and nothing else in the game may
+                         depend on whether an item is present (blockers, entry rewards, terminate_chars):
+                         CX_ERR_UNSUPPORTED otherwise.  Items are numbered pickup drape by pickup drape in z-order,
+                         row-major within a drape (cx_get_pickups bit i = item i)                            */
 } cx_kind;
 
 /* Output flag bits, one byte per env-step. */
@@ -141,6 +154,9 @@ typedef struct cx_entity_desc {
                               in call order, then the board is re-rendered (engine.py:242-281,163)     */
   int8_t z_move[CX_MAX_ACTIONS][CX_MAX_ZDIRS];  /* z-index (initial order) of move_this                  */
   int8_t z_front[CX_MAX_ACTIONS][CX_MAX_ZDIRS]; /* z-index of in_front_of_that; -1: None = to the back  */
+  /* --- PICKUP only (ABI 7) --- */
+  uint8_t terminate_emptied; /* 1: the step that takes the drape's last item calls terminate_episode(emptied_value) */
+  float emptied_value;     /* discount passed by that call                                                   */
 } cx_entity_desc;
 
 typedef enum cx_visible_op {
@@ -205,6 +221,7 @@ typedef struct cx_game_info {
                               runs on the general (per-cell painter) kernel                          */
   int32_t tracks_performance; /* cx_game_desc::n_perf_regions > 0: every step kernel keeps the per-env
                               performance and CX_STAT_PERFORMANCE_SUM                                */
+  int32_t n_pickups;       /* item cells of all CX_KIND_PICKUP drapes (0..64); every env keeps which remain */
 } cx_game_info;
 
 /* Episode statistics kept at the head of the state blob (8 doubles), all-reducible as-is. */
@@ -402,6 +419,10 @@ CX_API int cx_get_episode_state(const cx_game* game, const void* d_state, int64_
  * float32. */
 CX_API int cx_get_episode_performance(const cx_game* game, const void* d_state, int64_t n_envs, float* d_perf,
                                       void* stream);
+
+/* Items every env still holds (valid when info.n_pickups > 0): d_bits [n] uint64, bit i set = item i (numbering:
+ * CX_KIND_PICKUP) is still on the board.  cx_reset and an auto reset restore all items; a frozen env keeps its own. */
+CX_API int cx_get_pickups(const cx_game* game, const void* d_state, int64_t n_envs, uint64_t* d_bits, void* stream);
 
 /* The kernels accumulate the episode statistics in partial blocks inside the state blob (one per group of warps, so
  * that their atomics do not serialise on one line).  cx_stats_fold adds them into the float64[CX_STATS_DOUBLES] block at
