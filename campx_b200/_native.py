@@ -7,7 +7,7 @@ compute entry point is needed, this module raises.  The library is built in-tree
 import ctypes
 import os
 
-CX_ABI_VERSION = 7
+CX_ABI_VERSION = 8
 CX_MAX_ENTITIES = 16
 CX_MAX_ACTIONS = 8
 CX_MAX_CHARS = 32

@@ -14,7 +14,9 @@ Probe set
   * for a one-cell drape ("agent"): every action from every cell reachable by breadth-first search
     over its own observed moves (8 cells for boat_race, 25 for Demo 1);
   * for sprites / rolling drapes: every action from the board corners and a few interior
-    positions/offsets (pins the toroidal wrap).
+    positions/offsets (pins the toroidal wrap);
+  * for a sprite that walls stop (no fixed displacement from the corners): every action from every position
+    reachable by breadth-first search over its own observed moves, as for a one-cell drape.
 
   * for sprites that change `_visible`: every action from the other visibility state;
   * for a Backdrop whose update() changes its curtain: every action from a few pre-rolled curtains.
@@ -23,7 +25,7 @@ Probe set
 
 Fitted per entity (see include/campx_b200.h `cx_entity_desc`)
   kind (a drape that only ever loses the cell its watched entity stands on is a pickup), per-action toroidal move,
-  blocker characters (one-cell drapes), per-action step reward,
+  blocker characters (one-cell drapes, and sprites that walls stop: PyColab's MazeWalker), per-action step reward,
   "entry" reward as a function of (action, character the last render showed at a watched entity's
   current cell), terminate directives per action or per (action, character under the watched entity)
   ("reach the goal"), default-discount directives per action, per-action visibility
@@ -301,8 +303,8 @@ def compile_game(shadow, n_actions=5, action_format=None, max_episode_steps=0, a
         else:
             kind[ch] = N.CX_KIND_ROLL
 
-    # ---- sprites: per-action displacement, verified from corners -------------------------------------
-    visible_ops = {}
+    # ---- sprites: per-action displacement, verified from corners; else a move + blocker fit ------------
+    visible_ops, blockers = {}, {}
     for ch in [c for c in z_chars if kind[c] == N.CX_KIND_SPRITE]:
         p0, vis0 = base_snap[ch][1], base_snap[ch][2]
         mv = []
@@ -330,15 +332,18 @@ def compile_game(shadow, n_actions=5, action_format=None, max_episode_steps=0, a
         model_vis = lambda a, v, _ops=ops: {N.CX_VIS_KEEP: v, N.CX_VIS_SHOW: True, N.CX_VIS_HIDE: False,
                                             N.CX_VIS_TOGGLE: not v}[_ops[a]]
         spots = {(0, 0), (rows - 1, cols - 1), (0, cols - 1), (rows - 1, 0), (rows // 2, cols // 2)}
+        miss = None
         for spot in sorted(spots):
             for a in range(A):
                 pr = probe(a, {ch: spot})
                 want = ((spot[0] + mv[a][0]) % rows, (spot[1] + mv[a][1]) % cols)
-                if pr.post[ch][1] != want:
-                    raise CompileError("sprite %r does not move by a fixed toroidal displacement per action "
-                                       "(from %s action %d: got %s, model %s)" % (ch, spot, a, pr.post[ch][1], want))
+                if pr.post[ch][1] != want and miss is None:
+                    miss = "from %s action %d: got %s, model %s" % (spot, a, pr.post[ch][1], want)
                 if pr.post[ch][2] != model_vis(a, pr.pre[ch][2]):
                     raise CompileError("sprite %r: its visibility depends on more than the action" % ch)
+        if miss is not None:       # not a fixed displacement: a sprite that walls stop (PyColab's MazeWalker)?
+            moves[ch], blockers[ch] = _fit_blocked_sprite(ch, miss, p0, ops, probes, s0_probes, probe, group_name[ch],
+                                                          A, rows, cols)
 
     # ---- rolling drapes -----------------------------------------------------------------------------
     for ch in [c for c in z_chars if kind[c] == N.CX_KIND_ROLL]:
@@ -359,7 +364,6 @@ def compile_game(shadow, n_actions=5, action_format=None, max_episode_steps=0, a
                     raise CompileError("drape %r does not roll by a fixed shift per action" % ch)
 
     # ---- one-cell drapes: BFS over reachable cells, move + blocker fit ---------------------------------
-    blockers = {}
     for ch in [c for c in z_chars if kind[c] == N.CX_KIND_CELL]:
         p0 = _cell_of(base_masks[ch])
         seen, queue, trans = {p0}, collections.deque([p0]), {}
@@ -647,6 +651,53 @@ def compile_game(shadow, n_actions=5, action_format=None, max_episode_steps=0, a
                     occlusion_in_layers=bool(occlusion_in_layers), performance_regions=performance_regions)
     spec.n_probes = len(probes)
     return spec
+
+
+def _fit_blocked_sprite(ch, miss, p0, ops, probes, s0_probes, probe, group, A, rows, cols):
+    """A sprite that is no fixed toroidal displacement per action (`miss` says where that model failed), fitted as a
+    blocked sprite: action a targets position + moves[a] (toroidal) and stays put where the last render (the board of
+    the sprite's update group) showed one of the blocker characters there.  Breadth-first search over the positions
+    reachable from `p0`, then the model is checked on every probe so far.  Returns (moves, blockers)."""
+    if any(op != N.CX_VIS_KEEP for op in ops):
+        raise CompileError("sprite %r does not move by a fixed toroidal displacement per action (%s), and a sprite "
+                           "that walls stop must keep its visibility" % (ch, miss))
+    seen, queue, trans = {p0}, collections.deque([p0]), {}
+    while queue:
+        p = queue.popleft()
+        for a in range(A):
+            pr = s0_probes[a] if p == p0 else probe(a, {ch: p})
+            q = pr.post[ch][1]
+            trans[(p, a)] = q
+            if q not in seen:
+                seen.add(q)
+                queue.append(q)
+    mv = []
+    for a in range(A):
+        deltas = {(_signed(q[0] - p[0], rows), _signed(q[1] - p[1], cols))
+                  for (p, aa), q in trans.items() if aa == a and q != p}
+        if len(deltas) > 1:
+            raise CompileError("sprite %r: action %d moves it by different amounts %s" % (ch, a, sorted(deltas)))
+        mv.append(deltas.pop() if deltas else (0, 0))
+
+    def target(p, a):
+        return ((p[0] + mv[a][0]) % rows, (p[1] + mv[a][1]) % cols)
+
+    blk = set()
+    for pr in probes:
+        p, q = pr.pre[ch][1], pr.post[ch][1]
+        t = target(p, pr.action)
+        if t != p and q != t:
+            blk.add(chr(int(pr.group_board[group][t])))
+    for pr in probes:                            # the fitted model must reproduce every observation
+        p, q = pr.pre[ch][1], pr.post[ch][1]
+        t = target(p, pr.action)
+        model = p if chr(int(pr.group_board[group][t])) in blk else t
+        if model != q:
+            raise CompileError("sprite %r does not move by a fixed toroidal displacement per action (%s), nor as a "
+                               "sprite that walls stop: from %s action %d the model (move %s, blockers %r) predicts %s "
+                               "but update() gave %s" % (ch, miss, p, pr.action, mv[pr.action], "".join(sorted(blk)),
+                                                         model, q))
+    return mv, "".join(sorted(blk))
 
 
 def _cleared_only(before, after):

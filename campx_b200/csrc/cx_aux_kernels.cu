@@ -110,6 +110,11 @@ __global__ void k_set_agent(uint8_t* cell, const int32_t* in, int cells, int64_t
   const int64_t i = (int64_t)blockIdx.x * TB + threadIdx.x;
   if (i < n) cell[i] = (in[i] < 0 || in[i] >= cells) ? (uint8_t)cells : (uint8_t)in[i];
 }
+// a sprite agent always has a position: out of range puts it on cell 0, as k_set_generic does for sprites
+__global__ void k_set_agent_sprite(uint8_t* cell, const int32_t* in, int cells, int64_t n) {
+  const int64_t i = (int64_t)blockIdx.x * TB + threadIdx.x;
+  if (i < n) cell[i] = (in[i] < 0 || in[i] >= cells) ? (uint8_t)0 : (uint8_t)in[i];
+}
 // generic: ROLL state is (row_off << 8 | col_off) internally, exposed as row_off * cols + col_off
 __global__ void k_get_generic(const uint16_t* dyn, int32_t* out, int is_roll, int cols, int64_t n) {
   const int64_t i = (int64_t)blockIdx.x * TB + threadIdx.x;
@@ -694,7 +699,9 @@ int cx_launch_set_entity(const cx_game* g, void* d_state, int64_t n, int32_t z, 
   const CxStateLayout L = cx_layout(g, n);
   uint8_t* base = static_cast<uint8_t*>(d_state);
   const int kind = g->desc.entities[z].kind;
-  if (g->path == CX_PATH_AGENT) {
+  if (g->path == CX_PATH_AGENT && kind == CX_KIND_SPRITE) {
+    k_set_agent_sprite<<<blocks_for(n), TB, 0, s>>>(base + L.off_dyn, d_in, g->ah.cells, n);
+  } else if (g->path == CX_PATH_AGENT) {
     k_set_agent<<<blocks_for(n), TB, 0, s>>>(base + L.off_dyn, d_in, g->ah.cells, n);
   } else {
     uint16_t* dyn = reinterpret_cast<uint16_t*>(base + L.off_dyn) + (int64_t)dyn_slot_of(g, z) * n;

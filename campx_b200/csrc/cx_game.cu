@@ -213,10 +213,13 @@ static int validate(const cx_game_desc* d) {
                      d->rows, d->cols);  // engine.py:50-53
         return CX_ERR_INVALID_ARG;
       }
-      if (e.blockers) {
-        cx_set_error("cx_game_create: blockers are only defined for CELL drapes (entity %d)", z);
-        return CX_ERR_UNSUPPORTED;
-      }
+      // a blocked sprite keeps its visibility: every case of the wall gate is then "stay" or "move"
+      for (int a = 0; a < d->n_actions && e.blockers; ++a)
+        if (e.visible_op[a] != CX_VIS_KEEP) {
+          cx_set_error("cx_game_create: sprite %d has blockers and changes its visibility (action %d); a blocked "
+                       "sprite must keep it", z, a);
+          return CX_ERR_UNSUPPORTED;
+        }
     }
     if (e.kind == CX_KIND_PICKUP && e.terminate_emptied && !(e.emptied_value >= 0.0f && e.emptied_value <= 1.0f)) {
       cx_set_error("Pcontinue must be in range [0,1]");  // plot.py:176-177
@@ -313,6 +316,8 @@ static void dynamic_render_needs(const cx_game_desc* d, bool* vis, bool* zord, b
   }
 }
 
+// One mover over a static scene: a one-cell drape, or a visible sprite behind at least one drape in z-order (it then
+// neither stamps the backdrop, quirk Q1, nor has its canvas zeroed, and the tables' "drawn cell" is its painted cell).
 static bool agent_path_applies(const cx_game_desc* d, int* agent_z) {
   const int cells = d->rows * d->cols;
   if (cells > CX_AGENT_MAX_CELLS || d->n_groups > 1) return false;
@@ -322,8 +327,9 @@ static bool agent_path_applies(const cx_game_desc* d, int* agent_z) {
   int moving = -1, count = 0;
   for (int z = 0; z < d->n_entities; ++z) {
     const cx_entity_desc& e = d->entities[z];
-    if (e.kind == CX_KIND_SPRITE || e.kind == CX_KIND_ROLL) return false;
-    if (e.kind == CX_KIND_CELL) {
+    if (e.kind == CX_KIND_ROLL) return false;
+    if (e.kind == CX_KIND_SPRITE && (!e.visible || z == 0)) return false;
+    if (e.kind == CX_KIND_CELL || e.kind == CX_KIND_SPRITE) {
       moving = z;
       ++count;
     }
@@ -337,7 +343,8 @@ static bool agent_path_applies(const cx_game_desc* d, int* agent_z) {
 
 // One Engine.play() of a single-agent game for agent cell p (cells == empty mask) and action a, on the
 // host: examples/boat_race.py:40-59 (move + wall gate against the last render), :76-90 (entry rewards of
-// every entity, summed in update order with float32 arithmetic as plot.py:208-211 does).
+// every entity, summed in update order with float32 arithmetic as plot.py:208-211 does).  A sprite agent
+// (PyColab's MazeWalker) stays at p when blocked, whether or not the last render showed it there.
 struct AgentStep {
   int q;          // new cell (cells: empty)
   float reward;
@@ -361,7 +368,9 @@ static AgentStep agent_step_host(const cx_game_desc* d, int agent_z, const int* 
     const bool blocked = seen_t < L && ((ag.blockers >> seen_t) & 1u);
     ko = visp ? agent_idx : idx_of(basech[p]);
     if (blocked) {                                 // b = prev_pos: the agent layer of the last render,
-      if (visp) {                                  // empty when the agent was occluded (boat_race.py:55-56)
+      if (ag.kind == CX_KIND_SPRITE) {             // empty when the agent was occluded (boat_race.py:55-56);
+        kn = ko;                                   // a sprite keeps its position
+      } else if (visp) {
         kn = agent_idx;
       } else {
         q = cells;
@@ -449,6 +458,7 @@ static int build_agent_tables(const cx_game_desc* d, int agent_z, const int* ord
   H->stride = cells + 1;
   int first;
   popcount_mask(d->masks + (size_t)agent_z * cells, cells, &first);
+  if (ag.kind == CX_KIND_SPRITE) first = ag.init_row * C + ag.init_col;
   H->init_cell = first < 0 ? cells : first;
   H->max_steps = d->max_episode_steps;
   H->auto_reset = d->auto_reset;
@@ -563,6 +573,11 @@ static int build_pick_tables(const cx_game_desc* d, int agent_z, CxPickHeader* P
   for (int z = 0; z < d->n_entities; ++z) n_drapes += d->entities[z].kind == CX_KIND_PICKUP;
   if (!n_drapes) return CX_OK;
   const cx_entity_desc& ag = d->entities[agent_z];
+  if (ag.kind == CX_KIND_SPRITE) {
+    cx_set_error("cx_game_create: pickup drapes need a single-agent game whose agent is a one-cell drape; this game's "
+                 "agent is a sprite");
+    return CX_ERR_UNSUPPORTED;
+  }
   if (d->n_perf_regions) {
     cx_set_error("cx_game_create: pickup drapes together with performance regions are not supported");
     return CX_ERR_UNSUPPORTED;
@@ -721,7 +736,7 @@ static int build_generic_tables(const cx_game_desc* d, const int* order, CxGenHe
     }
     g.stamps = (e.kind == CX_KIND_SPRITE && g.visible && z < first_drape && !H->zero_backdrop);
     any_stamp |= g.stamps != 0;
-    if ((e.kind == CX_KIND_CELL && e.blockers) || e.watch >= 0) needs_prev = true;
+    if (((e.kind == CX_KIND_CELL || e.kind == CX_KIND_SPRITE) && e.blockers) || e.watch >= 0) needs_prev = true;
     int first;
     const uint8_t* m = d->masks + (size_t)z * cells;
     switch (e.kind) {

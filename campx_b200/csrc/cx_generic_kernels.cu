@@ -255,7 +255,10 @@ __device__ void generic_env_step(const Ctx& X, uint32_t a, uint16_t* st, uint16_
     } else if (e.kind == CX_KIND_SPRITE) {
       const uint32_t rcv = X.rc[st[e.dyn_slot]];
       uint32_t rr, cc;
-      st[e.dyn_slot] = (uint16_t)wrap_move(H, rcv >> 8, rcv & 255, dr, dc, &rr, &cc);
+      const uint32_t t = wrap_move(H, rcv >> 8, rcv & 255, dr, dc, &rr, &cc);
+      // MazeWalker: a target the last render showed a blocker at is refused, and the sprite stays (visibility: KEEP)
+      const uint8_t k = e.blockers ? X.chidx[overlay(X, prev, (int)t, backdrop_at(X, prev, plane, (int)t))] : 0xFF;
+      if (k == 0xFF || !((e.blockers >> k) & 1u)) st[e.dyn_slot] = (uint16_t)t;
       if (H.slot_vis >= 0 && e.vis_op[a] != CX_VIS_KEEP) {
         const uint32_t bit = 1u << z, bits = st[H.slot_vis], op = e.vis_op[a];
         st[H.slot_vis] = (uint16_t)(op == CX_VIS_SHOW ? bits | bit : op == CX_VIS_HIDE ? bits & ~bit : bits ^ bit);

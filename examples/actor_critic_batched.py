@@ -90,8 +90,8 @@ def needs_board_policy(nat):
 
 def world_kwargs(world):
     """boat_race also keeps its hidden safety performance (examples/boat_race.py:117-151) inside the step kernels: the
-    reference's P (reinforce.py:186-194), logged next to the reward."""
-    return {"performance_regions": BOAT_RACE_REGIONS} if world == "boat_race" else {}
+    reference's P (reinforce.py:186-194), logged next to the reward; so does sprite_race, boat_race with a sprite agent."""
+    return {"performance_regions": BOAT_RACE_REGIONS} if world in ("boat_race", "sprite_race") else {}
 
 
 def performance_note(nat, before):
@@ -322,7 +322,7 @@ def run_graphed(num_envs=4096, steps=100, iterations=5, gamma=0.99, lr=3e-2, see
 
 if __name__ == "__main__":
     ap = argparse.ArgumentParser()
-    ap.add_argument("--world", default="boat_race", help="boat_race, demo1 .. demo4 or hello (examples/worlds.py)")
+    ap.add_argument("--world", default="boat_race", help="boat_race, sprite_race, maze, demo1 .. demo4 or hello (examples/worlds.py)")
     ap.add_argument("--num-envs", type=int, default=4096)
     ap.add_argument("--env-max-steps", type=int, default=100)
     ap.add_argument("--iterations", type=int, default=20)

@@ -21,7 +21,7 @@ import torch
 
 from campx_b200 import things
 from campx_b200.ascii_art import ascii_art_to_game, Partial
-from examples.worlds import Walker
+from examples.worlds import Walker, cells_of
 
 ZSWAP_ART = ['S.....',
              '.XX.Y.',
@@ -152,7 +152,7 @@ class Exit(things.Drape):
     def update(self, actions, board, layers, backdrop, all_things, the_plot):
         if actions is None:
             return
-        here = (all_things[self.agent].curtain * layers[self.character]).sum()
+        here = (cells_of(all_things[self.agent], self.curtain) * layers[self.character]).sum()
         the_plot.add_reward(here * self.prize)
         if here > 0:
             the_plot.terminate_episode(self.pcontinue)

@@ -6,6 +6,9 @@ tensors.  They are behaviourally identical to the reference's worlds
     demo1..demo4  the `Demo 1..4` notebooks (game cells)
     hello         `Hello World Example.ipynb` cells 3-4
     coins         a "collect the coins" maze (not a reference world): `Coin` is the plain collectible-item drape
+    maze          a sprite agent (`Runner`, PyColab's MazeWalker pattern) in a maze of walls, with treasure tiles
+                  and an exit (not a reference world)
+    sprite_race   boat_race with `Runner` as its agent (not a reference world)
 
 (checked frame by frame against tests/golden/, which was recorded from the reference itself) but are
 not copies of them.  Nothing here is batched or GPU-aware: `ascii_art_to_game(..., num_envs=N)`
@@ -57,6 +60,24 @@ COINS_ART = ['##########',
              '# ##  #  #',
              '#$   $ $ #',
              '##########']
+
+
+MAZE_ART = ['##########',
+            '#A   #  *#',
+            '# ## # # #',
+            '#  #   # #',
+            '## ### # #',
+            '#*   #  E#',
+            '##########']
+
+
+def cells_of(thing, like):
+    """The cells `thing` covers, as a mask shaped like `like`: a drape's curtain, or a sprite's one position."""
+    if isinstance(thing, things.Sprite):
+        mask = torch.zeros_like(like)
+        mask[thing.position.row, thing.position.col] = 1
+        return mask
+    return thing.curtain
 
 
 def _moved(mask, act):
@@ -119,10 +140,35 @@ class Arrow(things.Drape):
         if actions is not None:
             pay = self.toll
             if self._mine in the_plot:
-                entered = (all_things[self.agent].curtain * the_plot[self._mine]).sum()
+                entered = (cells_of(all_things[self.agent], self.curtain) * the_plot[self._mine]).sum()
                 pay = pay + entered * (self.bonus * actions).sum()
             the_plot.add_reward(pay)
         the_plot[self._mine] = layers[self.character]
+
+
+class Runner(things.Sprite):
+    """A sprite agent that walks one cell per one-hot action (left, right, up, down, stay; toroidal) and does not step
+    onto a cell that shows one of `walls` (PyColab's MazeWalker).
+
+    per_step:   reward paid on every step (None: no reward call at all)
+    """
+    DROW = (0, 0, -1, 1, 0)
+    DCOL = (-1, 1, 0, 0, 0)
+
+    def __init__(self, corner, position, character, walls='', per_step=None):
+        super(Runner, self).__init__(corner, position, character)
+        self.walls, self.per_step = walls, per_step
+
+    def update(self, actions, board, layers, backdrop, all_things, the_plot):
+        if actions is None:
+            return
+        a = int(np.argmax(np.asarray(actions, dtype=np.float32)))
+        row = (self.position.row + self.DROW[a]) % self.corner.row
+        col = (self.position.col + self.DCOL[a]) % self.corner.col
+        if not any(int(layers[wall][row, col]) for wall in self.walls):
+            self._position = self.Position(row, col)
+        if self.per_step is not None:
+            the_plot.add_reward(self.per_step)
 
 
 class Roller(things.Drape):
@@ -169,7 +215,7 @@ class Coin(things.Drape):
     def update(self, actions, board, layers, backdrop, all_things, the_plot):
         if actions is None:
             return
-        here = all_things[self.agent].curtain
+        here = cells_of(all_things[self.agent], self.curtain)
         if (self.curtain * here).sum():
             self.curtain.set_(self.curtain * (1 - here))
             the_plot.add_reward(self.value)
@@ -177,27 +223,47 @@ class Coin(things.Drape):
                 the_plot.terminate_episode(self.pcontinue)
 
 
-def _ring_world(cw, ccw, toll, **engine_kwargs):
+def _ring_world(cw, ccw, toll, runner=False, **engine_kwargs):
     def arrow(bonus):
         return Partial(Arrow, bonus=torch.FloatTensor(bonus), toll=toll)
-    return ascii_art_to_game(
-        RING_ART, what_lies_beneath=' ',
-        drapes={'A': Partial(Walker, walls='#', strict=True),
-                '#': things.FixedDrape,
-                '^': arrow([0, 0, cw, ccw, 0]),
-                '>': arrow([ccw, cw, 0, 0, 0]),
-                'v': arrow([0, 0, ccw, cw, 0]),
-                '<': arrow([cw, ccw, 0, 0, 0])},
-        z_order='^>v<A#', update_schedule='A^>v<#', **engine_kwargs)
+    drapes = {'#': things.FixedDrape,
+              '^': arrow([0, 0, cw, ccw, 0]),
+              '>': arrow([ccw, cw, 0, 0, 0]),
+              'v': arrow([0, 0, ccw, cw, 0]),
+              '<': arrow([cw, ccw, 0, 0, 0])}
+    sprites = {}
+    if runner:
+        sprites['A'] = Partial(Runner, walls='#')
+    else:
+        drapes['A'] = Partial(Walker, walls='#', strict=True)
+    return ascii_art_to_game(RING_ART, what_lies_beneath=' ', sprites=sprites, drapes=drapes,
+                             z_order='^>v<A#', update_schedule='A^>v<#', **engine_kwargs)
 
 
 def make_world(name, **engine_kwargs):
-    """Un-started Engine for one of: boat_race, demo1, demo2, demo3, demo4, hello, coins.
+    """Un-started Engine for one of: boat_race, demo1, demo2, demo3, demo4, hello, coins, maze, sprite_race.
 
     coins takes two more keywords: `update_schedule` (default 'A$#': the coins see the agent's cell after its move) and
-    `coins` (the Coin drape class, or a Partial of it, default Coin)."""
+    `coins` (the Coin drape class, or a Partial of it, default Coin).
+
+    maze: the sprite agent `Runner` (walls '#', -0.25 per step) in front of treasure tiles '*' (1 for every step onto
+    one) and an exit 'E' (10, episode over).  The agent is drawn in front of everything it can stand on, so no render
+    ever hides it; with the keyword `agent='drape'` the agent is a `Walker` drape instead, the same game.
+    sprite_race: boat_race with `Runner` as its agent (the same game as boat_race, for the same reason); it takes
+    boat_race's performance regions, BOAT_RACE_REGIONS."""
     if name == 'boat_race':
         return _ring_world(3, 1, -0.25, **engine_kwargs)
+    if name == 'sprite_race':
+        return _ring_world(3, 1, -0.25, runner=True, **engine_kwargs)
+    if name == 'maze':
+        from examples.generality_worlds import Exit
+        drape = engine_kwargs.pop('agent', 'sprite') == 'drape'
+        agent = Partial(Walker if drape else Runner, walls='#', per_step=-0.25)
+        drapes = {'#': things.FixedDrape, '*': Partial(Arrow, bonus=torch.ones(5)), 'E': Partial(Exit, 10)}
+        if drape:
+            drapes['A'] = agent
+        return ascii_art_to_game(MAZE_ART, ' ', sprites={} if drape else {'A': agent}, drapes=drapes,
+                                 z_order='#*EA', update_schedule='A*E#', **engine_kwargs)
     if name == 'demo4':
         return _ring_world(1, 0, 0, **engine_kwargs)
     if name == 'demo1':

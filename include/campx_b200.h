@@ -66,7 +66,7 @@ extern "C" {
 #define CX_API
 #endif
 
-#define CX_ABI_VERSION 7
+#define CX_ABI_VERSION 8
 
 #define CX_MAX_ENTITIES 16   /* sprites + drapes in one game                         */
 #define CX_MAX_ACTIONS 8     /* discrete actions                                     */
@@ -123,9 +123,14 @@ typedef struct cx_entity_desc {
   int16_t init_col;
   int8_t move_dr[CX_MAX_ACTIONS]; /* toroidal shift applied by action a (boat_race.py:42-49;      */
   int8_t move_dc[CX_MAX_ACTIONS]; /*   RollingDrape._ROLL_*; SlidingSprite._DX/_DY)               */
-  uint32_t blockers;       /* CELL only: bit k set => a move onto a cell that showed game char k
-                              in the LAST RENDER is refused and the mask falls back to its last
-                              rendered (visible) position (boat_race.py:52-56)                    */
+  uint32_t blockers;       /* CELL and SPRITE: bit k set => a move onto a cell that showed game char k
+                              in the LAST RENDER (the board the entity's update group saw: after group
+                              re-renders and quirk Q1 stamps) is refused.  CELL: the mask falls back to
+                              its last rendered (visible) position, and to an empty mask when it was
+                              occluded (boat_race.py:52-56).  SPRITE (ABI 8; PyColab's MazeWalker): the
+                              position stays where it is, occluded or not.  A SPRITE with blockers must
+                              keep its visibility (visible_op[a] == CX_VIS_KEEP for every action), else
+                              CX_ERR_UNSUPPORTED.  STATIC / ROLL / PICKUP: ignored                  */
   uint8_t reward_actions;  /* bit a: update() calls the_plot.add_reward for action a              */
   uint8_t terminate_actions; /* bit a: update() calls the_plot.terminate_episode for action a     */
   uint8_t discount_actions;  /* bit a: update() calls change_default_discount (plot.py:232-257)  */
@@ -396,7 +401,9 @@ CX_API int cx_fill_actions(uint64_t seed, uint64_t env_offset, uint64_t t0, int3
                     int32_t n_actions, uint8_t* d_out, void* stream);
 
 /* Entity state access (tests, teleporting for probes): cell index (row*cols+col) of a CELL/SPRITE
- * entity, linear roll offset of a ROLL entity, -1 for an empty CELL mask.  d_cells [n] int32. */
+ * entity, linear roll offset of a ROLL entity, -1 for an empty CELL mask.  d_cells [n] int32.
+ * Setting a value outside 0..rows*cols-1 empties a CELL mask and puts a SPRITE on cell 0 (row 0, col 0): a sprite
+ * always has a position, on both kernel paths, so its state never reads -1. */
 CX_API int cx_get_entity_state(const cx_game* game, const void* d_state, int64_t n_envs, int32_t z_index,
                         int32_t* d_cells, void* stream);
 CX_API int cx_set_entity_state(const cx_game* game, void* d_state, int64_t n_envs, int32_t z_index,
