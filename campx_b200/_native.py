@@ -7,7 +7,7 @@ compute entry point is needed, this module raises.  The library is built in-tree
 import ctypes
 import os
 
-CX_ABI_VERSION = 8
+CX_ABI_VERSION = 9
 CX_MAX_ENTITIES = 16
 CX_MAX_ACTIONS = 8
 CX_MAX_CHARS = 32
@@ -21,8 +21,9 @@ CX_ERR_UNSUPPORTED = -2
 CX_ERR_CUDA = -3
 CX_ERR_NOMEM = -4
 
-CX_KIND_STATIC, CX_KIND_CELL, CX_KIND_ROLL, CX_KIND_SPRITE, CX_KIND_PICKUP = 0, 1, 2, 3, 4
-CX_MAX_PICKUPS = 64          # item cells of all pickup drapes of one game
+CX_KIND_STATIC, CX_KIND_CELL, CX_KIND_ROLL, CX_KIND_SPRITE, CX_KIND_PICKUP, CX_KIND_DOOR = 0, 1, 2, 3, 4, 5
+CX_MAX_PICKUPS = 64          # item cells of all pickup drapes of one game (door games: items plus door cells)
+CX_MAX_DOORS = 3             # door drapes of one game
 CX_VIS_KEEP, CX_VIS_SHOW, CX_VIS_HIDE, CX_VIS_TOGGLE = 0, 1, 2, 3
 
 CX_FLAG_TERMINATED = 0x01
@@ -76,6 +77,7 @@ class EntityDesc(ctypes.Structure):
         ("z_front", (ctypes.c_int8 * CX_MAX_ZDIRS) * CX_MAX_ACTIONS),
         ("terminate_emptied", ctypes.c_uint8),
         ("emptied_value", ctypes.c_float),
+        ("door_key", ctypes.c_int8),
     ]
 
 

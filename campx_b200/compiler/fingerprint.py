@@ -21,10 +21,13 @@ Probe set
   * for sprites that change `_visible`: every action from the other visibility state;
   * for a Backdrop whose update() changes its curtain: every action from a few pre-rolled curtains.
   * for a pickup drape (collectible items): every probe above that took an item again with that item already
-    taken, and with that item as the drape's last one.
+    taken, and with that item as the drape's last one;
+  * for every pickup drape, and for all of them together: the drape emptied, with what that opens open, every action
+    from every cell the agent reaches there; and the drape holding one item only (this is what shows a door).
 
 Fitted per entity (see include/campx_b200.h `cx_entity_desc`)
-  kind (a drape that only ever loses the cell its watched entity stands on is a pickup), per-action toroidal move,
+  kind (a drape that only ever loses the cell its watched entity stands on is a pickup; one that clears all of itself
+  once a pickup drape is empty is a door), per-action toroidal move,
   blocker characters (one-cell drapes, and sprites that walls stop: PyColab's MazeWalker), per-action step reward,
   "entry" reward as a function of (action, character the last render showed at a watched entity's
   current cell), terminate directives per action or per (action, character under the watched entity)
@@ -364,62 +367,58 @@ def compile_game(shadow, n_actions=5, action_format=None, max_episode_steps=0, a
                     raise CompileError("drape %r does not roll by a fixed shift per action" % ch)
 
     # ---- one-cell drapes: BFS over reachable cells, move + blocker fit ---------------------------------
+    reached, observed = {}, {}                     # per one-cell drape: cells reached, [(p, a, q, probe)]
     for ch in [c for c in z_chars if kind[c] == N.CX_KIND_CELL]:
         p0 = _cell_of(base_masks[ch])
-        seen, queue, trans = {p0}, collections.deque([p0]), {}
+        seen, queue, trans = {p0}, collections.deque([p0]), []
         while queue:
             p = queue.popleft()
             for a in range(A):
                 pr = s0_probes[a] if p == p0 else probe(a, {ch: ("cell", p)})
                 q = _cell_of(pr.post[ch][1])
-                trans[(p, a)] = (q, pr)
+                trans.append((p, a, q, pr))
                 if q is not None and q not in seen:
                     if len(seen) >= N.CX_MAX_CELLS:
                         raise CompileError("reachable set too large")
                     seen.add(q)
                     queue.append(q)
-        mv = []
-        for a in range(A):
-            deltas = set()
-            for (p, aa), (q, _) in trans.items():
-                if aa == a and q is not None and q != p:
-                    deltas.add((_signed(q // cols - p // cols, rows), _signed(q % cols - p % cols, cols)))
-            if len(deltas) > 1:
-                raise CompileError("drape %r: action %d moves it by different amounts %s" % (ch, a, sorted(deltas)))
-            mv.append(deltas.pop() if deltas else (0, 0))
-        moves[ch] = mv
-        blk = set()
+        moves[ch], blockers[ch] = _fit_cell_drape(ch, trans, group_name[ch], A, rows, cols)
+        reached[ch], observed[ch] = seen, trans
 
-        def target(p, a):
-            return ((p // cols + mv[a][0]) % rows) * cols + (p % cols + mv[a][1]) % cols
-
-        for (p, a), (q, pr) in trans.items():
-            t = target(p, a)
-            if t != p and q != t:
-                seen_char = int(pr.group_board[group_name[ch]].reshape(-1)[t])
-                blk.add(chr(seen_char))
-        for (p, a), (q, pr) in trans.items():     # the fitted model must reproduce every observation
-            board = pr.group_board[group_name[ch]].reshape(-1)
-            t = target(p, a)
-            vis = int(board[p]) == ord(ch)
-            blocked = chr(int(board[t])) in blk
-            model = (p if vis else None) if blocked else t
-            if model != q:
-                raise CompileError("drape %r: from cell %d action %d the model (move %s, blockers %r) predicts "
-                                   "%s but update() gave %s" % (ch, p, a, mv[a], "".join(sorted(blk)), model, q))
-        blockers[ch] = "".join(sorted(blk))
-
-    # ---- pickup drapes: items the agent collects ----------------------------------------------------------
+    # ---- pickup drapes: items the agent collects; door drapes: opened once a pickup drape is empty ----------
     # A drape that looked static from the initial state may still lose an item once the agent stands elsewhere.
     for ch in z_chars:
         if kind[ch] == N.CX_KIND_STATIC and any(
                 not np.array_equal(pr.post[ch][1], pr.pre[ch][1]) for pr in probes) and all(
                 _cleared_only(pr.pre[ch][1], pr.post[ch][1]) for pr in probes):
             kind[ch] = N.CX_KIND_PICKUP
-    pickups = {}
+    pickups, doors = {}, {}
     if any(k == N.CX_KIND_PICKUP for k in kind.values()):
-        pickups = _fit_pickups(z_chars, kind, base_masks, base_snap, probes, probe, rank, A, rows, cols,
-                               len(base.update_groups), performance_regions, occlusion_in_layers)
+        agent = _pickup_agent(z_chars, kind, rows, cols, len(base.update_groups), performance_regions,
+                              occlusion_in_layers)
+        probed = []
+        while True:
+            # a drape that only ever loses the cell the agent stands on is a pickup; one that changes otherwise (a
+            # whole door opening) may be a door.  The probes with pickup drapes emptied show more of both: a pickup
+            # behind a door, a door that updates before its key.
+            for ch in z_chars:
+                if kind[ch] in (N.CX_KIND_STATIC, N.CX_KIND_PICKUP) and any(
+                        not np.array_equal(pr.post[ch][1], pr.pre[ch][1]) for pr in probes):
+                    kind[ch] = N.CX_KIND_PICKUP if all(
+                        _cleared_only(pr.pre[ch][1], pr.post[ch][1]) and _takes_the_agents_cell(pr, ch, agent)
+                        for pr in probes) else N.CX_KIND_DOOR
+            keys = [c for c in z_chars if kind[c] == N.CX_KIND_PICKUP]
+            fresh = [k for k in keys if k not in probed]
+            if not fresh:
+                break
+            _check_pickup_cells(z_chars, kind, agent, base_masks)
+            scenes = [(k,) for k in fresh] + ([tuple(keys)] if len(keys) > 1 else [])
+            _probe_emptied(scenes, fresh, agent, z_chars, kind, base_masks, reached, observed, probe, A, rows, cols)
+            probed += fresh
+        pickups = _fit_pickups(z_chars, kind, agent, base_masks, probes, probe, A, rows, cols)
+        doors = _fit_doors(z_chars, kind, agent, keys, base_masks, probes, rank)
+        # the agent's move and blockers, checked (and its blockers completed) behind the opened doors too
+        moves[agent], blockers[agent] = _fit_cell_drape(agent, observed[agent], group_name[agent], A, rows, cols)
 
     # ---- backdrop: static apart from the sprite stamps of quirk Q1, or rolled by Backdrop.update() ------------
     def first_drape_of(order_):
@@ -503,6 +502,10 @@ def compile_game(shadow, n_actions=5, action_format=None, max_episode_steps=0, a
             specs.append(EntitySpec(character=ch, kind=N.CX_KIND_PICKUP, mask=base_masks[ch], update_rank=rank[ch],
                                     update_group=group_of[ch], watch=agent,
                                     entry_reward={a: {ch: reward[a]} for a in range(A)}, terminate_emptied=emptied))
+            continue
+        if ch in doors:
+            specs.append(EntitySpec(character=ch, kind=N.CX_KIND_DOOR, mask=base_masks[ch], update_rank=rank[ch],
+                                    update_group=group_of[ch], door_key=doors[ch]))
             continue
         obs = []                                  # (probe, action, f32 reward or None)
         term, disc, zord = {}, {}, {}
@@ -706,13 +709,8 @@ def _cleared_only(before, after):
     return bool(np.isin(after, (0, 1)).all() and np.all(after <= (before != 0)))
 
 
-def _fit_pickups(z_chars, kind, base_masks, base_snap, probes, probe, rank, A, rows, cols, n_groups,
-                 performance_regions, occlusion_in_layers):
-    """Fit every CX_KIND_PICKUP candidate: when its update() runs and its curtain holds the watched agent's current
-    cell (the entry-reward query: the post-move cell if it updates after the agent, the pre-move cell otherwise), it
-    clears that one cell and calls add_reward(r[a]); if that emptied the curtain it may call terminate_episode(v);
-    nothing else.  Probes are added with the item already taken and with it as the last one.  Returns
-    {char: (agent char, [r[a]], v or None)}."""
+def _pickup_agent(z_chars, kind, rows, cols, n_groups, performance_regions, occlusion_in_layers):
+    """The one-cell drape agent of a game with CX_KIND_PICKUP candidates; refuses any other kind of game."""
     chars = [c for c in z_chars if kind[c] == N.CX_KIND_PICKUP]
     cells_ = [c for c in z_chars if kind[c] == N.CX_KIND_CELL]
     for ch in chars:
@@ -725,11 +723,16 @@ def _fit_pickups(z_chars, kind, base_masks, base_snap, probes, probe, rank, A, r
             raise CompileError("pickup drape %r together with performance_regions is not supported" % ch)
         if not occlusion_in_layers:
             raise CompileError("pickup drape %r needs occluded layers (occlusion_in_layers=True)" % ch)
-    agent = cells_[0]
+    return cells_[0]
+
+
+def _check_pickup_cells(z_chars, kind, agent, base_masks):
+    """Where the items of the CX_KIND_PICKUP drapes may lie: below the agent, one drape per cell, none under the agent's
+    initial cell, at most CX_MAX_PICKUPS in all."""
     z = {c: i for i, c in enumerate(z_chars)}
     agent_cell = _cell_of(base_masks[agent])
     owner, total = {}, 0
-    for ch in chars:
+    for ch in [c for c in z_chars if kind[c] == N.CX_KIND_PICKUP]:
         if z[ch] > z[agent]:
             raise CompileError("pickup drape %r lies in front of the agent %r in z-order; it must be below it"
                                % (ch, agent))
@@ -742,6 +745,136 @@ def _fit_pickups(z_chars, kind, base_masks, base_snap, probes, probe, rank, A, r
             total += 1
         if total > N.CX_MAX_PICKUPS:
             raise CompileError("more than %d item cells in all (pickup drape %r)" % (N.CX_MAX_PICKUPS, ch))
+
+
+def _fit_cell_drape(ch, trans, group, A, rows, cols):
+    """Per-action move and blocker characters of one-cell drape `ch` from its observed transitions [(p, a, q, probe)]:
+    action a moves it by one fixed toroidal delta, and a target cell that showed a blocker in the last render (the
+    board of its update group) keeps it where it was drawn (nowhere when it was not drawn).  The model must reproduce
+    every observation."""
+    mv = []
+    for a in range(A):
+        deltas = set()
+        for p, aa, q, _ in trans:
+            if aa == a and q is not None and q != p:
+                deltas.add((_signed(q // cols - p // cols, rows), _signed(q % cols - p % cols, cols)))
+        if len(deltas) > 1:
+            raise CompileError("drape %r: action %d moves it by different amounts %s" % (ch, a, sorted(deltas)))
+        mv.append(deltas.pop() if deltas else (0, 0))
+    blk = set()
+
+    def target(p, a):
+        return ((p // cols + mv[a][0]) % rows) * cols + (p % cols + mv[a][1]) % cols
+
+    for p, a, q, pr in trans:
+        t = target(p, a)
+        if t != p and q != t:
+            seen_char = int(pr.group_board[group].reshape(-1)[t])
+            blk.add(chr(seen_char))
+    for p, a, q, pr in trans:     # the fitted model must reproduce every observation
+        board = pr.group_board[group].reshape(-1)
+        t = target(p, a)
+        vis = int(board[p]) == ord(ch)
+        blocked = chr(int(board[t])) in blk
+        model = (p if vis else None) if blocked else t
+        if model != q:
+            raise CompileError("drape %r: from cell %d action %d the model (move %s, blockers %r) predicts "
+                               "%s but update() gave %s" % (ch, p, a, mv[a], "".join(sorted(blk)), model, q))
+    return mv, "".join(sorted(blk))
+
+
+def _takes_the_agents_cell(pr, ch, agent):
+    """In probe `pr`, drape `ch` lost at most the cell the agent stood on as `ch` updated (the pickup rule)."""
+    pre, post = pr.pre[ch][1].reshape(-1), pr.post[ch][1].reshape(-1)
+    c = _cell_of(pr.after[ch][agent][1])
+    model = pre.copy()
+    if c is not None:
+        model[c] = 0
+    return np.array_equal(post, pre) or np.array_equal(post, model)
+
+
+def _probe_emptied(scenes, keys, agent, z_chars, kind, base_masks, reached, observed, probe, A, rows, cols):
+    """Probes of the states the initial one does not show: the pickup drapes of each scene emptied, with whatever that
+    opened open, every action from every cell the agent reaches there by breadth-first search (starting from every
+    cell it reached before); and each of `keys` holding one item only, every action from the agent's start.  Every fit
+    runs on them: a door opens in them, the cells behind it are reached, and an entity that depends on a drape's
+    emptying some other way is refused.  The agent's transitions go to `observed`, the cells it reached to
+    `reached`."""
+    cells = reached[agent]
+    for emptied in scenes:
+        scene = {k: ("mask", np.zeros((rows, cols), np.uint8)) for k in emptied}
+        seed = probe(A - 1, dict(scene))          # one step on: the drapes that open when these are empty are open
+        for c in z_chars:
+            if kind[c] in (N.CX_KIND_STATIC, N.CX_KIND_DOOR) and not np.array_equal(seed.post[c][1], seed.pre[c][1]):
+                scene[c] = ("mask", seed.post[c][1].astype(np.uint8))
+        seen, queue = set(cells), collections.deque(sorted(cells))
+        while queue:
+            p = queue.popleft()
+            for a in range(A):
+                pr = probe(a, dict(scene, **{agent: ("cell", p)}))
+                q = _cell_of(pr.post[agent][1])
+                observed[agent].append((p, a, q, pr))
+                if q is not None and q not in seen:
+                    seen.add(q)
+                    queue.append(q)
+        cells |= seen
+    for k in keys:
+        for c in np.flatnonzero(base_masks[k].reshape(-1)):
+            one = np.zeros(rows * cols, np.uint8)
+            one[c] = 1
+            for a in range(A):
+                probe(a, {k: ("mask", one.reshape(rows, cols))})
+
+
+def _fit_doors(z_chars, kind, agent, keys, base_masks, probes, rank):
+    """Fit every CX_KIND_DOOR candidate D: a drape whose curtain stays what it was while one pickup drape K (its key)
+    still holds an item as D updates, and is empty from the first update that finds K empty on; D calls no plot
+    directive.  Returns {door char: key char}."""
+    z = {c: i for i, c in enumerate(z_chars)}
+    out = {}
+    for ch in [c for c in z_chars if kind[c] == N.CX_KIND_DOOR]:
+        def opens_with(k):
+            for pr in probes:
+                pre, post = pr.pre[ch][1], pr.post[ch][1]
+                if not np.array_equal(post, pre if pr.after[ch][k][1].any() else np.zeros_like(pre)):
+                    return False
+            return True
+        key = next((k for k in keys if opens_with(k)), None)
+        if key is None:
+            raise CompileError("drape %r changes its curtain in a way that is neither static, a pickup nor a door (a "
+                               "door keeps its whole curtain while one pickup drape holds an item, and clears all of it "
+                               "once that drape is empty)" % ch)
+        events = sorted({k for pr in probes for k, _ in pr.events.get(ch, ())})
+        if events:
+            raise CompileError("door drape %r calls %s; a door may call no plot directive" % (ch, events))
+        if rank[ch] < rank[key]:
+            raise CompileError("door drape %r updates before its key drape %r, so it opens one step after the key is "
+                               "taken; a door must update after its key" % (ch, key))
+        if z[ch] > z[agent]:
+            raise CompileError("door drape %r lies in front of the agent %r in z-order; it must be below it"
+                               % (ch, agent))
+        m = base_masks[ch].reshape(-1) != 0
+        for k in keys:
+            if (m & (base_masks[k].reshape(-1) != 0)).any():
+                raise CompileError("door drape %r shares a cell with an item of pickup drape %r" % (ch, k))
+        if m[_cell_of(base_masks[agent])]:
+            raise CompileError("door drape %r covers the agent's initial cell" % ch)
+        for other in out:
+            if (m & (base_masks[other].reshape(-1) != 0)).any():
+                raise CompileError("door drapes %r and %r share a cell" % (other, ch))
+        out[ch] = key
+        if len(out) > N.CX_MAX_DOORS:
+            raise CompileError("more than %d door drapes (door drape %r)" % (N.CX_MAX_DOORS, ch))
+    return out
+
+
+def _fit_pickups(z_chars, kind, agent, base_masks, probes, probe, A, rows, cols):
+    """Fit every CX_KIND_PICKUP candidate: when its update() runs and its curtain holds the watched agent's current
+    cell (the entry-reward query: the post-move cell if it updates after the agent, the pre-move cell otherwise), it
+    clears that one cell and calls add_reward(r[a]); if that emptied the curtain it may call terminate_episode(v);
+    nothing else.  Probes are added with the item already taken and with it as the last one.  Returns
+    {char: (agent char, [r[a]], v or None)}."""
+    chars = [c for c in z_chars if kind[c] == N.CX_KIND_PICKUP]
 
     def watched(pr, ch):
         return _cell_of(pr.after[ch][agent][1])

@@ -24,7 +24,9 @@
 //
 // Games with collectible items (CX_KIND_PICKUP) run only here, in the PICK build: each lane keeps its env's u64 of
 // remaining items (CxPickHeader) and every ring slot remembers which items it shows; an item whose bit differs is
-// poked between its present and absent bytes (board and layered tile) when the slot comes up.
+// poked between its present and absent bytes (board and layered tile) when the slot comes up.  Key-locked doors
+// (CX_KIND_DOOR) are a function of the items: a step looks its (action, cell) up in the table of the doors its start
+// shows, and the cells of the doors a frame shows closed are bits of the same shown word as the items.
 #include "cx_agent_common.cuh"
 #include "cx_philox.cuh"
 
@@ -147,13 +149,30 @@ __global__ void __launch_bounds__(OBS_THREADS) k_agent_rollout_obs(const __grid_
     (wbase + r * slot_bytes + OBS_TILE * cells + lane * lay_bytes)[agent_k * cells + c] = v;
   };
 
-  // PICK: the static scene (basech / basek / baselay) shows every item; slot r shows the items in shown_items[r].
+  // PICK: the static scene (basech / basek / baselay) shows every item and every door closed; slot r shows the items
+  // and closed door cells in shown_items[r] (CxPickHeader).
   const uint8_t* __restrict__ s_item_at = smem + H.blob_bytes_ext + P.pk.item_at;
+  const uint64_t* __restrict__ s_drape_cells =
+      reinterpret_cast<const uint64_t*>(smem + H.blob_bytes_ext + P.pk.drape_cells);
   const CxPickItem* __restrict__ s_items = reinterpret_cast<const CxPickItem*>(smem + H.blob_bytes_ext + P.pk.items);
   const CxPickDrape* __restrict__ s_drapes =
       reinterpret_cast<const CxPickDrape*>(smem + H.blob_bytes_ext + P.pk.drapes);
   uint64_t items = 0, shown_items[RING];
   if constexpr (PICK) items = mine ? P.pick[env] : P.pk.all;
+  // PICK: the doors of `items` -- the open ones, the shown-word bits of the closed door cells, and the offsets of the
+  // open doors' step tables from the agent header's.  They change only when a key drape gives up its last item (it
+  // opens its doors) and at an auto reset (every door closes), so a step that takes nothing does no door work.
+  uint32_t open = 0, tt_off = 0, tr_off = 0, td_off = 0;
+  uint64_t closed = 0;
+  auto door_tables = [&]() {
+    tt_off = open ? P.pk.tt_first + (open - 1) * P.pk.tt_size : 0;
+    tr_off = open ? P.pk.tr_first + (open - 1) * P.pk.tt_size : 0;
+    td_off = open ? P.pk.td_first + (open - 1) * P.pk.td_size : 0;
+  };
+  if constexpr (PICK) {
+    open = cx_doors(P.pk, items, &closed);
+    door_tables();
+  }
   auto poke_item = [&](int r, uint32_t i, bool present) {  // item i of ring slot r (the agent is not drawn on it)
     const CxPickItem it = s_items[i];
     const uint32_t c = it.cell, kp = s_basek[c];
@@ -198,9 +217,9 @@ __global__ void __launch_bounds__(OBS_THREADS) k_agent_rollout_obs(const __grid_
   for (int r = 0; r < RING; ++r) {
     drawn[r] = shown;
     lcell[r] = none;
-    if constexpr (PICK) {  // the items this env has already taken leave every slot
-      shown_items[r] = P.pk.all;
-      sync_items(r, items);
+    if constexpr (PICK) {  // the items this env has already taken, and the doors that opened, leave every slot
+      shown_items[r] = P.pk.scene_all;
+      sync_items(r, items | closed);
     }
     if (shown != none) draw_agent(r, shown);
     if (layers && unocc && cell != none) {
@@ -251,9 +270,17 @@ __global__ void __launch_bounds__(OBS_THREADS) k_agent_rollout_obs(const __grid_
       // ---- phase A: the env's step (same table as k_agent_rollout) ----
       const uint32_t a = min(act[u], n_actions);
       const uint32_t idx = a * stride + cell;
-      uint32_t e = s_tt[idx];
-      float rw = s_tr[idx];
-      float dc = want_discount ? s_td[H.td_per_cell ? idx : a] : 1.0f;
+      uint32_t e;
+      float rw, dc;
+      if constexpr (PICK) {  // the doors this step's last render shows open select their own tables
+        e = s_tt[idx + tt_off];
+        rw = s_tr[idx + tr_off];
+        dc = want_discount ? s_td[(H.td_per_cell ? idx : a) + td_off] : 1.0f;
+      } else {
+        e = s_tt[idx];
+        rw = s_tr[idx];
+        dc = want_discount ? s_td[H.td_per_cell ? idx : a] : 1.0f;
+      }
       if (TRACK && (ts & CX_OVER_BIT)) {
         e = cell | (shown << 8) | (CX_FROZEN_FLAGS << 16);
         rw = 0.0f;
@@ -263,7 +290,7 @@ __global__ void __launch_bounds__(OBS_THREADS) k_agent_rollout_obs(const __grid_
       const uint32_t show = mine ? (e >> 8) & 0xFF : none;
       const uint32_t stood = mine ? p : none;   // the agent's cell in this step's frame (before any auto reset)
       uint32_t f = cx_tt_flags<PERF>(e);
-      uint64_t frame_items = 0;   // PICK: the items of this step's frame (before an auto reset)
+      uint64_t frame_items = 0;   // PICK: the shown word of this step's frame (before an auto reset)
       if constexpr (PICK) {
         // one look-up at the watched cell: the agent's cell after the move when the pickups update after it, before
         // the move otherwise (the entry-reward query); a bad action or a frozen env takes nothing
@@ -277,12 +304,24 @@ __global__ void __launch_bounds__(OBS_THREADS) k_agent_rollout_obs(const __grid_
             f |= CX_FLAG_TERMINATED;
             dc = D.emptied_value;
           }
+          if (D.opens && !(items & D.items)) {   // a key drape's last item: its doors open (cx_doors)
+            open |= D.opens;
+            closed &= ~s_drape_cells[s_items[i].drape];
+            door_tables();
+          }
         }
-        frame_items = items;
+        frame_items = items | closed;
       }
       if (TRACK && mine && cx_episode_step<PERF>(f, rw, ts, rt, stats, max_steps, auto_reset, &pf, cx_tt_perf(e))) {
         p = H.init_cell;
-        if constexpr (PICK) items = P.pk.all;   // an auto reset puts every item back
+        if constexpr (PICK) {   // an auto reset puts every item back, and closes every door
+          items = P.pk.all;
+          if (open) {
+            open = 0;
+            closed = P.pk.scene_all & ~P.pk.all;
+            door_tables();
+          }
+        }
       }
       if (mine) {
         cell = p;
@@ -397,6 +436,8 @@ int launch_obs_ring(int ring, const ObsParams& P, unsigned grid, size_t smem, cu
 bool cx_agent_obs_applies(const cx_game* g, bool layers) {
   return g->path == CX_PATH_AGENT && obs_smem_bytes(g, layers) <= 200 * 1024;
 }
+
+size_t cx_agent_obs_smem_bytes(const cx_game* g) { return obs_smem_bytes(g, false); }
 
 int cx_launch_agent_rollout_obs(const cx_game* g, void* d_state, int64_t n, int32_t T, const uint8_t* d_actions,
                                 const CxSynth& synth, float* d_reward, float* d_discount, uint8_t* d_flags,

@@ -84,11 +84,11 @@ __global__ void k_dynbd_reset(uint8_t* dynbd, const uint8_t* backdrop, int cells
   dynbd[i] = backdrop[i - e * cells];
 }
 
-// pick (games with pickups, else null): the items each env holds; basech shows every item, a taken one shows its
-// under_ch (CxPickItem)
+// pick (games with pickups, else null): the items each env holds; basech shows every item and every door closed, a
+// taken item or an open door's cell shows its under_ch (CxPickItem, CxPickHeader)
 __global__ void k_agent_render(const uint8_t* cell, const uint8_t* basech, const uint8_t* shown, int cells,
                                int agent_char, uint8_t* board, int64_t n, const uint64_t* pick,
-                               const uint8_t* item_at, const CxPickItem* items) {
+                               const uint8_t* item_at, const CxPickItem* items, const CxPickHeader ph) {
   const int64_t i = (int64_t)blockIdx.x * TB + threadIdx.x;
   if (i >= n * cells) return;
   const int64_t e = i / cells;
@@ -96,7 +96,9 @@ __global__ void k_agent_render(const uint8_t* cell, const uint8_t* basech, const
   uint8_t v = basech[c];
   if (pick) {
     const uint32_t k = item_at[c];
-    if (k != CX_NO_ITEM && !((pick[e] >> k) & 1)) v = items[k].under_ch;
+    uint64_t closed;
+    cx_doors(ph, pick[e], &closed);
+    if (k != CX_NO_ITEM && !(((pick[e] | closed) >> k) & 1)) v = items[k].under_ch;
   }
   if (shown[cell[e]] == c) v = (uint8_t)agent_char;
   board[i] = v;
@@ -668,7 +670,7 @@ int cx_launch_render(const cx_game* g, const void* d_state, int64_t n, uint8_t* 
   k_agent_render<<<blocks_for(n * g->ah.cells), TB, 0, s>>>(
       base + L.off_dyn, g->d_blob + g->ah.off_basech, g->d_blob + g->ah.off_shown, g->ah.cells, g->ah.agent_char, d_board,
       n, g->info.n_pickups ? reinterpret_cast<const uint64_t*>(base + L.off_pick) : nullptr, pk + g->ph.item_at,
-      reinterpret_cast<const CxPickItem*>(pk + g->ph.items));
+      reinterpret_cast<const CxPickItem*>(pk + g->ph.items), g->ph);
   CX_CUDA_OK(cudaGetLastError());
   return CX_OK;
 }
@@ -680,8 +682,8 @@ int cx_launch_get_entity(const cx_game* g, const void* d_state, int64_t n, int32
   const CxStateLayout L = cx_layout(g, n);
   const uint8_t* base = static_cast<const uint8_t*>(d_state);
   const int kind = g->desc.entities[z].kind;
-  if (kind == CX_KIND_STATIC || kind == CX_KIND_PICKUP) {
-    cx_set_error("cx_get_entity_state: entity %d is static or a pickup drape", z);
+  if (kind == CX_KIND_STATIC || kind == CX_KIND_PICKUP || kind == CX_KIND_DOOR) {
+    cx_set_error("cx_get_entity_state: entity %d is static, a pickup or a door drape", z);
     return CX_ERR_INVALID_ARG;
   }
   if (g->path == CX_PATH_AGENT) {

@@ -184,8 +184,14 @@ static int validate(const cx_game_desc* d) {
         cx_set_error("cx_game_create: character %d used by two entities", e.character);  // engine.py:343-350
         return CX_ERR_INVALID_ARG;
       }
-    if (e.kind > CX_KIND_PICKUP) {
+    if (e.kind > CX_KIND_DOOR) {
       cx_set_error("cx_game_create: entity %d has unknown kind %d", z, e.kind);
+      return CX_ERR_INVALID_ARG;
+    }
+    if (e.kind == CX_KIND_DOOR && (e.door_key < 0 || e.door_key >= d->n_entities ||
+                                   d->entities[e.door_key].kind != CX_KIND_PICKUP)) {
+      cx_set_error("cx_game_create: door entity %d names z-index %d as its key, which is not a pickup drape", z,
+                   e.door_key);
       return CX_ERR_INVALID_ARG;
     }
     if (e.update_rank >= d->n_entities || seen_rank[e.update_rank]++) {
@@ -426,9 +432,10 @@ static AgentStep agent_step_host(const cx_game_desc* d, int agent_z, const int* 
 }
 
 // Static composition without the agent (painter's algorithm, engine.py:306-321) and where the agent is visible; pickup
-// drapes with all their items (items_present) or none.
+// drapes with all their items (items_present) or none; door drapes closed but for the open ones (bit d: the d-th door
+// in z-order is open).
 static void compose_static(const cx_game_desc* d, int agent_z, bool items_present, std::vector<uint8_t>* basech,
-                           std::vector<uint8_t>* vis) {
+                           std::vector<uint8_t>* vis, uint32_t doors_open = 0) {
   const int cells = d->rows * d->cols;
   basech->assign(cells + 1, 0);
   vis->assign(cells + 1, 0);
@@ -436,7 +443,9 @@ static void compose_static(const cx_game_desc* d, int agent_z, bool items_presen
     (*basech)[c] = d->backdrop[c];
     (*vis)[c] = 1;
   }
+  int door = 0;
   for (int z = 0; z < d->n_entities; ++z) {
+    if (d->entities[z].kind == CX_KIND_DOOR && ((doors_open >> door++) & 1)) continue;
     if (z == agent_z || (d->entities[z].kind == CX_KIND_PICKUP && !items_present)) continue;
     const uint8_t* m = d->masks + (size_t)z * cells;
     for (int c = 0; c < cells; ++c)
@@ -444,6 +453,58 @@ static void compose_static(const cx_game_desc* d, int agent_z, bool items_presen
         (*basech)[c] = d->entities[z].character;
         if (z > agent_z) (*vis)[c] = 0;  // painted after (in front of) the agent
       }
+  }
+}
+
+// Nothing but the pickups' own reward and termination may depend on an item's presence: one Engine.play() from every
+// cell under every action must not change when all items are put back (`absent` -> `present`, same doors).
+static int check_items_irrelevant(const cx_game_desc* d, int agent_z, const int* order, const std::vector<uint8_t>& absent,
+                                  const std::vector<uint8_t>& present, const std::vector<uint8_t>& vis) {
+  const int cells = d->rows * d->cols;
+  for (int p = 0; p < cells; ++p) {
+    for (int a = 0; a < d->n_actions; ++a) {
+      const AgentStep x = agent_step_host(d, agent_z, order, absent.data(), vis.data(), a, p);
+      const AgentStep y = agent_step_host(d, agent_z, order, present.data(), vis.data(), a, p);
+      if (x.q != y.q || memcmp(&x.reward, &y.reward, 4) || x.over != y.over || memcmp(&x.discount, &y.discount, 4)) {
+        cx_set_error("cx_game_create: the step from cell %d under action %d depends on whether an item is present "
+                     "(an item or the character under it is a blocker, an entry-reward or a terminate character of "
+                     "another entity); only the pickup drape's own reward and termination may", p, a);
+        return CX_ERR_UNSUPPORTED;
+      }
+    }
+  }
+  return CX_OK;
+}
+
+// The transition tables (CxAgentHeader::off_tt / off_tr / off_td layout) of the static scene `absent`, agent visible
+// where `vis` says.
+static void fill_step_tables(const cx_game_desc* d, int agent_z, const int* order, const CxAgentHeader& H,
+                             const std::vector<uint8_t>& absent, const std::vector<uint8_t>& vis, uint32_t* tt,
+                             float* tr, float* td) {
+  const int cells = d->rows * d->cols, A = d->n_actions, S = cells + 1;
+  for (int a = 0; a <= A; ++a) {
+    if (!H.td_per_cell) td[a] = a < A ? H.act.discount[a] : 1.0f;
+    for (int p = 0; p <= cells; ++p) {
+      int q = p;
+      float reward = 0.0f, disc = 1.0f;
+      uint32_t flags = CX_FLAG_BAD_ACTION | CX_FLAG_REWARD_NONE;  // row A: env left untouched
+      if (a < A) {
+        const AgentStep st = agent_step_host(d, agent_z, order, absent.data(), vis.data(), a, p);
+        q = st.q;
+        reward = st.reward;
+        disc = st.discount;
+        flags = (st.over ? CX_FLAG_TERMINATED : 0) | (H.act.reward_none[a] ? CX_FLAG_REWARD_NONE : 0);
+      }
+      if (H.td_per_cell) td[a * S + p] = disc;
+      const int shown = (q < cells && vis[q]) ? q : cells;
+      // the step's performance rides in the spare top byte: no table, no load of its own (row A and the empty
+      // mask: 0)
+      int perf = 0;
+      if (d->n_perf_regions && a < A && p < cells && q < cells)
+        perf = cx_perf_step(d->perf_regions[p], d->perf_regions[q], d->n_perf_regions);
+      tt[a * S + p] = (uint32_t)q | ((uint32_t)shown << 8) | (flags << 16) | ((uint32_t)(uint8_t)(int8_t)perf << 24);
+      tr[a * S + p] = reward;
+    }
   }
 }
 
@@ -465,24 +526,13 @@ static int build_agent_tables(const cx_game_desc* d, int agent_z, const int* ord
   build_action_table(d, order, &H->act);
 
   // The step tables are lowered with every item absent, the scene (basech and what derives from it) shows every item
-  // present.  Games without pickups: the two are the same.
+  // present.  Games without pickups: the two are the same.  Doors: closed (the tables of the other door states are
+  // build_pick_tables').
   std::vector<uint8_t> absent, vis, basech, unused;
   compose_static(d, agent_z, false, &absent, &vis);
   compose_static(d, agent_z, true, &basech, &unused);   // (pickups in front of the agent: build_pick_tables refuses)
-  for (int p = 0; p < cells; ++p) {
-    // nothing but the pickups' own reward and termination may depend on an item's presence: one Engine.play() from
-    // every cell under every action must not change when all items are put back
-    for (int a = 0; a < A; ++a) {
-      const AgentStep x = agent_step_host(d, agent_z, order, absent.data(), vis.data(), a, p);
-      const AgentStep y = agent_step_host(d, agent_z, order, basech.data(), vis.data(), a, p);
-      if (x.q != y.q || memcmp(&x.reward, &y.reward, 4) || x.over != y.over || memcmp(&x.discount, &y.discount, 4)) {
-        cx_set_error("cx_game_create: the step from cell %d under action %d depends on whether an item is present "
-                     "(an item or the character under it is a blocker, an entry-reward or a terminate character of "
-                     "another entity); only the pickup drape's own reward and termination may", p, a);
-        return CX_ERR_UNSUPPORTED;
-      }
-    }
-  }
+  int rc = check_items_irrelevant(d, agent_z, order, absent, basech, vis);
+  if (rc != CX_OK) return rc;
   const int S = cells + 1;
   for (int z = 0; z < d->n_entities; ++z)
     for (int a = 0; a < A; ++a)
@@ -490,35 +540,8 @@ static int build_agent_tables(const cx_game_desc* d, int agent_z, const int* ord
   H->off_tt = B->reserve((size_t)(A + 1) * S * 4);
   H->off_tr = B->reserve((size_t)(A + 1) * S * 4);
   H->off_td = B->reserve((size_t)(A + 1) * (H->td_per_cell ? S : 1) * 4);
-  {
-    uint32_t* tt = (uint32_t*)&B->bytes[H->off_tt];
-    float* tr = (float*)&B->bytes[H->off_tr];
-    float* td = (float*)&B->bytes[H->off_td];
-    for (int a = 0; a <= A; ++a) {
-      if (!H->td_per_cell) td[a] = a < A ? H->act.discount[a] : 1.0f;
-      for (int p = 0; p <= cells; ++p) {
-        int q = p;
-        float reward = 0.0f, disc = 1.0f;
-        uint32_t flags = CX_FLAG_BAD_ACTION | CX_FLAG_REWARD_NONE;  // row A: env left untouched
-        if (a < A) {
-          const AgentStep st = agent_step_host(d, agent_z, order, absent.data(), vis.data(), a, p);
-          q = st.q;
-          reward = st.reward;
-          disc = st.discount;
-          flags = (st.over ? CX_FLAG_TERMINATED : 0) | (H->act.reward_none[a] ? CX_FLAG_REWARD_NONE : 0);
-        }
-        if (H->td_per_cell) td[a * S + p] = disc;
-        const int shown = (q < cells && vis[q]) ? q : cells;
-        // the step's performance rides in the spare top byte: no table, no load of its own (row A and the empty
-        // mask: 0)
-        int perf = 0;
-        if (d->n_perf_regions && a < A && p < cells && q < cells)
-          perf = cx_perf_step(d->perf_regions[p], d->perf_regions[q], d->n_perf_regions);
-        tt[a * S + p] = (uint32_t)q | ((uint32_t)shown << 8) | (flags << 16) | ((uint32_t)(uint8_t)(int8_t)perf << 24);
-        tr[a * S + p] = reward;
-      }
-    }
-  }
+  fill_step_tables(d, agent_z, order, *H, absent, vis, (uint32_t*)&B->bytes[H->off_tt], (float*)&B->bytes[H->off_tr],
+                   (float*)&B->bytes[H->off_td]);
   H->off_basech = B->reserve(S);
   memcpy(&B->bytes[H->off_basech], basech.data(), S);
   H->off_shown = B->reserve(S);
@@ -565,8 +588,10 @@ static int build_agent_tables(const cx_game_desc* d, int agent_z, const int* ord
   return CX_OK;
 }
 
-// The CX_KIND_PICKUP region of a single-agent game (CxPickHeader), appended to the blob behind the agent tables.
-static int build_pick_tables(const cx_game_desc* d, int agent_z, CxPickHeader* P, Blob* B) {
+// The CX_KIND_PICKUP (and CX_KIND_DOOR) region of a single-agent game (CxPickHeader), appended to the blob behind the
+// agent tables.
+static int build_pick_tables(const cx_game_desc* d, int agent_z, const int* order, const CxAgentHeader& H,
+                             CxPickHeader* P, Blob* B) {
   const int cells = d->rows * d->cols;
   memset(P, 0, sizeof(*P));
   int n_drapes = 0, side = -1;
@@ -593,9 +618,11 @@ static int build_pick_tables(const cx_game_desc* d, int agent_z, CxPickHeader* P
   std::vector<uint8_t> item_at(cells + 1, CX_NO_ITEM);
   std::vector<CxPickItem> items;
   std::vector<CxPickDrape> drapes;
+  std::vector<int> drape_of(d->n_entities, -1);
   for (int z = 0; z < d->n_entities; ++z) {
     const cx_entity_desc& e = d->entities[z];
     if (e.kind != CX_KIND_PICKUP) continue;
+    drape_of[z] = (int)drapes.size();
     const int ch = e.character;
     if (z > agent_z) {
       cx_set_error("cx_game_create: pickup drape '%c' lies in front of the agent in z-order; pickup drapes must be below "
@@ -661,14 +688,101 @@ static int build_pick_tables(const cx_game_desc* d, int agent_z, CxPickHeader* P
   P->n_items = (int32_t)items.size();
   P->after = side > 0 ? 1 : 0;
   P->all = P->n_items == 64 ? ~0ull : (1ull << P->n_items) - 1;
+  P->scene_all = P->all;
+
+  // doors: their cells follow the items (CxPickHeader)
+  std::vector<uint8_t> open_all, unused;
+  compose_static(d, agent_z, true, &open_all, &unused, ~0u);
+  for (int z = 0; z < d->n_entities; ++z) {
+    const cx_entity_desc& e = d->entities[z];
+    if (e.kind != CX_KIND_DOOR) continue;
+    const int ch = e.character, k = e.door_key;
+    if (P->n_doors >= CX_MAX_DOORS) {
+      cx_set_error("cx_game_create: door drape '%c' is one more than the %d doors a game may have", ch, CX_MAX_DOORS);
+      return CX_ERR_UNSUPPORTED;
+    }
+    if (z > agent_z) {
+      cx_set_error("cx_game_create: door drape '%c' lies in front of the agent in z-order; doors must be below it", ch);
+      return CX_ERR_UNSUPPORTED;
+    }
+    if (e.update_rank < d->entities[k].update_rank) {   // it would open one step after its key drape empties
+      cx_set_error("cx_game_create: door drape '%c' updates before its key drape '%c'; a door must update after its key",
+                   ch, d->entities[k].character);
+      return CX_ERR_UNSUPPORTED;
+    }
+    bool acts = e.reward_actions || e.terminate_actions || e.discount_actions || e.watch >= 0;
+    for (int a = 0; a < d->n_actions; ++a)
+      acts |= e.terminate_chars[a] || e.n_zdirs[a] || e.move_dr[a] || e.move_dc[a];
+    if (acts) {
+      cx_set_error("cx_game_create: door drape '%c' moves, watches an entity or calls a plot directive; a door may not",
+                   ch);
+      return CX_ERR_UNSUPPORTED;
+    }
+    const uint8_t* m = d->masks + (size_t)z * cells;
+    for (int c = 0; c < cells; ++c) {
+      if (!m[c]) continue;
+      if (item_at[c] != CX_NO_ITEM) {
+        cx_set_error("cx_game_create: door drape '%c' shares cell %d with an item or another door", ch, c);
+        return CX_ERR_UNSUPPORTED;
+      }
+      if (c == agent_cell) {
+        cx_set_error("cx_game_create: door drape '%c' covers the agent's initial cell %d", ch, c);
+        return CX_ERR_UNSUPPORTED;
+      }
+      if ((int)items.size() >= CX_MAX_PICKUPS) {
+        cx_set_error("cx_game_create: more than %d item and door cells in all (door drape '%c')", CX_MAX_PICKUPS, ch);
+        return CX_ERR_UNSUPPORTED;
+      }
+      CxPickItem it;
+      it.cell = (uint8_t)c;
+      it.under_ch = open_all[c];
+      const int kc = char_index(d, open_all[c]);
+      it.under_k = (uint8_t)(kc < 0 ? 0xFF : kc);
+      it.drape = (uint8_t)P->n_doors;
+      P->door_cells[P->n_doors] |= 1ull << items.size();
+      item_at[c] = (uint8_t)items.size();
+      items.push_back(it);
+    }
+    P->door_keys[P->n_doors] = drapes[drape_of[k]].items;
+    drapes[drape_of[k]].opens |= 1u << P->n_doors;
+    P->scene_all |= P->door_cells[P->n_doors];
+    ++P->n_doors;
+  }
+
+  const int A = d->n_actions, states = 1 << P->n_doors;
+  P->tt_size = (A + 1) * (cells + 1);
+  P->td_size = (A + 1) * (H.td_per_cell ? cells + 1 : 1);
   P->item_at = 0;
   P->items = (cells + 1 + 15) / 16 * 16;
   P->drapes = (P->items + (int32_t)(items.size() * sizeof(CxPickItem)) + 15) / 16 * 16;
-  P->bytes = (P->drapes + (int32_t)(drapes.size() * sizeof(CxPickDrape)) + 15) / 16 * 16;
+  P->door_tt = (P->drapes + (int32_t)(drapes.size() * sizeof(CxPickDrape)) + 15) / 16 * 16;
+  P->door_tr = P->door_tt + (states - 1) * P->tt_size * 4;
+  P->door_td = P->door_tr + (states - 1) * P->tt_size * 4;
+  P->drape_cells = (P->door_td + (states - 1) * P->td_size * 4 + 15) / 16 * 16;
+  P->bytes = P->drape_cells + (P->n_doors ? (int32_t)drapes.size() * 8 + 15 : 0) / 16 * 16;
+  P->tt_first = (H.blob_bytes_ext + P->door_tt - H.off_tt) / 4;
+  P->tr_first = (H.blob_bytes_ext + P->door_tr - H.off_tr) / 4;
+  P->td_first = (H.blob_bytes_ext + P->door_td - H.off_td) / 4;
   P->off = B->reserve(P->bytes);
   memcpy(&B->bytes[P->off + P->item_at], item_at.data(), cells + 1);
   memcpy(&B->bytes[P->off + P->items], items.data(), items.size() * sizeof(CxPickItem));
   memcpy(&B->bytes[P->off + P->drapes], drapes.data(), drapes.size() * sizeof(CxPickDrape));
+  for (int dr = 0; dr < (P->n_doors ? (int)drapes.size() : 0); ++dr) {
+    uint64_t c = 0;
+    for (int d = 0; d < P->n_doors; ++d)
+      if ((drapes[dr].opens >> d) & 1) c |= P->door_cells[d];
+    memcpy(&B->bytes[P->off + P->drape_cells + dr * 8], &c, 8);
+  }
+  for (int st = 1; st < states; ++st) {   // the step tables of every other door state, with the same item check
+    std::vector<uint8_t> absent, present, vis;
+    compose_static(d, agent_z, false, &absent, &vis, (uint32_t)st);
+    compose_static(d, agent_z, true, &present, &unused, (uint32_t)st);
+    const int rc = check_items_irrelevant(d, agent_z, order, absent, present, vis);
+    if (rc != CX_OK) return rc;
+    uint8_t* r = &B->bytes[P->off];
+    fill_step_tables(d, agent_z, order, H, absent, vis, (uint32_t*)(r + P->door_tt) + (st - 1) * P->tt_size,
+                     (float*)(r + P->door_tr) + (st - 1) * P->tt_size, (float*)(r + P->door_td) + (st - 1) * P->td_size);
+  }
   B->pad();
   return CX_OK;
 }
@@ -1042,7 +1156,7 @@ extern "C" int cx_game_create(const cx_game_desc* desc, cx_game** out) {
   if (agent_path_applies(desc, &agent_z)) {
     g->path = CX_PATH_AGENT;
     rc = build_agent_tables(desc, agent_z, order, &g->ah, &blob);
-    if (rc == CX_OK) rc = build_pick_tables(desc, agent_z, &g->ph, &blob);
+    if (rc == CX_OK) rc = build_pick_tables(desc, agent_z, order, g->ah, &g->ph, &blob);
     if (rc != CX_OK) {
       delete g;
       return rc;
@@ -1099,6 +1213,13 @@ extern "C" int cx_game_create(const cx_game_desc* desc, cx_game** out) {
   I.state_bytes_per_env = (g->path == CX_PATH_AGENT ? 1 : 2 * g->gh.n_dyn) + (tracks ? 6 : 0) +
                           (I.has_dynamic_backdrop ? cells : 0) + (I.tracks_performance ? 4 : 0) +
                           (I.n_pickups ? 8 : 0);
+  if (g->ph.n_doors && cx_agent_obs_smem_bytes(g) > 227 * 1024) {   // door games run on the lane-per-env kernel only
+    cx_set_error("cx_game_create: the step tables of the %d door states (%d bytes) and the board tiles need %zu bytes of "
+                 "shared memory per CTA, more than the 227 KB a CTA can have; use fewer doors, actions or cells",
+                 1 << g->ph.n_doors, g->ph.bytes, cx_agent_obs_smem_bytes(g));
+    delete g;
+    return CX_ERR_UNSUPPORTED;
+  }
 
   CX_CUDA_OK(cudaGetDevice(&g->device));
   CX_CUDA_OK(cudaDeviceGetAttribute(&g->sm_count, cudaDevAttrMultiProcessorCount, g->device));
@@ -1412,8 +1533,9 @@ extern "C" int cx_get_entity_state(const cx_game* g, const void* d_state, int64_
     cx_set_error("cx_get_entity_state: bad z_index %d or NULL output", z);
     return CX_ERR_INVALID_ARG;
   }
-  if (g->desc.entities[z].kind == CX_KIND_PICKUP) {
-    cx_set_error("cx_get_entity_state: entity %d is a pickup drape (its items: cx_get_pickups)", z);
+  if (g->desc.entities[z].kind == CX_KIND_PICKUP || g->desc.entities[z].kind == CX_KIND_DOOR) {
+    cx_set_error("cx_get_entity_state: entity %d is a pickup or door drape (its items, and with them the doors: "
+                 "cx_get_pickups)", z);
     return CX_ERR_INVALID_ARG;
   }
   return cx_launch_get_entity(g, d_state, n, z, d_cells, (cudaStream_t)stream);
@@ -1427,8 +1549,9 @@ extern "C" int cx_set_entity_state(const cx_game* g, void* d_state, int64_t n, i
     cx_set_error("cx_set_entity_state: bad z_index %d or NULL input", z);
     return CX_ERR_INVALID_ARG;
   }
-  if (g->desc.entities[z].kind == CX_KIND_STATIC || g->desc.entities[z].kind == CX_KIND_PICKUP) {
-    cx_set_error("cx_set_entity_state: entity %d is static or a pickup drape", z);
+  if (g->desc.entities[z].kind == CX_KIND_STATIC || g->desc.entities[z].kind == CX_KIND_PICKUP ||
+      g->desc.entities[z].kind == CX_KIND_DOOR) {
+    cx_set_error("cx_set_entity_state: entity %d is static, a pickup or a door drape", z);
     return CX_ERR_INVALID_ARG;
   }
   return cx_launch_set_entity(g, d_state, n, z, d_cells, (cudaStream_t)stream);

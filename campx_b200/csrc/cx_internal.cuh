@@ -93,18 +93,18 @@ struct CxAgentHeader {
 // bytes when the bit changes.
 #define CX_MAX_PICKUPS 64
 #define CX_NO_ITEM 0xFF
-struct CxPickItem {          // one item cell
+struct CxPickItem {          // one item cell, or one door cell
   uint8_t cell;
-  uint8_t under_ch;          // board character once the item is taken (the static scene without it)
+  uint8_t under_ch;          // board character once the item is taken / the door is open (the static scene without it)
   uint8_t under_k;           // its channel in the canonical order (0xFF: not a game character)
-  uint8_t drape;             // index into the CxPickDrape array
+  uint8_t drape;             // index into the CxPickDrape array (door cells: the door's index)
 };
 struct CxPickDrape {         // one pickup drape
   uint64_t items;            // bits of its items
   float reward[CX_MAX_ACTIONS + 1];  // add_reward value of a step that takes one of them (entry_reward[a][own char])
   float emptied_value;       // discount of the terminate_episode call once the last one is taken
   int32_t terminates;        // cx_entity_desc::terminate_emptied
-  int32_t pad;
+  uint32_t opens;            // doors whose key it is (bit d: door d), open once it is empty
 };
 struct CxPickHeader {
   int32_t n_items;           // 0: the game has no pickups
@@ -112,11 +112,42 @@ struct CxPickHeader {
   int32_t off;               // byte offset of the staged region in the blob (16-byte aligned) ...
   int32_t bytes;             // ... and its size (a multiple of 16)
   int32_t item_at;           // region offsets: u8 [cells+1] item index of every cell (CX_NO_ITEM: none) ...
-  int32_t items;             // ... CxPickItem [n_items] ...
+  int32_t items;             // ... CxPickItem [n_items + door cells] ...
   int32_t drapes;            // ... CxPickDrape [n_drapes] (8-byte aligned)
   int32_t pad;
   uint64_t all;              // every item present
+  // ---- key-locked doors (CX_KIND_DOOR).  Door d is open iff (items & door_keys[d]) == 0: the open doors of a step
+  // are a function of the items at its start, and the doors a frame shows of the items at its end.  The cells of
+  // every door follow the items as further CxPickItem entries (under_ch / under_k: the scene without the door), so
+  // that item_at and the ring slots' shown words cover them: bit n_items + j of a slot's word = door cell j shown
+  // closed.  The step tables of the other door states (1 .. 2^n_doors - 1; state 0, every door closed, is the agent
+  // header's) follow the CxPickDrape array.
+  int32_t n_doors;           // 0..CX_MAX_DOORS
+  int32_t door_tt, door_tr, door_td;  // region offsets of u32 / f32 / f32 [2^n_doors - 1][table] step tables
+  int32_t tt_size, td_size;  // elements of one tt / tr table ((n_actions+1)*(cells+1)) and of one td table
+  int32_t tt_first, tr_first, td_first;  // staged: element offset of door state 1's tt / tr / td from the agent
+                             // header's (the region lies behind the observation extension in shared memory)
+  int32_t drape_cells;       // region offset of u64 [n_drapes]: shown-word bits of the cells of the doors each
+                             // pickup drape opens (door games only)
+  uint64_t door_keys[CX_MAX_DOORS];   // items of each door's key drape
+  uint64_t door_cells[CX_MAX_DOORS];  // shown-word bits of each door's cells
+  uint64_t scene_all;        // the static scene's shown word: every item present, every door closed
 };
+
+// The doors of a game in the state `items`: returns bit d set = door d open; *closed = shown-word bits of the cells of
+// the closed doors.  The one statement of the door rule for the kernels.
+__host__ __device__ inline uint32_t cx_doors(const CxPickHeader& P, uint64_t items, uint64_t* closed) {
+  uint32_t open = 0;
+  uint64_t shut = 0;
+  for (int d = 0; d < P.n_doors; ++d) {
+    if (items & P.door_keys[d])
+      shut |= P.door_cells[d];
+    else
+      open |= 1u << d;
+  }
+  *closed = shut;
+  return open;
+}
 
 // ---- generic path tables ----
 struct CxGenEntity {
@@ -305,6 +336,7 @@ int cx_launch_agent_rollout_obs(const cx_game* g, void* d_state, int64_t n, int3
                                 const CxSynth& synth, float* d_reward, float* d_discount, uint8_t* d_flags,
                                 uint8_t* d_board, uint8_t* d_layered /* or null */, cudaStream_t s);
 bool cx_agent_obs_applies(const cx_game* g, bool layers);
+size_t cx_agent_obs_smem_bytes(const cx_game* g);   // its shared memory for board-only rollouts, one tile per warp
 // the whole policy rollout of a single-agent game in one launch (cx_agent_policy_kernels.cu)
 int cx_launch_agent_policy_rollout(const cx_game* g, void* d_state, int64_t n, int32_t T, const float* d_w1t,
                                    const float* d_b1, int32_t n_hidden, const float* d_w2, const float* d_b2, uint64_t seed,

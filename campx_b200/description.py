@@ -13,7 +13,7 @@ import numpy as np
 from . import _native as N
 
 KIND_NAMES = {N.CX_KIND_STATIC: "static", N.CX_KIND_CELL: "cell", N.CX_KIND_ROLL: "roll",
-              N.CX_KIND_SPRITE: "sprite", N.CX_KIND_PICKUP: "pickup"}
+              N.CX_KIND_SPRITE: "sprite", N.CX_KIND_PICKUP: "pickup", N.CX_KIND_DOOR: "door"}
 
 
 @dataclasses.dataclass
@@ -38,11 +38,12 @@ class EntitySpec:
     z_orders: Optional[Dict[int, List[tuple]]] = None     # action -> [(move_this, in_front_of_that or None), ...]
     terminate_emptied: Optional[float] = None             # pickups: discount passed to terminate_episode by the step
                                                           # that takes the last item (None: no such call)
+    door_key: Optional[str] = None                        # doors: the pickup drape whose emptying opens it
 
     def summary(self):
         out = {"char": self.character, "kind": KIND_NAMES[self.kind], "rank": self.update_rank,
                "group": self.update_group}
-        if self.kind not in (N.CX_KIND_STATIC, N.CX_KIND_PICKUP):
+        if self.kind not in (N.CX_KIND_STATIC, N.CX_KIND_PICKUP, N.CX_KIND_DOOR):
             out["moves"] = [tuple(m) for m in (self.moves or [])]
         if self.blockers:
             out["blockers"] = "".join(sorted(self.blockers))
@@ -67,6 +68,8 @@ class EntitySpec:
             out["z_orders"] = {a: list(v) for a, v in sorted(self.z_orders.items())}
         if self.terminate_emptied is not None:
             out["terminate_emptied"] = self.terminate_emptied
+        if self.door_key is not None:
+            out["door_key"] = self.door_key
         return out
 
 
@@ -179,6 +182,8 @@ class GameSpec:
                     c.z_front[a][k] = -1 if front_of is None else z_of[front_of]
             if e.terminate_emptied is not None:
                 c.terminate_emptied, c.emptied_value = 1, float(e.terminate_emptied)
+            if e.door_key is not None:
+                c.door_key = z_of[e.door_key]
         backdrop = np.ascontiguousarray(np.asarray(self.backdrop, dtype=np.uint8).reshape(-1))
         masks = np.ascontiguousarray(masks)
         d.backdrop = backdrop.ctypes.data_as(ctypes.POINTER(ctypes.c_uint8))

@@ -417,6 +417,13 @@ class Engine(object):
         out[:, torch.from_numpy(cells).to(dev)] = held.bool()
         return out.view(self._num_envs, self._rows, self._cols)
 
+    def door_open(self, character):
+        """bool [num_envs]: whether door drape `character` is open in every env (its key drape holds no item)."""
+        doors = [e.character for e in self._spec.entities if e.kind == N.CX_KIND_DOOR]
+        if character not in doors:
+            raise ValueError('{} is not a door drape of this game'.format(repr(character)))
+        return self._native.doors()[:, doors.index(character)]
+
     def episode_stats(self):
         return self._native.stats()
 

@@ -5,6 +5,7 @@ PyTorch is plumbing here (device memory, streams); every byte of simulation work
 libcampx_b200.so.  Nothing in this module has a CPU code path.
 """
 import ctypes
+import numpy as np
 
 import torch
 
@@ -388,6 +389,22 @@ class NativeGame(object):
         with torch.cuda.device(self.device):
             N.check(self._lib.cx_get_pickups(self._handle, _ptr(self.state), self.num_envs, _ptr(bits), _stream()))
         return bits
+
+    def doors(self):
+        """bool [num_envs, n_doors]: which key-locked doors (CX_KIND_DOOR drapes, in z-order) are open in every env.  A
+        door is open once its key drape holds no item: this reads `pickups()`."""
+        first, items_of = 0, {}        # item numbering: pickup drapes in z-order, row-major cells (cx_get_pickups)
+        for e in self.spec.entities:
+            if e.kind == N.CX_KIND_PICKUP:
+                n = int(np.count_nonzero(e.mask))
+                items_of[e.character] = ((1 << n) - 1) << first
+                first += n
+        keys = [items_of[e.door_key] for e in self.spec.entities if e.kind == N.CX_KIND_DOOR]
+        if not keys:
+            return torch.zeros((self.num_envs, 0), dtype=torch.bool, device=self.device)
+        masks = torch.tensor([k - (1 << 64) if k >= 1 << 63 else k for k in keys], dtype=torch.int64,
+                             device=self.device)
+        return (self.pickups()[:, None] & masks) == 0
 
     def fold_stats(self):
         """Add the kernels' partial statistics blocks into the float64[8] block at the head of the state blob

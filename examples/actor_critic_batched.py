@@ -322,7 +322,8 @@ def run_graphed(num_envs=4096, steps=100, iterations=5, gamma=0.99, lr=3e-2, see
 
 if __name__ == "__main__":
     ap = argparse.ArgumentParser()
-    ap.add_argument("--world", default="boat_race", help="boat_race, sprite_race, maze, demo1 .. demo4 or hello (examples/worlds.py)")
+    ap.add_argument("--world", default="boat_race", help="boat_race, sprite_race, maze, coins, doorkey, doorkey2, demo1 .. demo4 or hello "
+                                              "(examples/worlds.py; coins and doorkey: not in --mode persistent)")
     ap.add_argument("--num-envs", type=int, default=4096)
     ap.add_argument("--env-max-steps", type=int, default=100)
     ap.add_argument("--iterations", type=int, default=20)

@@ -6,6 +6,8 @@ tensors.  They are behaviourally identical to the reference's worlds
     demo1..demo4  the `Demo 1..4` notebooks (game cells)
     hello         `Hello World Example.ipynb` cells 3-4
     coins         a "collect the coins" maze (not a reference world): `Coin` is the plain collectible-item drape
+    doorkey       MiniGrid's DoorKey (not a reference world): take the key `k` (a `Coin` worth nothing), the `Door`
+                  opens, walk through to the exit; doorkey2 has two keys and two doors in a row
     maze          a sprite agent (`Runner`, PyColab's MazeWalker pattern) in a maze of walls, with treasure tiles
                   and an exit (not a reference world)
     sprite_race   boat_race with `Runner` as its agent (not a reference world)
@@ -60,6 +62,19 @@ COINS_ART = ['##########',
              '# ##  #  #',
              '#$   $ $ #',
              '##########']
+
+
+DOORKEY_ART = ['#########',
+               '#A  #   #',
+               '#   D   #',
+               '# k #  E#',
+               '#########']
+
+DOORKEY2_ART = ['############',
+                '#A  #  K#  #',
+                '#   D   d E#',
+                '# k #   #  #',
+                '############']
 
 
 MAZE_ART = ['##########',
@@ -206,7 +221,7 @@ class Slider(things.Sprite):
 
 class Coin(things.Drape):
     """Collectible items: a coin pays `value` once when the agent stands on it, then disappears; taking the last one
-    ends the episode with discount `pcontinue`."""
+    ends the episode with discount `pcontinue` (None: it does not end the episode, e.g. a key)."""
 
     def __init__(self, curtain, character, value=1.0, pcontinue=0.0, agent='A'):
         super(Coin, self).__init__(curtain, character)
@@ -219,8 +234,21 @@ class Coin(things.Drape):
         if (self.curtain * here).sum():
             self.curtain.set_(self.curtain * (1 - here))
             the_plot.add_reward(self.value)
-            if not self.curtain.any():
+            if not self.curtain.any() and self.pcontinue is not None:
                 the_plot.terminate_episode(self.pcontinue)
+
+
+class Door(things.Drape):
+    """A door locked by the key drape `key`: it opens (its whole curtain clears) in the first step that finds every key
+    taken, and stays open for the rest of the episode.  It must update after its key."""
+
+    def __init__(self, curtain, character, key='k'):
+        super(Door, self).__init__(curtain, character)
+        self.key = key
+
+    def update(self, actions, board, layers, backdrop, all_things, the_plot):
+        if actions is not None and not all_things[self.key].curtain.any():
+            self.curtain.set_(self.curtain * 0)
 
 
 def _ring_world(cw, ccw, toll, runner=False, **engine_kwargs):
@@ -241,7 +269,8 @@ def _ring_world(cw, ccw, toll, runner=False, **engine_kwargs):
 
 
 def make_world(name, **engine_kwargs):
-    """Un-started Engine for one of: boat_race, demo1, demo2, demo3, demo4, hello, coins, maze, sprite_race.
+    """Un-started Engine for one of: boat_race, demo1, demo2, demo3, demo4, hello, coins, doorkey, doorkey2, maze,
+    sprite_race.
 
     coins takes two more keywords: `update_schedule` (default 'A$#': the coins see the agent's cell after its move) and
     `coins` (the Coin drape class, or a Partial of it, default Coin).
@@ -249,6 +278,8 @@ def make_world(name, **engine_kwargs):
     maze: the sprite agent `Runner` (walls '#', -0.25 per step) in front of treasure tiles '*' (1 for every step onto
     one) and an exit 'E' (10, episode over).  The agent is drawn in front of everything it can stand on, so no render
     ever hides it; with the keyword `agent='drape'` the agent is a `Walker` drape instead, the same game.
+    doorkey: the `Walker` agent (walls '#' and the door 'D') takes the key 'k' (a `Coin` worth 0 that ends nothing), the
+    door opens, and the exit 'E' pays 10 and ends the episode.  doorkey2: key 'k' opens door 'D', key 'K' door 'd'.
     sprite_race: boat_race with `Runner` as its agent (the same game as boat_race, for the same reason); it takes
     boat_race's performance regions, BOAT_RACE_REGIONS."""
     if name == 'boat_race':
@@ -283,6 +314,16 @@ def make_world(name, **engine_kwargs):
                                  sprites={'1': Partial(Slider, 0), '2': Partial(Slider, 1),
                                           '3': Partial(Slider, 2), '4': Partial(Slider, 3)},
                                  drapes={'@': Roller}, z_order='12@34', **engine_kwargs)
+    if name in ('doorkey', 'doorkey2'):
+        from examples.generality_worlds import Exit
+        two = name == 'doorkey2'
+        drapes = {'A': Partial(Walker, walls='#Dd' if two else '#D'), 'k': Partial(Coin, value=0.0, pcontinue=None),
+                  'D': Door, 'E': Partial(Exit, 10), '#': things.FixedDrape}
+        if two:
+            drapes.update({'K': Partial(Coin, value=0.0, pcontinue=None), 'd': Partial(Door, key='K')})
+        return ascii_art_to_game(DOORKEY2_ART if two else DOORKEY_ART, ' ', drapes=drapes,
+                                 z_order='kKDdEA#' if two else 'kDEA#',
+                                 update_schedule='AEkKDd#' if two else 'AEkD#', **engine_kwargs)
     if name == 'coins':
         schedule = engine_kwargs.pop('update_schedule', 'A$#')
         coin = engine_kwargs.pop('coins', Coin)

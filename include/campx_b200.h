@@ -35,6 +35,8 @@
  *   cx_get_episode_performance             (the P / P_av columns of examples/reinforce.py:186-194)
  *   CX_KIND_PICKUP, cx_get_pickups     <-  a collectible-item Drape (clears the agent's cell, add_reward, and
  *                                          terminate_episode once empty: the "collect the coins" pattern)
+ *   CX_KIND_DOOR                       <-  a key-locked door Drape (clears its whole curtain once its key drape, a
+ *                                          CX_KIND_PICKUP drape, is empty: MiniGrid's DoorKey)
  *   cx_discounted_returns              <-  finish_episode() return scan     examples/actor_critic.py:115-135
  *   cx_fill_actions                    <-  random-action rollouts           examples/actor_critic.py:90-98
  *                                          (synthetic benchmark input; counter-based Philox4x32-10)
@@ -66,7 +68,7 @@ extern "C" {
 #define CX_API
 #endif
 
-#define CX_ABI_VERSION 8
+#define CX_ABI_VERSION 9
 
 #define CX_MAX_ENTITIES 16   /* sprites + drapes in one game                         */
 #define CX_MAX_ACTIONS 8     /* discrete actions                                     */
@@ -89,7 +91,7 @@ typedef enum cx_kind {
   CX_KIND_CELL = 1,   /* Drape with a one-cell mask that moves (AgentDrape, boat_race.py:28-59)  */
   CX_KIND_ROLL = 2,   /* Drape whose whole mask rolls toroidally (RollingDrape, Hello World)      */
   CX_KIND_SPRITE = 3, /* Sprite: (row, col) position (SlidingSprite, Hello World)                 */
-  CX_KIND_PICKUP = 4  /* Drape of collectible items (coins, keys, pellets): when its curtain holds the watched
+  CX_KIND_PICKUP = 4, /* Drape of collectible items (coins, keys, pellets): when its curtain holds the watched
                          entity's current cell as it updates, it clears that one cell and calls
                          add_reward(entry_reward[a][own char]); terminate_emptied: terminate_episode(emptied_value)
                          when that emptied the curtain.  Nothing else.  Single-agent games only (info.path == 1),
@@ -100,7 +102,17 @@ typedef enum cx_kind {
                          depend on whether an item is present (blockers, entry rewards, terminate_chars):
                          CX_ERR_UNSUPPORTED otherwise.  Items are numbered pickup drape by pickup drape in z-order,
                          row-major within a drape (cx_get_pickups bit i = item i)                            */
+  CX_KIND_DOOR = 5    /* Drape locked by a key drape (door_key, a CX_KIND_PICKUP drape): its curtain is its mask while
+                         the key drape holds an item, and empty from the first step whose update() finds the key
+                         drape empty until the episode resets.  No plot directive, no move.  The door updates after
+                         its key drape, lies below the agent in z-order, shares no cell with an item, another door
+                         or the agent's initial cell; at most CX_MAX_DOORS doors (several may share one key drape),
+                         items plus door cells at most 64: CX_ERR_UNSUPPORTED otherwise.  Door state is not stored:
+                         door d is open iff none of its key drape's items remain (cx_get_pickups).  Steps read the
+                         LAST render, so step t sees the doors as step t-1 left them                            */
 } cx_kind;
+
+#define CX_MAX_DOORS 3       /* CX_KIND_DOOR drapes in one game                      */
 
 /* Output flag bits, one byte per env-step. */
 #define CX_FLAG_TERMINATED 0x01  /* the_plot.terminate_episode() was called  (plot.py:161-184) */
@@ -130,7 +142,7 @@ typedef struct cx_entity_desc {
                               occluded (boat_race.py:52-56).  SPRITE (ABI 8; PyColab's MazeWalker): the
                               position stays where it is, occluded or not.  A SPRITE with blockers must
                               keep its visibility (visible_op[a] == CX_VIS_KEEP for every action), else
-                              CX_ERR_UNSUPPORTED.  STATIC / ROLL / PICKUP: ignored                  */
+                              CX_ERR_UNSUPPORTED.  STATIC / ROLL / PICKUP / DOOR: ignored           */
   uint8_t reward_actions;  /* bit a: update() calls the_plot.add_reward for action a              */
   uint8_t terminate_actions; /* bit a: update() calls the_plot.terminate_episode for action a     */
   uint8_t discount_actions;  /* bit a: update() calls change_default_discount (plot.py:232-257)  */
@@ -162,6 +174,8 @@ typedef struct cx_entity_desc {
   /* --- PICKUP only (ABI 7) --- */
   uint8_t terminate_emptied; /* 1: the step that takes the drape's last item calls terminate_episode(emptied_value) */
   float emptied_value;     /* discount passed by that call                                                   */
+  /* --- DOOR only (ABI 9) --- */
+  int8_t door_key;         /* z-index of the CX_KIND_PICKUP drape whose emptying opens the door                */
 } cx_entity_desc;
 
 typedef enum cx_visible_op {
