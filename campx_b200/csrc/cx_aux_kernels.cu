@@ -538,7 +538,8 @@ __global__ void __launch_bounds__(POLICY_THREADS)
   // round of memory latency covers both operands for n_in <= 256 (a loop of load -> store pays it per iteration) ----
   const float* blk = x + e0 * n_in;                            // [n_here][n_in], contiguous
   const int total = n_here * n_in;
-  const uint32_t inv = 0xFFFFFFFFu / (uint32_t)n_in + 1u;      // k / n_in by multiplication (k * n_in < 2^32)
+  const uint32_t inv = 0xFFFFFFFFu / (uint32_t)n_in + 1u;      // k / n_in by multiplication (k * n_in < 2^32); wraps
+                                                               // to 0 for n_in == 1, where k / n_in is k
   const bool w_vec = n_hidden == 32 && (reinterpret_cast<uintptr_t>(w1t) & 15) == 0;
   const bool x_vec = (reinterpret_cast<uintptr_t>(blk) & 15) == 0;
   const int w_q = w_vec ? n_in * 8 : 0, x_q = x_vec ? total / 4 : 0;   // float4 counts on the vector paths
@@ -559,7 +560,7 @@ __global__ void __launch_bounds__(POLICY_THREADS)
         const float vv[4] = {vx[u].x, vx[u].y, vx[u].z, vx[u].w};
 #pragma unroll
         for (int c = 0; c < 4; ++c) {
-          const uint32_t k = 4u * q + c, e = __umulhi(k, inv), d = k - e * (uint32_t)n_in;
+          const uint32_t k = 4u * q + c, e = n_in == 1 ? k : __umulhi(k, inv), d = k - e * (uint32_t)n_in;
           s_x[d * POLICY_PITCH + e] = vv[c];
         }
       }
@@ -571,7 +572,7 @@ __global__ void __launch_bounds__(POLICY_THREADS)
       s_w[k] = j < n_hidden ? __ldg(w1t + (size_t)d * n_hidden + j) : 0.0f;
     }
   for (int k = (x_vec ? (total & ~3) : 0) + tid; k < total; k += POLICY_THREADS) {
-    const uint32_t e = __umulhi((uint32_t)k, inv), d = (uint32_t)k - e * (uint32_t)n_in;
+    const uint32_t e = n_in == 1 ? (uint32_t)k : __umulhi((uint32_t)k, inv), d = (uint32_t)k - e * (uint32_t)n_in;
     s_x[d * POLICY_PITCH + e] = __ldcs(blk + k);
   }
   if (n_here < 32)                                             // lanes without an env compute on zeros

@@ -11,6 +11,7 @@ import torch
 from oracle import campx_oracle as O
 from examples.worlds import make_world as _make_reference_world, BOAT_RACE_REGIONS
 from examples.generality_worlds import make_generality_world
+from tests.helpers.policy_reference import philox4
 
 pytestmark = pytest.mark.gpu
 
@@ -240,18 +241,6 @@ def test_rollout_equals_play_and_sharding_is_deterministic():
         obs, reward, _ = step.play(a_full[t])
         assert torch.equal(obs.board, out_full[0][t]) and torch.equal(reward, out_full[1][t])
         assert torch.equal(step.flags, out_full[3][t])
-
-
-def philox4(seed, quad, t):
-    """Host reference of campx_b200/csrc/cx_philox.cuh (Philox4x32-10)."""
-    M0, M1, W0, W1 = 0xD2511F53, 0xCD9E8D57, 0x9E3779B9, 0xBB67AE85
-    k0, k1 = seed & 0xFFFFFFFF, seed >> 32
-    c = [quad & 0xFFFFFFFF, quad >> 32, t & 0xFFFFFFFF, t >> 32]
-    for _ in range(10):
-        p0, p1 = M0 * c[0], M1 * c[2]
-        c = [(p1 >> 32) ^ c[1] ^ k0, p1 & 0xFFFFFFFF, (p0 >> 32) ^ c[3] ^ k1, p0 & 0xFFFFFFFF]
-        k0, k1 = (k0 + W0) & 0xFFFFFFFF, (k1 + W1) & 0xFFFFFFFF
-    return c
 
 
 def test_philox_actions_match_host_reference():
